@@ -61,6 +61,9 @@ def parse():
                     help="parameter points of the full-grid light-curve sweep in extra.config4 (BASELINE configs[3])")
     ap.add_argument("--no-extra", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's lnprob and RHS-evaluation count of every walker as "
+                         "DIR/<output>_<dataset>.npy (float64, rank 0), to compare two builds output for output")
     return ap.parse_args()
 
 
@@ -240,6 +243,21 @@ class ClockSampler(threading.Thread):
                 "reasons": sorted(reasons), "samples": len(sm)}
 
 
+DUMP_ROWS = 1 << 20     # walker rows per dumped output: six outputs plus the row index stay under 64 MB
+
+
+def dump_outputs(path, outputs):
+    """Write every per-walker output as path/<name>.npy in float64.  Past DUMP_ROWS walkers each output keeps the
+    same seeded sample of rows, and the rows kept are written as walker_index.npy."""
+    os.makedirs(path, exist_ok=True)
+    W = len(next(iter(outputs.values())))
+    if W > DUMP_ROWS:
+        rows = np.sort(np.random.RandomState(0).choice(W, DUMP_ROWS, replace=False))
+        outputs = {**{k: v[rows] for k, v in outputs.items()}, "walker_index": rows}
+    for name, a in outputs.items():
+        np.save(os.path.join(path, f"{name}.npy"), np.asarray(a, dtype=np.float64))
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -300,6 +318,9 @@ def run_ours(args):
     wall = time.perf_counter() - wall0
     gpu_launches = sum(lk.kernels_launched() for lk in liks.values()) - launches0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {f"{what}_{n}": buf[n].double().cpu().numpy()
+                                         for n in DATASETS for what, buf in (("lnprob", d_lnp), ("n_rhs", d_nrhs))})
     ms = sum(a.elapsed_time(b) for a, b in ev)
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
     if world > 1:
