@@ -260,6 +260,17 @@ int mp_chain_moments(const double* d_chain, int64_t n, int32_t ndim, double* mea
                      int32_t device, void* stream);
 int mp_chain_order_statistics(const double* d_chain, int64_t n, int32_t ndim, int32_t col,
                               const int64_t* ranks, int32_t n_ranks, double* values, int32_t device, void* stream);
+/* Walker-averaged normalised autocorrelation function of a device-resident chain [n_steps][nwalkers][ndim]
+ * (emcee's integrated_time before the window): rows first, first+thin, ...; lags [lag_begin, lag_end) of the
+ * n = ceil((n_steps-first)/thin) retained rows; acf is a HOST array [ndim][lag_end-lag_begin].  Synchronises.
+ *   acf[d][k-lag_begin] = (1/nwalkers) sum_w C_wd(k) / C_wd(0),   C_wd(k) = sum_{t<n-k} s_t s_{t+k},
+ * s_t the series of walker w, dimension d minus its mean, computed directly (no FFT).  The mean is taken after
+ * shifting the series by its first retained sample, so an exactly constant series (a stuck walker, or n = 1)
+ * has C(0) = 0 and makes acf[d] NaN -- what emcee's formula gives in exact arithmetic.  The sums run in a fixed
+ * order (no atomics): two calls on one chain return identical bits on any stream.                           */
+int mp_chain_autocorr(const double* d_chain, int64_t n_steps, int32_t nwalkers, int32_t ndim,
+                      int64_t first, int64_t thin, int64_t lag_begin, int64_t lag_end,
+                      double* acf, int32_t device, void* stream);
 
 /* The comparison model of the reference's figure 5 (code/figure_5.py:222-363, "Ben's model": an accreting-mass
  * magnetar with an exponentially draining disc, explicit Euler steps of 1 s in a Python loop over 1e6 elements).

@@ -145,6 +145,8 @@ def declare(lib):
     lib.mp_peer_barrier.argtypes = [C.c_int32, vp, C.POINTER(vp), C.c_int32, C.c_int32, C.c_uint64, vp, vp]
     lib.mp_chain_moments.argtypes = [vp, C.c_int64, C.c_int32, vp, vp, C.c_int32, vp]
     lib.mp_chain_order_statistics.argtypes = [vp, C.c_int64, C.c_int32, C.c_int32, vp, C.c_int32, vp, C.c_int32, vp]
+    lib.mp_chain_autocorr.argtypes = [vp, C.c_int64, C.c_int32, C.c_int32, C.c_int64, C.c_int64, C.c_int64, C.c_int64,
+                                      vp, C.c_int32, vp]
     lib.mp_gompertz_curves.argtypes = [vp, C.c_int32, vp, C.c_int64, C.c_int32, vp, C.c_int32]
     lib.mp_kernels_launched.argtypes = [vp]
     lib.mp_kernels_launched.restype = C.c_int64
@@ -158,7 +160,7 @@ EXPORTS = ["mp_abi_version", "mp_device_count", "mp_last_error", "mp_create", "m
            "mp_curve_nodes", "mp_model_curves", "mp_model_curves_device", "mp_rhs_batch",
            "mp_stretch_half_step", "mp_fp64_peak_tflops", "mp_last_stiff_count",
            "mp_ensemble_half_step", "mp_ensemble_sync", "mp_ensemble_unpack", "mp_ensemble_order",
-           "mp_chain_moments", "mp_chain_order_statistics", "mp_gompertz_curves", "mp_kernels_launched",
+           "mp_chain_moments", "mp_chain_order_statistics", "mp_chain_autocorr", "mp_gompertz_curves", "mp_kernels_launched",
            "mp_peer_alloc", "mp_peer_open", "mp_peer_close", "mp_peer_free", "mp_peer_barrier"]
 
 

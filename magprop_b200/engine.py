@@ -197,6 +197,20 @@ def chain_order_statistics(d_chain: int, n: int, ndim: int, col: int, ranks, dev
     return out
 
 
+def chain_autocorr(d_chain: int, n_steps: int, nwalkers: int, ndim: int, first=0, thin=1, lag_begin=0, lag_end=None,
+                   device=0, stream=0) -> np.ndarray:
+    """Walker-averaged normalised autocorrelation function [ndim, lag_end - lag_begin] of a device-resident chain
+    [n_steps, nwalkers, ndim] (raw pointer), over rows first, first + thin, ...; ``lag_end=None``: every lag of the
+    retained rows.  The mean over walkers of emcee's ``function_1d`` (``synth_mcmc.function_1d``)."""
+    lib = A.load()
+    n = (int(n_steps) - int(first) + int(thin) - 1) // int(thin) if thin >= 1 else 0
+    lag_end = n if lag_end is None else int(lag_end)
+    out = np.empty((max(0, int(ndim)), max(0, lag_end - int(lag_begin))))
+    A.check(lib.mp_chain_autocorr(d_chain, n_steps, nwalkers, ndim, first, thin, lag_begin, lag_end, A.ptr(out), device,
+                                  stream or None))
+    return out
+
+
 def gompertz_curves(pars, n_steps=10 ** 6, stride=1, alpha=0.1, cs7=1.0, k=0.9, omass=1.4, dipeff=1.0, propeff=1.0, device=0):
     """The comparison model of the reference's figure 5 (``code/figure_5.py:222-363``) on the device:
     returns ``(t, curves)`` with ``curves[W, 3, n_out]`` = Ltot, Lprop, Ldip (/1e50) at ``t = 1 + i*stride`` s."""

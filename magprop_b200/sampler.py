@@ -356,16 +356,59 @@ class DeviceEnsemble:
         t = self.torch
         chain = t.empty((nsteps, self.nwalkers, self.ndim), dtype=t.float64, device=self.device) if store else None
         lps = t.empty((nsteps, self.nwalkers), dtype=t.float64, device=self.device) if store else None
+        self._advance(nsteps, chain, lps, 0)
+        self.sync()
+        return (chain, lps) if store else None
+
+    def _advance(self, nsteps, chain=None, lps=None, row=0):
+        """nsteps steps; with ``chain``, rows row, row + 1, ... of chain / lps receive the state after each step."""
         for it in range(nsteps):
             self._half(0)
             self._half(1)
             self.step += 1
-            if store:
+            if chain is not None:
                 self.sync()
-                chain[it].copy_(self.coords)
-                lps[it].copy_(self.lnp)
+                chain[row + it].copy_(self.coords)
+                lps[row + it].copy_(self.lnp)
+
+    def run_until_converged(self, max_steps, check_every=100, n_tau=50, tau_rtol=0.01, c=5):
+        """Run until the chain has converged, as emcee's "monitoring convergence" recipe does: every ``check_every``
+        steps the integrated autocorrelation time tau of the chain so far is computed (without the length check), and
+        the run stops once every parameter has ``step > n_tau * tau`` and ``|tau - tau_prev| / tau < tau_rtol`` (tau_prev:
+        the previous check's; a NaN tau never passes).  Stops at ``max_steps`` otherwise.  The chain is stored in one
+        ``[max_steps, nwalkers, ndim]`` buffer on the ensemble's device; tau comes from ``integrated_time_device``
+        there, from ``integrated_time`` for a CPU ensemble.  With ``dist`` every rank decides from its full replica
+        and the decision is all-reduced, so all ranks stop at the same step.
+
+        Returns ``(chain[:n], lnp[:n], tau_history [n_checks, ndim], converged)``; the chain is that of ``run(n)``."""
+        from .synthetic.synth_mcmc import integrated_time, integrated_time_device
+        max_steps, check_every = int(max_steps), int(check_every)
+        if max_steps < 1 or check_every < 1:
+            raise ValueError("max_steps and check_every must be positive")
+        t = self.torch
+        chain = t.empty((max_steps, self.nwalkers, self.ndim), dtype=t.float64, device=self.device)
+        lps = t.empty((max_steps, self.nwalkers), dtype=t.float64, device=self.device)
+        history, tau_prev, converged, n = [], np.full(self.ndim, np.inf), False, 0
+        while n < max_steps and not converged:
+            k = min(check_every, max_steps - n)
+            self._advance(k, chain, lps, n)
+            n += k
+            if n % check_every:
+                break
+            if self.device.type == "cuda":
+                tau = integrated_time_device(chain[:n], c=c, quiet=True)
+            else:
+                tau = integrated_time(chain[:n].numpy(), c=c, quiet=True)
+            history.append(tau)
+            with np.errstate(invalid="ignore", divide="ignore"):
+                ok = bool(np.all(n > n_tau * tau) and np.all(np.abs(tau_prev - tau) / tau < tau_rtol))
+            if self.dist:
+                flag = t.tensor([int(ok)], dtype=t.int32, device=self.device)
+                self.dist.all_reduce(flag, op=self.dist.ReduceOp.MIN)
+                ok = bool(flag.item())
+            converged, tau_prev = ok, tau
         self.sync()
-        return (chain, lps) if store else None
+        return chain[:n], lps[:n], np.array(history).reshape(len(history), self.ndim), converged
 
     def check_peers(self):
         """Raise if a cross-GPU barrier timed out (a peer died)."""

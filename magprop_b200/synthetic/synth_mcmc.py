@@ -135,16 +135,41 @@ def integrated_time(x, c=5, tol=50, quiet=False):
     if len(x.shape) != 3:
         raise ValueError("invalid dimensions")
     n_t, n_w, n_d = x.shape
-    tau_est = np.empty(n_d)
-    windows = np.empty(n_d, dtype=int)
+    f = np.zeros((n_d, n_t))
     for d in range(n_d):
-        f = np.zeros(n_t)
         for k in range(n_w):
-            f += function_1d(x[:, k, d])
-        f /= n_w
-        taus = 2.0 * np.cumsum(f) - 1.0
-        windows[d] = _auto_window(taus, c)
-        tau_est[d] = taus[windows[d]]
+            f[d] += function_1d(x[:, k, d])
+        f[d] /= n_w
+    return _tau_from_acf(lambda lo, hi: f[:, lo:hi], n_t, n_d, c, tol, quiet)
+
+
+def _tau_from_acf(acf, n_t, n_d, c, tol, quiet):
+    """Sokal's window and emcee's length check on a walker-averaged ACF of ``n_t`` rows that ``acf(lo, hi)`` delivers
+    as lags [lo, hi) ([n_d, hi - lo]).  Lags are requested in blocks [0, L) with L = min(n_t, 128), 256, ... until every
+    dimension's window lies inside them, so about twice the window is computed instead of all n_t lags.  The result is
+    the full-length one bit for bit: ``np.cumsum`` adds in order, so the taus of a prefix are the prefix of the taus,
+    and the first M with M >= c*tau(M) is decided as soon as the prefix holds one M that passes and one that fails."""
+    f = np.empty((n_d, 0))
+    tau_est = np.empty(n_d)
+    done = np.zeros(n_d, dtype=bool)
+    L = 0
+    while not done.all():
+        hi = min(n_t, max(128, 2 * L))
+        f = np.concatenate([f, acf(L, hi)], axis=1)
+        L = hi
+        for d in np.flatnonzero(~done):
+            taus = 2.0 * np.cumsum(f[d]) - 1.0
+            m = np.arange(L) < c * taus
+            if L == n_t:
+                window = _auto_window(taus, c)
+            elif np.isnan(taus[0]):          # every tau is NaN (a constant series): so is the estimate, whatever the window
+                window = 0
+            elif m.any() and not m.all():
+                window = int(np.argmin(m))
+            else:
+                continue
+            tau_est[d] = taus[window]
+            done[d] = True
     flag = tol * tau_est > n_t
     if np.any(flag):
         msg = ("The chain is shorter than {0} times the integrated autocorrelation time for {1} parameter(s). "
@@ -153,6 +178,34 @@ def integrated_time(x, c=5, tol=50, quiet=False):
         if not quiet:
             raise AutocorrError(tau_est, msg)
     return tau_est
+
+
+def integrated_time_device(chain, c=5, tol=50, quiet=False, discard=0, thin=1):
+    """``integrated_time`` of a float64 CUDA tensor chain [n_steps, nwalkers, ndim], computed where the chain lies:
+    the walker-averaged autocorrelation function comes from ``mp_chain_autocorr`` for the lags Sokal's window needs,
+    and only [ndim, L] numbers reach the host.  Same window, same ``AutocorrError``, as ``integrated_time``.
+
+    ``discard`` / ``thin`` follow emcee 3's ``EnsembleSampler.get_autocorr_time(discard, thin)``: the rows are those of
+    ``Backend.get_value``, ``chain[discard + thin - 1::thin]``, and the returned tau is multiplied by ``thin`` (the
+    length check and the tau an ``AutocorrError`` carries are those of the thinned chain, as there)."""
+    import torch
+    from ..engine import chain_autocorr
+    if not (isinstance(chain, torch.Tensor) and chain.is_cuda and chain.dtype == torch.float64 and chain.dim() == 3):
+        raise ValueError("integrated_time_device: chain must be a float64 CUDA tensor [n_steps, nwalkers, ndim]")
+    discard, thin = int(discard), int(thin)
+    n_steps, n_w, n_d = chain.shape
+    first = discard + thin - 1
+    if discard < 0 or thin < 1 or first >= n_steps:
+        raise ValueError("integrated_time_device: no rows left after discard / thin")
+    chain = chain.contiguous()
+    n_t = len(range(first, n_steps, thin))
+    device = chain.device.index
+    stream = torch.cuda.current_stream(chain.device).cuda_stream
+
+    def acf(lo, hi):
+        return chain_autocorr(chain.data_ptr(), n_steps, n_w, n_d, first, thin, lo, hi, device=device, stream=stream)
+
+    return thin * _tau_from_acf(acf, n_t, n_d, c, tol, quiet)
 
 
 # ---- the reference's output files ------------------------------------------------------------
