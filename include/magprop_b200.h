@@ -233,6 +233,28 @@ int mp_ensemble_unpack(const mp_ensemble* ens, uint64_t step, int32_t split, con
 int mp_ensemble_order(int32_t nwalkers, uint64_t seed, uint64_t step, int32_t randomize_split,
                       int32_t* d_order, void* stream);
 
+/* ---- parallel-tempered ensembles (emcee 2's PTSampler / ptemcee) -------------------------------------
+ * ntemps temperatures x n = e->nwalkers walkers per temperature: coords [ntemps][n][ndim], lnp [ntemps][n] and
+ * accepted / status / n_rhs [ntemps][n]; row r = t*n + w.  lnp is UNTEMPERED (lnlike + lnprior).  betas is a HOST
+ * array of ntemps inverse temperatures: betas[0] == 1, strictly decreasing, all > 0; ntemps <= MP_MAX_TEMPS and
+ * ntemps*n < 2^31.  world must be 1, n_peers 0 and pack_out NULL.  Every argument is checked on the host before
+ * any device work (MP_ERR_BAD_ARG).
+ *
+ * mp_tempered_half_step: half-step `split` of every temperature in ONE fused launch.  Each temperature moves as
+ *   mp_ensemble_half_step moves one ensemble -- shared split P of (seed, step), partners from the complementary half
+ *   of the same temperature, Philox counter (2*step + split, r) -- except that the accept test is
+ *   (ndim-1) ln z + beta_t lnp(q) - beta_t lnp(x) > ln u'.  With ntemps = 1 it is mp_ensemble_half_step bit for bit.
+ * mp_tempered_swap: once per MCMC step, after half-step 1.  For t = ntemps-1 down to 1 and every column j, walker j
+ *   of temperature t swaps its row and lnp with walker j of t-1 iff
+ *   ln u < (betas[t-1] - betas[t]) (lnp[t][j] - lnp[t-1][j]),  u from Philox counter (step, t*n + j, word 3).
+ *   d_swap_accepted[ntemps-1] (may be NULL) counts the accepted swaps of each adjacent pair (t-1, t).
+ *   Runs on the current device.                                                                               */
+#define MP_MAX_TEMPS 256
+int mp_tempered_half_step(mp_handle* h, const mp_ensemble* e, int32_t ntemps, const double* betas, uint64_t step,
+                          int32_t split, void* stream);
+int mp_tempered_swap(const mp_ensemble* e, int32_t ntemps, const double* betas, uint64_t step,
+                     int32_t* d_swap_accepted, void* stream);
+
 /* Peer-mappable device memory for the replicas (CUDA IPC; one process per GPU on one node).
  * mp_peer_alloc: cudaMalloc + export a 64-byte handle other processes pass to mp_peer_open, which maps the
  * block into the caller's address space on `device` (NVLink peer access).  mp_peer_barrier: every rank calls

@@ -14,6 +14,7 @@ import numpy as np
 MP_MAX_NDIM = 9
 MP_ABI_VERSION = 2
 MP_MAX_PEERS = 15
+MP_MAX_TEMPS = 256
 
 MP_OK, MP_ERR_BAD_ARG, MP_ERR_DATA_RANGE, MP_ERR_CUDA, MP_ERR_BAD_GRID, MP_ERR_NO_DATA = range(6)
 
@@ -138,6 +139,8 @@ def declare(lib):
     lib.mp_ensemble_sync.argtypes = [C.POINTER(Ensemble), C.c_uint64, vp]
     lib.mp_ensemble_unpack.argtypes = [C.POINTER(Ensemble), C.c_uint64, C.c_int32, vp, vp]
     lib.mp_ensemble_order.argtypes = [C.c_int32, C.c_uint64, C.c_uint64, C.c_int32, vp, vp]
+    lib.mp_tempered_half_step.argtypes = [vp, C.POINTER(Ensemble), C.c_int32, vp, C.c_uint64, C.c_int32, vp]
+    lib.mp_tempered_swap.argtypes = [C.POINTER(Ensemble), C.c_int32, vp, C.c_uint64, vp, vp]
     lib.mp_peer_alloc.argtypes = [C.c_int32, C.c_uint64, C.POINTER(vp), C.c_char_p]
     lib.mp_peer_open.argtypes = [C.c_int32, C.c_char_p, C.POINTER(vp)]
     lib.mp_peer_close.argtypes = [C.c_int32, vp]
@@ -160,6 +163,7 @@ EXPORTS = ["mp_abi_version", "mp_device_count", "mp_last_error", "mp_create", "m
            "mp_curve_nodes", "mp_model_curves", "mp_model_curves_device", "mp_rhs_batch",
            "mp_stretch_half_step", "mp_fp64_peak_tflops", "mp_last_stiff_count",
            "mp_ensemble_half_step", "mp_ensemble_sync", "mp_ensemble_unpack", "mp_ensemble_order",
+           "mp_tempered_half_step", "mp_tempered_swap",
            "mp_chain_moments", "mp_chain_order_statistics", "mp_chain_autocorr", "mp_gompertz_curves", "mp_kernels_launched",
            "mp_peer_alloc", "mp_peer_open", "mp_peer_close", "mp_peer_free", "mp_peer_barrier"]
 

@@ -10,7 +10,8 @@
 //                     light-curve output; or the stretch move's accept step)           per walker with a shuffle-
 //                                                                                       reduced chi-square
 // plus rhs_kernel (the coupled reference RHS for ODEs()/odes() callers), the ensemble-order and peer-barrier
-// helpers of the device-resident sampler, and dfma_peak_kernel (FP64 FMA roofline denominator).
+// helpers of the device-resident sampler, pt_swap_kernel (replica exchange of a parallel-tempered ensemble), and
+// dfma_peak_kernel (FP64 FMA roofline denominator).
 #include <cuda_runtime.h>
 
 #include <cstddef>
@@ -198,7 +199,7 @@ __global__ void order_scatter_kernel(int W, const int* __restrict__ key, int* __
 
 // The stretch move wrapped around an evaluation (mp_stretch_half_step / mp_ensemble_half_step):
 //   z = ((a-1) u + 1)^2 / a ; q = c - (c - s) z ; accept iff (ndim-1) ln z + lp(q) - lp(s) > ln u'
-// (Goodman & Weare 2010; emcee's RedBlueMove).  setup_kernel forms the proposals, the reduce kernels accept.
+// (Goodman & Weare 2010; emcee's RedBlueMove); tempered: beta_t lp(q) - beta_t lp(s).  setup_kernel forms the proposals, the reduce kernels accept.
 struct Move {
   double* coords;        // [nwalkers][ndim], updated in place
   double* lnp;           // [nwalkers]
@@ -210,6 +211,11 @@ struct Move {
   SplitPerm perm;
   int pos0, cpos0;
   int n_complement;
+  // ... or a tempered ensemble (mp_tempered_half_step; null on every other path): mover mover0 + i is the
+  // tempered_mover of the positions above, its partner comes from its own temperature, and the accept test
+  // weighs the log-probabilities by betas[t]
+  const double* betas;
+  int mover0;
   double a;
   uint64_t seed, step;   // step: the half-step counter (RNG counter word)
   double* prop;          // [n_active][ndim] the proposals (work space)
@@ -236,7 +242,7 @@ struct Move {
 
 struct Draw {
   double z, ua;
-  int me, partner, pj;
+  int me, partner, pj, t;
 };
 // Which rank's replica holds walker w's current row (see Move).
 __device__ __forceinline__ int home_before_this_step(const Move& m, int w) {
@@ -249,10 +255,17 @@ __device__ __forceinline__ const double* replica_coords(const Move& m, int home)
 __device__ __forceinline__ const double* replica_lnp(const Move& m, int home) {
   return home == m.rank ? m.lnp : m.peer_lnp[home < m.rank ? home : home - 1];
 }
-// counter = (half-step, walker); two Philox blocks give u_z, u_partner, u_accept
+// counter = (half-step, walker); two Philox blocks give u_z, u_partner, u_accept.  (Tempered: walker = global row.)
 __device__ __forceinline__ Draw draw_for(const Move& m, int i) {
   Draw d;
-  d.me = m.active ? m.active[i] : (int)perm_at(m.perm, (uint32_t)(m.pos0 + i));
+  d.t = 0;
+  if (m.betas) {
+    const TemperedMover tm = tempered_mover(m.perm, (uint32_t)m.pos0, (uint32_t)(m.mover0 + i));
+    d.t = (int)tm.t;
+    d.me = (int)tm.row;
+  } else {
+    d.me = m.active ? m.active[i] : (int)perm_at(m.perm, (uint32_t)(m.pos0 + i));
+  }
   const Philox r0 = philox4x32_10((uint32_t)m.step, (uint32_t)(m.step >> 32), (uint32_t)d.me, 0u,
                                   (uint32_t)m.seed, (uint32_t)(m.seed >> 32));
   const Philox r1 = philox4x32_10((uint32_t)m.step, (uint32_t)(m.step >> 32), (uint32_t)d.me, 1u,
@@ -264,7 +277,8 @@ __device__ __forceinline__ Draw draw_for(const Move& m, int i) {
   d.z = __ddiv_rn(__dmul_rn(zr, zr), m.a);
   int pj = (int)(up * m.n_complement);
   if (pj >= m.n_complement) pj = m.n_complement - 1;
-  d.partner = m.complement ? m.complement[pj] : (int)perm_at(m.perm, (uint32_t)(m.cpos0 + pj));
+  if (m.betas) d.partner = (int)tempered_partner(m.perm, (uint32_t)m.cpos0, (uint32_t)d.t, (uint32_t)pj);
+  else d.partner = m.complement ? m.complement[pj] : (int)perm_at(m.perm, (uint32_t)(m.cpos0 + pj));
   d.pj = pj;
   return d;
 }
@@ -594,7 +608,13 @@ __device__ __forceinline__ void deliver(const Problem& p, const Work& k, const S
   const int me = d.me;
   const double* q = m.prop + (size_t)i * ndim;
   const double lp_old = m.lnp[me];
-  const double lnpdiff = __dadd_rn(__dadd_rn(__dmul_rn(ndim - 1.0, log(d.z)), lp_new), -lp_old);
+  double lq = lp_new, lx = lp_old;           // tempered: beta_t lp (lnp stays untempered)
+  if (m.betas) {
+    const double b = m.betas[d.t];
+    lq = __dmul_rn(b, lp_new);
+    lx = __dmul_rn(b, lp_old);
+  }
+  const double lnpdiff = __dadd_rn(__dadd_rn(__dmul_rn(ndim - 1.0, log(d.z)), lq), -lx);
   const bool accept = lnpdiff > log(d.ua);
   if (accept) {
     for (int c = 0; c < ndim; ++c) m.coords[(size_t)me * ndim + c] = q[c];
@@ -760,6 +780,39 @@ __global__ void sync_replica_kernel(const __grid_constant__ Move m, int n, int n
 __global__ void order_kernel(SplitPerm perm, int n, int* __restrict__ order) {
   const int g = blockIdx.x * blockDim.x + threadIdx.x;
   if (g < n) order[g] = (int)perm_at(perm, (uint32_t)g);
+}
+
+// Replica exchange of a tempered ensemble (mp_tempered_swap): thread j owns column j and walks the adjacent pairs
+// from the hottest down, so a row can travel more than one temperature in one step, as in ptemcee.  Columns are
+// independent: no thread reads another's rows.  Accepted swaps are counted per pair, one atomic per warp.
+struct PtLadder {
+  double beta[MP_MAX_TEMPS];
+};
+__global__ void pt_swap_kernel(double* __restrict__ coords, double* __restrict__ lnp, int n, int ndim, int ntemps,
+                               const __grid_constant__ PtLadder lad, uint64_t seed, uint64_t step, int* __restrict__ accepted) {
+  const int j = blockIdx.x * blockDim.x + threadIdx.x;
+  const bool have = j < n;
+  for (int t = ntemps - 1; t >= 1; --t) {
+    bool sw = false;
+    if (have) {
+      const size_t hot = (size_t)t * n + j, cold = hot - n;
+      const double lh = lnp[hot], lc = lnp[cold];
+      sw = pt_swap_accept(seed, step, (uint32_t)hot, lad.beta[t - 1], lad.beta[t], lh, lc);
+      if (sw) {
+        for (int c = 0; c < ndim; ++c) {
+          const double x = coords[hot * ndim + c];
+          coords[hot * ndim + c] = coords[cold * ndim + c];
+          coords[cold * ndim + c] = x;
+        }
+        lnp[hot] = lc;
+        lnp[cold] = lh;
+      }
+    }
+    if (accepted) {
+      const unsigned b = __ballot_sync(kFull, sw);
+      if ((threadIdx.x & 31) == 0 && b) atomicAdd(accepted + t - 1, __popc(b));
+    }
+  }
 }
 
 // ---- cross-GPU flag barrier over peer-mapped memory ---------------------------------------------
@@ -1196,6 +1249,8 @@ struct mp_handle {
     StiffRec* squeue = nullptr;
     double* prop = nullptr;
     size_t cap_walkers = 0, cap_ybuf = 0, cap_prop = 0;
+    double* betas = nullptr;     // the ladder of the tempered half-steps on this lane, and its host copy
+    std::vector<double> betas_host;
     int* hint_host = nullptr;    // mapped pinned int[4]: counters[4..7] of the last large launch on this lane (see launch_eval)
     int* hint_dev = nullptr;     // the device's pointer to it
   } lanes[2];
@@ -1302,6 +1357,7 @@ extern "C" void mp_destroy(mp_handle* h) {
     if (L.hint_host) cudaFreeHost(L.hint_host);
     cudaFree(L.recs); cudaFree(L.ybuf); cudaFree(L.status); cudaFree(L.n_rhs); cudaFree(L.work);
     cudaFree(L.counters); cudaFree(L.squeue); cudaFree(L.prop); cudaFree(L.key); cudaFree(L.hist); cudaFree(L.slot_wid);
+    cudaFree(L.betas);
     if (L.stream) cudaStreamDestroy(L.stream);
   };
   for (auto& L : h->lanes) free_lane(L);
@@ -1423,6 +1479,7 @@ static int launch_eval(mp_handle* h, const Problem& p, const double* d_theta, in
     Move ms = m;
     if (MOVE) {
       if (ms.active) ms.active += i0;
+      else if (ms.betas) ms.mover0 += i0;     // (a tempered slab may span temperatures: offset the mover, not the position)
       else ms.pos0 += i0;
       ms.prop = Lp->prop;
       if (ms.pack_out) ms.pack_out += (size_t)i0 * (ndim + 1);
@@ -1756,16 +1813,9 @@ extern "C" int mp_ensemble_sync(const mp_ensemble* e, uint64_t step, void* strea
   return MP_OK;
 }
 
-extern "C" int mp_ensemble_half_step(mp_handle* h, const mp_ensemble* e, uint64_t step, int32_t split, void* stream) {
-  if (!h) return fail(MP_ERR_BAD_ARG, "mp_ensemble_half_step: null handle");
-  int rc = check_ensemble(e, "mp_ensemble_half_step");
-  if (rc) return rc;
-  if (split != 0 && split != 1) return fail(MP_ERR_BAD_ARG, "mp_ensemble_half_step: split must be 0 or 1");
-  MP_CUDA(cudaSetDevice(h->device));
+// The move of this rank's share of half `split` at MCMC step `step` (everything but the pull side).
+static void fill_ensemble_move(const mp_ensemble* e, uint64_t step, int split, Move& m) {
   const int half = e->nwalkers / 2, n_mine = half / e->world;
-  Problem p;
-  if ((rc = fill_move_problem(h, p, e->ndim, n_mine))) return rc;
-  Move m;
   std::memset(&m, 0, sizeof(m));
   m.coords = e->coords;
   m.lnp = e->lnp;
@@ -1779,7 +1829,6 @@ extern "C" int mp_ensemble_half_step(mp_handle* h, const mp_ensemble* e, uint64_
   m.accepted = e->accepted;
   m.status = e->status;
   m.n_rhs = e->n_rhs;
-  if ((rc = fill_pull(e, step, m, "mp_ensemble_half_step"))) return rc;
   m.split = split;
   m.pack_out = e->pack_out;
   if (e->bad_rows && e->bad_count && e->bad_capacity > 0) {
@@ -1787,8 +1836,89 @@ extern "C" int mp_ensemble_half_step(mp_handle* h, const mp_ensemble* e, uint64_
     m.bad_count = e->bad_count;
     m.bad_capacity = e->bad_capacity;
   }
+}
+
+extern "C" int mp_ensemble_half_step(mp_handle* h, const mp_ensemble* e, uint64_t step, int32_t split, void* stream) {
+  if (!h) return fail(MP_ERR_BAD_ARG, "mp_ensemble_half_step: null handle");
+  int rc = check_ensemble(e, "mp_ensemble_half_step");
+  if (rc) return rc;
+  if (split != 0 && split != 1) return fail(MP_ERR_BAD_ARG, "mp_ensemble_half_step: split must be 0 or 1");
+  MP_CUDA(cudaSetDevice(h->device));
+  const int n_mine = e->nwalkers / 2 / e->world;
+  Problem p;
+  if ((rc = fill_move_problem(h, p, e->ndim, n_mine))) return rc;
+  Move m;
+  fill_ensemble_move(e, step, split, m);
+  if ((rc = fill_pull(e, step, m, "mp_ensemble_half_step"))) return rc;
   return launch_eval<kModeLnprob, true>(h, p, nullptr, n_mine, Sink{nullptr, nullptr, nullptr}, nullptr, nullptr, &m,
                                         (cudaStream_t)stream);
+}
+
+// ---- parallel tempering ----------------------------------------------------------------------------
+// Both tempered entry points check everything on the host, before any device work: a bad ladder is
+// MP_ERR_BAD_ARG on a machine without a GPU too.
+static int check_tempered(const mp_ensemble* e, int32_t ntemps, const double* betas, const char* who) {
+  int rc = check_ensemble(e, who);
+  if (rc) return rc;
+  const std::string w(who);
+  if (e->world != 1 || e->n_peers != 0 || e->pack_out)
+    return fail(MP_ERR_BAD_ARG, w + ": a tempered ensemble runs on one rank (world 1, no peers, no pack_out)");
+  if (e->ndim < 1 || e->ndim > MP_MAX_NDIM) return fail(MP_ERR_BAD_ARG, w + ": bad ndim");
+  if (ntemps < 1 || ntemps > MP_MAX_TEMPS || !betas)
+    return fail(MP_ERR_BAD_ARG, w + ": ntemps must be in [1, MP_MAX_TEMPS] and betas non-null");
+  if ((int64_t)ntemps * e->nwalkers >= ((int64_t)1 << 31))
+    return fail(MP_ERR_BAD_ARG, w + ": ntemps * nwalkers must be below 2^31");
+  if (betas[0] != 1.0) return fail(MP_ERR_BAD_ARG, w + ": betas[0] must be 1");
+  for (int t = 1; t < ntemps; ++t)
+    if (!(betas[t] > 0.0 && betas[t] < betas[t - 1]))     // (NaN fails too)
+      return fail(MP_ERR_BAD_ARG, w + ": betas must be strictly decreasing and positive");
+  return MP_OK;
+}
+
+// The ladder a lane's tempered half-steps read: copied in stream order, and only when it differs from the last one.
+static int upload_ladder(mp_handle::Lane& L, int ntemps, const double* betas, cudaStream_t stream) {
+  if (L.betas_host.size() == (size_t)ntemps && std::equal(betas, betas + ntemps, L.betas_host.begin())) return MP_OK;
+  if (!L.betas) MP_CUDA(cudaMalloc((void**)&L.betas, MP_MAX_TEMPS * sizeof(double)));
+  L.betas_host.clear();
+  MP_CUDA(cudaMemcpyAsync(L.betas, betas, (size_t)ntemps * sizeof(double), cudaMemcpyHostToDevice, stream));
+  L.betas_host.assign(betas, betas + ntemps);
+  return MP_OK;
+}
+
+extern "C" int mp_tempered_half_step(mp_handle* h, const mp_ensemble* e, int32_t ntemps, const double* betas, uint64_t step,
+                                     int32_t split, void* stream) {
+  int rc = check_tempered(e, ntemps, betas, "mp_tempered_half_step");
+  if (rc) return rc;
+  if (!h) return fail(MP_ERR_BAD_ARG, "mp_tempered_half_step: null handle");
+  if (split != 0 && split != 1) return fail(MP_ERR_BAD_ARG, "mp_tempered_half_step: split must be 0 or 1");
+  MP_CUDA(cudaSetDevice(h->device));
+  const cudaStream_t s = (cudaStream_t)stream;
+  const int half = e->nwalkers / 2, n_movers = ntemps * half;
+  Problem p;
+  if ((rc = fill_move_problem(h, p, e->ndim, n_movers))) return rc;
+  mp_handle::Lane* L = nullptr;
+  lane_for(h, s, -1, &L);
+  if ((rc = upload_ladder(*L, ntemps, betas, s))) return rc;
+  Move m;
+  fill_ensemble_move(e, step, split, m);
+  m.rank = 0;
+  m.half = m.n_mine = half;
+  m.betas = L->betas;
+  return launch_eval<kModeLnprob, true>(h, p, nullptr, n_movers, Sink{nullptr, nullptr, nullptr}, nullptr, nullptr, &m, s);
+}
+
+extern "C" int mp_tempered_swap(const mp_ensemble* e, int32_t ntemps, const double* betas, uint64_t step,
+                                int32_t* d_swap_accepted, void* stream) {
+  int rc = check_tempered(e, ntemps, betas, "mp_tempered_swap");
+  if (rc) return rc;
+  if (ntemps == 1) return MP_OK;
+  PtLadder lad;
+  std::memset(&lad, 0, sizeof(lad));
+  std::memcpy(lad.beta, betas, (size_t)ntemps * sizeof(double));
+  pt_swap_kernel<<<(e->nwalkers + 127) / 128, 128, 0, (cudaStream_t)stream>>>(e->coords, e->lnp, e->nwalkers, e->ndim, ntemps,
+                                                                              lad, e->seed, step, d_swap_accepted);
+  MP_CUDA(cudaGetLastError());
+  return MP_OK;
 }
 
 extern "C" int mp_ensemble_unpack(const mp_ensemble* e, uint64_t step, int32_t split, const double* d_packed, void* stream) {

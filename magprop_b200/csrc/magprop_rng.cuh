@@ -1,7 +1,9 @@
-// magprop_rng.cuh -- counter-based random numbers of the ensemble move: Philox4x32-10 draws and the keyed
-// permutation that defines the per-step random halves.  Plain C++ apart from the qualifiers, so the CPU
-// tests can compile it for the host and pin it against their NumPy restatement.
+// magprop_rng.cuh -- counter-based random numbers of the ensemble move: Philox4x32-10 draws, the keyed
+// permutation that defines the per-step random halves, and parallel tempering's mover -> row mapping and swap
+// decision.  Plain C++ apart from the qualifiers, so the CPU tests can compile it for the host and pin it against
+// their NumPy restatement.
 #pragma once
+#include <math.h>
 #include <stdint.h>
 
 #if defined(__CUDACC__)
@@ -97,6 +99,31 @@ inline SplitPerm make_split_perm(int n, uint64_t seed, uint64_t step, int random
   p.k0 = k.c[0];
   p.k1 = k.c[1];
   return p;
+}
+
+// ---- parallel tempering: T temperatures x n walkers, row r = t*n + w -----------------------------------
+// Every temperature is one ensemble moved as above, all sharing the split P of the step.  Mover g of a tempered
+// half-step is the (g mod n/2)-th mover of temperature g / (n/2); its partner is drawn from the same temperature.
+struct TemperedMover {
+  uint32_t t, row;
+};
+MP_RNG_HD TemperedMover tempered_mover(const SplitPerm& p, uint32_t pos0, uint32_t g) {
+  const uint32_t half = p.n / 2u;
+  TemperedMover m;
+  m.t = g / half;
+  m.row = m.t * p.n + perm_at(p, pos0 + (g - m.t * half));
+  return m;
+}
+MP_RNG_HD uint32_t tempered_partner(const SplitPerm& p, uint32_t cpos0, uint32_t t, uint32_t pj) {
+  return t * p.n + perm_at(p, cpos0 + pj);
+}
+// The replica exchange of column j between temperature t (row_hot = t*n + j) and t-1, at MCMC step `step`:
+// swap iff ln u < (beta_{t-1} - beta_t) (lnp_hot - lnp_cold), u from Philox counter (step, row_hot, 3) -- word 3
+// is used by no other draw.  lnp is untempered; a NaN (both -inf) rejects.
+MP_RNG_HD bool pt_swap_accept(uint64_t seed, uint64_t step, uint32_t row_hot, double beta_cold, double beta_hot,
+                              double lnp_hot, double lnp_cold) {
+  const Philox r = philox4x32_10((uint32_t)step, (uint32_t)(step >> 32), row_hot, 3u, (uint32_t)seed, (uint32_t)(seed >> 32));
+  return log(u01(r.c[0], r.c[1])) < (beta_cold - beta_hot) * (lnp_hot - lnp_cold);
 }
 
 }  // namespace mp

@@ -90,6 +90,39 @@ def run(grb, x, y, yerr, n_walk, n_step, seed=0, p0=None, device=0, dist=None, f
     return res
 
 
+def run_tempered(grb, x, y, yerr, n_walk, ntemps, n_step, beta_min, seed=0, discard=None, device=0):
+    """A parallel-tempered run (``TemperedEnsemble``): ``ntemps`` temperatures on a geometric ladder from 1 down to
+    ``beta_min``, ``n_walk`` walkers each, every temperature started from ``initial_ball``.  Returns the ``RunResult``
+    of the cold chain (``write_outputs`` and ``posterior_summary_device`` take it as they take ``run``'s) with
+    ``log_evidence`` / ``log_evidence_err`` (``thermodynamic_log_evidence`` over the steps after ``discard``; None:
+    the first half), ``betas``, ``swap_acceptance`` [ntemps - 1] and the device-resident cold chain and lnp of every
+    temperature (``chain_device``, ``lnp_device``) attached.  The ladder should reach the prior:
+    ``beta_min * <lnL>_{beta_min}`` is the part of ln Z the hottest temperature stands for."""
+    from .. import _capi as A
+    from ..engine import Likelihood, time_grid
+    from ..sampler import TemperedEnsemble, geometric_betas, thermodynamic_log_evidence
+    from .mcmc_eqns import lower, upper
+
+    betas = geometric_betas(ntemps, beta_min)
+    discard = n_step // 2 if discard is None else int(discard)
+    rng = np.random.RandomState(seed)
+    p0 = np.stack([initial_ball(grb, n_walk, rng=rng) for _ in range(ntemps)])
+    lk = Likelihood(A.script_model_spec(), time_grid(None), x, y, yerr, lower, upper, device=device)
+    try:
+        ens = TemperedEnsemble.from_likelihood(lk, n_walk, p0.shape[2], betas, a=2.0, seed=seed)
+        ens.initialise(p0)
+        chain, lnp = ens.run(n_step, store=True)
+        log_z, dlog_z = thermodynamic_log_evidence(betas, lnp, discard=discard)
+        res = RunResult(chain.cpu().numpy(), lnp[:, 0].cpu().numpy(), ens.acceptance_fraction()[0].cpu().numpy(), seed)
+        res.log_evidence, res.log_evidence_err = log_z, dlog_z
+        res.betas = betas
+        res.swap_acceptance = ens.swap_acceptance_fraction().cpu().numpy()
+        res.chain_device, res.lnp_device = chain, lnp        # CUDA tensors [n_step, n_walk, ndim], [n_step, ntemps, n_walk]
+    finally:
+        lk.close()
+    return res
+
+
 # ---- integrated autocorrelation time (emcee.autocorr, restated; emcee is not installed) -----------
 def _next_pow_two(n):
     i = 1
