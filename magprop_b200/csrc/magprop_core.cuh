@@ -1707,7 +1707,9 @@ MP_HD void prepare_walker(const Spec& sp, const double* theta, int ndim, bool us
   r.k1 = in.k1;
   r.regime0 = in.regime;
   r.n_rhs = in.n_rhs;
-  if (in.status != kWalkerOk) r.status = kWalkerIntegratorFail;
+  // (t_end == t_start -- a handle without data, or one whose data all sit at the first grid time: the initial state
+  // is the whole solution, and the zero step integrator_init leaves for an empty span is not a failure)
+  if (in.status != kWalkerOk && t_end > t_start) r.status = kWalkerIntegratorFail;
 }
 
 // The explicit integrator as prepare_walker left it (C: the walker's disc-mass transient amplitude, Walker::C).

@@ -54,8 +54,9 @@ struct Problem {
 // Device work space of one launch (a slab of walkers), owned by the handle's lane.  Layouts follow the readers:
 //   recs   the stage-1 records as a structure of arrays -- 8-byte word k of walker i at recs[k*stride + i] -- so
 //          that the one-thread-per-walker kernels read and write them coalesced
-//   ybuf   node j of walker i at ybuf[i*ws + j*ns]: walker-minor (ws = 1, ns = stride) when stage 3 runs one
-//          thread per walker (small datasets), node-minor (ws = Nn, ns = 1) when it runs one warp per walker
+//   ybuf   node j of walker i at ybuf[i*ws + j*ns]: walker-minor (ws = 1, ns = the launch's slab size S) when stage 3
+//          runs one thread per walker (small datasets), node-minor (ws = Nn, ns = 1) when it runs one warp per walker;
+//          either way it spans S * Nn values (recs' stride is the lane's capacity, which may exceed S)
 struct Work {
   int W;               // walkers in the slab
   int stride;          // slab capacity
@@ -1471,8 +1472,10 @@ static int launch_eval(mp_handle* h, const Problem& p, const double* d_theta, in
   if (MOVE) m = *mv;
   else std::memset(&m, 0, sizeof(m));
   const bool coop = Nn > 64 || MODE == kModeCurves;   // by the DATASET only: a walker's lnprob never depends on the batch it is in
+  // (ybuf holds S * Nn values: its walker-minor stride is this launch's slab, not the lane's record capacity, which an
+  // earlier launch of more walkers on fewer nodes may have made larger)
   k.ws = coop ? (size_t)Nn : 1;
-  k.ns = coop ? 1 : (size_t)k.stride;
+  k.ns = coop ? 1 : (size_t)S;
   for (int i0 = 0; i0 < W; i0 += S) {
     const int n = std::min(S, W - i0);
     k.W = n;
