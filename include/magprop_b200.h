@@ -275,9 +275,13 @@ int mp_peer_barrier(int32_t device, uint64_t* d_my_flags, uint64_t* const* peer_
  *   mp_chain_moments            column means and the covariance matrix (n-1 normalisation, as np.cov /
  *                               np.corrcoef use); host outputs mean[ndim], cov[ndim][ndim]
  *   mp_chain_order_statistics   the ranks[r]-th smallest value (0-based) of column `col`, exactly (radix select
- *                               on the IEEE bit patterns); np.percentile's linear interpolation between two
- *                               neighbouring order statistics is the caller's (it is done AFTER un-logging,
- *                               plot_synth.py:160-166)                                                   */
+ *                               on the IEEE bit patterns, 64-bit counts): -0.0 before +0.0, every NaN last (a
+ *                               NaN comes back with its sign bit cleared); np.percentile's linear interpolation
+ *                               between two neighbouring order statistics is the caller's (it is done AFTER
+ *                               un-logging, plot_synth.py:160-166).  Ranks outside [0, n) are MP_ERR_BAD_ARG.
+ * Both run on `stream` with stream-ordered allocations and synchronise it before returning.  No floating-point
+ * atomics: the blocks' partial sums are added in a fixed order, so two calls on one chain return identical bits on
+ * any stream.                                                                                                */
 int mp_chain_moments(const double* d_chain, int64_t n, int32_t ndim, double* mean, double* cov,
                      int32_t device, void* stream);
 int mp_chain_order_statistics(const double* d_chain, int64_t n, int32_t ndim, int32_t col,

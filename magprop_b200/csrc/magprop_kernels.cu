@@ -847,7 +847,11 @@ __global__ void peer_barrier_kernel(uint64_t* my_flags, PeerFlags pf, int rank, 
 // ---- posterior summaries of a device-resident chain (plot_synth.py:150-166) -------------------------------
 // Column means and the centred cross-products (for np.corrcoef), and exact order statistics by radix select
 // (for np.percentile): the chain never leaves the device, the host receives a few dozen numbers.
-__global__ void chain_mean_kernel(const double* __restrict__ x, long long n, int ndim, double* __restrict__ sums) {
+// No floating-point atomics: every block writes its partial sums to part[block][q], and a one-block finish kernel adds
+// them in block order -- the result depends only on n and ndim, so two calls on one chain agree bit for bit.
+constexpr int kMomBlocks = 1184, kMomThreads = 256;
+
+__global__ void chain_mean_kernel(const double* __restrict__ x, long long n, int ndim, double* __restrict__ part) {
   __shared__ double sh[MP_MAX_NDIM][8];
   double acc[MP_MAX_NDIM];
   for (int d = 0; d < MP_MAX_NDIM; ++d) acc[d] = 0.0;
@@ -863,12 +867,22 @@ __global__ void chain_mean_kernel(const double* __restrict__ x, long long n, int
   if (threadIdx.x < ndim) {
     double v = 0.0;
     for (int w = 0; w < (int)(blockDim.x >> 5); ++w) v += sh[threadIdx.x][w];
-    atomicAdd(sums + threadIdx.x, v);
+    part[blockIdx.x * ndim + threadIdx.x] = v;
   }
 }
 
+// mean[d] = (sum of the blocks' partials in block order) / n
+__global__ void chain_mean_finish_kernel(const double* __restrict__ part, int blocks, long long n, int ndim,
+                                         double* __restrict__ mean) {
+  const int d = threadIdx.x;
+  if (d >= ndim) return;
+  double v = 0.0;
+  for (int b = 0; b < blocks; ++b) v += part[b * ndim + d];
+  mean[d] = v / (double)n;
+}
+
 __global__ void chain_cov_kernel(const double* __restrict__ x, long long n, int ndim, const double* __restrict__ mean,
-                                 double* __restrict__ cov /*[ndim][ndim], upper triangle*/) {
+                                 double* __restrict__ part /*[block][npair], pairs (a <= b) row by row*/) {
   __shared__ double sh[MP_MAX_NDIM * MP_MAX_NDIM][8];
   double acc[MP_MAX_NDIM * (MP_MAX_NDIM + 1) / 2];
   const int npair = ndim * (ndim + 1) / 2;
@@ -892,26 +906,54 @@ __global__ void chain_cov_kernel(const double* __restrict__ x, long long n, int 
   if (threadIdx.x < npair) {
     double v = 0.0;
     for (int w = 0; w < (int)(blockDim.x >> 5); ++w) v += sh[threadIdx.x][w];
-    int q = 0;
-    for (int a = 0; a < ndim; ++a)
-      for (int b = a; b < ndim; ++b, ++q)
-        if (q == (int)threadIdx.x) atomicAdd(cov + a * ndim + b, v);
+    part[blockIdx.x * npair + threadIdx.x] = v;
   }
 }
 
-// IEEE doubles as unsigned keys in ascending order (NaNs last).
+// cov[a][b] = cov[b][a] = (sum of the blocks' partials of pair (a, b) in block order) / max(n - 1, 1)
+__global__ void chain_cov_finish_kernel(const double* __restrict__ part, int blocks, long long n, int ndim,
+                                        double* __restrict__ cov) {
+  const int npair = ndim * (ndim + 1) / 2, q = threadIdx.x;
+  if (q >= npair) return;
+  int a = 0, r = q;
+  while (r >= ndim - a) {   // row a of the upper triangle holds pairs (a, a..ndim-1)
+    r -= ndim - a;
+    ++a;
+  }
+  const int b = a + r;
+  double v = 0.0;
+  for (int k = 0; k < blocks; ++k) v += part[k * npair + q];
+  v /= (double)(n > 1 ? n - 1 : 1);
+  cov[a * ndim + b] = v;
+  cov[b * ndim + a] = v;
+}
+
+// IEEE doubles as unsigned keys in ascending order: -inf < ... < -0 < +0 < ... < +inf < every NaN.  A NaN's sign bit
+// is dropped, so a NaN made with the sign bit set (0/0 on x86) sorts last too, as np.sort puts it.
 __device__ __forceinline__ unsigned long long order_key(double v) {
-  const unsigned long long b = (unsigned long long)__double_as_longlong(v);
+  unsigned long long b = (unsigned long long)__double_as_longlong(v);
+  if ((b & 0x7fffffffffffffffull) > 0x7ff0000000000000ull) b &= 0x7fffffffffffffffull;
   return (b >> 63) ? ~b : (b | 0x8000000000000000ull);
 }
 // One pass of the radix select on column `col`: histogram of the 16-bit digit at `shift` over the elements whose
-// higher digits equal those of `prefix`.
+// higher digits equal those of `prefix`.  64-bit bins, so a column of 2^32 or more equal digits cannot wrap one.  The
+// lanes of a warp that fall in the same bin add to it once (match + popc): a chain's ties (stuck walkers, a long
+// constant column) otherwise serialise on one address.
 __global__ void select_hist_kernel(const double* __restrict__ x, long long n, int ndim, int col, unsigned long long prefix,
-                                   int shift, unsigned* __restrict__ hist) {
+                                   int shift, unsigned long long* __restrict__ hist) {
   const unsigned long long himask = (shift >= 48) ? 0ull : (~0ull << (shift + 16));
-  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
-    const unsigned long long key = order_key(x[i * ndim + col]);
-    if ((key & himask) == (prefix & himask)) atomicAdd(hist + (unsigned)((key >> shift) & 0xffffull), 1u);
+  const int lane = threadIdx.x & 31;
+  const long long stride = (long long)gridDim.x * blockDim.x;
+  // base is the warp's first row: the loop condition is uniform over the warp, so every lane reaches the match
+  for (long long base = blockIdx.x * (long long)blockDim.x + (threadIdx.x & ~31); base < n; base += stride) {
+    const long long i = base + lane;
+    unsigned bin = 0xffffffffu;                          // no bin: past the end, or another prefix
+    if (i < n) {
+      const unsigned long long key = order_key(x[i * ndim + col]);
+      if ((key & himask) == (prefix & himask)) bin = (unsigned)((key >> shift) & 0xffffull);
+    }
+    const unsigned peers = __match_any_sync(kFull, bin);
+    if (bin != 0xffffffffu && lane == __ffs(peers) - 1) atomicAdd(hist + bin, (unsigned long long)__popc(peers));
   }
 }
 
@@ -2012,31 +2054,25 @@ extern "C" int mp_chain_moments(const double* d_chain, int64_t n, int32_t ndim, 
   if (mp_device_count() <= device || device < 0) return fail(MP_ERR_CUDA, "mp_chain_moments: no such CUDA device");
   MP_CUDA(cudaSetDevice(device));
   cudaStream_t st = (cudaStream_t)stream;
-  double* d_acc = nullptr;
-  MP_CUDA(cudaMalloc((void**)&d_acc, (ndim + ndim * ndim) * sizeof(double)));
-  cudaError_t e = cudaMemsetAsync(d_acc, 0, (ndim + ndim * ndim) * sizeof(double), st);
-  const int blocks = (int)std::min<int64_t>((n + 255) / 256, 1184);
-  std::vector<double> hm(ndim), hc((size_t)ndim * ndim);
-  if (e == cudaSuccess) {
-    chain_mean_kernel<<<blocks, 256, 0, st>>>(d_chain, n, ndim, d_acc);
-    e = cudaMemcpyAsync(hm.data(), d_acc, ndim * sizeof(double), cudaMemcpyDeviceToHost, st);
-  }
+  const int blocks = (int)std::min<int64_t>((n + kMomThreads - 1) / kMomThreads, kMomBlocks);
+  const int npair = ndim * (ndim + 1) / 2;
+  const size_t n_out = (size_t)ndim + (size_t)ndim * ndim;
+  double* d_buf = nullptr;
+  MP_CUDA(cudaMallocAsync((void**)&d_buf, (n_out + (size_t)blocks * npair) * sizeof(double), st));
+  double *d_mean = d_buf, *d_cov = d_mean + ndim, *d_part = d_cov + (size_t)ndim * ndim;   // part: [blocks][ndim or npair]
+  chain_mean_kernel<<<blocks, kMomThreads, 0, st>>>(d_chain, n, ndim, d_part);
+  chain_mean_finish_kernel<<<1, 32, 0, st>>>(d_part, blocks, n, ndim, d_mean);
+  chain_cov_kernel<<<blocks, kMomThreads, 0, st>>>(d_chain, n, ndim, d_mean, d_part);
+  chain_cov_finish_kernel<<<1, 64, 0, st>>>(d_part, blocks, n, ndim, d_cov);
+  std::vector<double> h(n_out);
+  cudaError_t e = cudaGetLastError();
+  if (e == cudaSuccess) e = cudaMemcpyAsync(h.data(), d_buf, n_out * sizeof(double), cudaMemcpyDeviceToHost, st);
+  const cudaError_t ef = cudaFreeAsync(d_buf, st);
+  if (e == cudaSuccess) e = ef;
   if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-  if (e == cudaSuccess) {
-    for (int d = 0; d < ndim; ++d) hm[d] /= (double)n;
-    e = cudaMemcpyAsync(d_acc, hm.data(), ndim * sizeof(double), cudaMemcpyHostToDevice, st);
-  }
-  if (e == cudaSuccess) {
-    chain_cov_kernel<<<blocks, 256, 0, st>>>(d_chain, n, ndim, d_acc, d_acc + ndim);
-    e = cudaMemcpyAsync(hc.data(), d_acc + ndim, (size_t)ndim * ndim * sizeof(double), cudaMemcpyDeviceToHost, st);
-  }
-  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-  cudaFree(d_acc);
   if (e != cudaSuccess) return fail(MP_ERR_CUDA, std::string("mp_chain_moments: ") + cudaGetErrorString(e));
-  for (int a = 0; a < ndim; ++a) {
-    mean[a] = hm[a];
-    for (int b = a; b < ndim; ++b) cov[a * ndim + b] = cov[b * ndim + a] = hc[(size_t)a * ndim + b] / (double)(n - 1 > 0 ? n - 1 : 1);
-  }
+  std::memcpy(mean, h.data(), ndim * sizeof(double));
+  std::memcpy(cov, h.data() + ndim, (size_t)ndim * ndim * sizeof(double));
   return MP_OK;
 }
 
@@ -2044,37 +2080,40 @@ extern "C" int mp_chain_order_statistics(const double* d_chain, int64_t n, int32
                                          int32_t n_ranks, double* values, int32_t device, void* stream) {
   if (!d_chain || !ranks || !values || n < 1 || ndim < 1 || col < 0 || col >= ndim || n_ranks < 0)
     return fail(MP_ERR_BAD_ARG, "mp_chain_order_statistics: bad argument");
+  for (int r = 0; r < n_ranks; ++r)
+    if (ranks[r] < 0 || ranks[r] >= n) return fail(MP_ERR_BAD_ARG, "mp_chain_order_statistics: rank outside [0, n)");
   if (mp_device_count() <= device || device < 0) return fail(MP_ERR_CUDA, "mp_chain_order_statistics: no such CUDA device");
   MP_CUDA(cudaSetDevice(device));
   cudaStream_t st = (cudaStream_t)stream;
-  unsigned* d_hist = nullptr;
-  MP_CUDA(cudaMalloc((void**)&d_hist, 65536 * sizeof(unsigned)));
-  std::vector<unsigned> hist(65536);
+  unsigned long long* d_hist = nullptr;
+  MP_CUDA(cudaMallocAsync((void**)&d_hist, 65536 * sizeof(unsigned long long), st));
+  std::vector<unsigned long long> hist(65536);
   const int blocks = (int)std::min<int64_t>((n + 255) / 256, 1184);
   cudaError_t e = cudaSuccess;
   for (int r = 0; r < n_ranks && e == cudaSuccess; ++r) {
-    int64_t k = ranks[r];
-    if (k < 0 || k >= n) { cudaFree(d_hist); return fail(MP_ERR_BAD_ARG, "mp_chain_order_statistics: rank outside [0, n)"); }
+    unsigned long long k = (unsigned long long)ranks[r];
     unsigned long long prefix = 0ull;
-    for (int shift = 48; shift >= 0 && e == cudaSuccess; shift -= 16) {
-      e = cudaMemsetAsync(d_hist, 0, 65536 * sizeof(unsigned), st);
-      if (e != cudaSuccess) break;
-      select_hist_kernel<<<blocks, 256, 0, st>>>(d_chain, n, ndim, col, prefix, shift, d_hist);
-      e = cudaMemcpyAsync(hist.data(), d_hist, 65536 * sizeof(unsigned), cudaMemcpyDeviceToHost, st);
+    for (int shift = 48; shift >= 0; shift -= 16) {
+      e = cudaMemsetAsync(d_hist, 0, 65536 * sizeof(unsigned long long), st);
+      if (e == cudaSuccess) {
+        select_hist_kernel<<<blocks, 256, 0, st>>>(d_chain, n, ndim, col, prefix, shift, d_hist);
+        e = cudaGetLastError();
+      }
+      if (e == cudaSuccess)
+        e = cudaMemcpyAsync(hist.data(), d_hist, 65536 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st);
       if (e == cudaSuccess) e = cudaStreamSynchronize(st);
       if (e != cudaSuccess) break;
       unsigned digit = 0;
-      for (; digit < 65536u; ++digit) {
-        if (k < (int64_t)hist[digit]) break;
-        k -= hist[digit];
-      }
+      for (; digit < 65535u && k >= hist[digit]; ++digit) k -= hist[digit];
       prefix |= (unsigned long long)digit << shift;
     }
     // key -> double
     const unsigned long long b = (prefix >> 63) ? (prefix & 0x7fffffffffffffffull) : ~prefix;
     std::memcpy(values + r, &b, sizeof(double));
   }
-  cudaFree(d_hist);
+  const cudaError_t ef = cudaFreeAsync(d_hist, st);
+  if (e == cudaSuccess) e = ef;
+  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
   if (e != cudaSuccess) return fail(MP_ERR_CUDA, std::string("mp_chain_order_statistics: ") + cudaGetErrorString(e));
   return MP_OK;
 }

@@ -129,7 +129,7 @@ def test_posterior_summary_on_the_device_matches_the_host_one(built, golden):
     # the summary
     s_dev, p_dev = P.posterior_summary_device(chain, x, y, yerr, grb="Humped")
     s_host, p_host, _, _ = P.posterior_summary(host, x, y, yerr, grb="Humped")
-    assert np.allclose(p_dev, p_host, rtol=1e-14, atol=0)
+    assert np.array_equal(p_dev, p_host)
     assert np.allclose(s_dev["correlations"], s_host["correlations"], rtol=1e-9, atol=1e-12)
     for k in s_host["pars"]:
         assert np.allclose(s_dev["pars"][k], s_host["pars"][k], rtol=1e-12, atol=1e-300)
