@@ -39,17 +39,9 @@
 #endif
 
 #include "disc_table.inc"
+#include "magprop_constants.hpp"
 
 namespace mp {
-
-// ---- physical constants: funcs.py:12-18, magnetar/funcs.py:7-13 -------------
-constexpr double kG = 6.674e-8;
-constexpr double kC = 3.0e10;
-constexpr double kR = 1.0e6;
-constexpr double kMsol = 1.99e33;
-constexpr double kM = 1.4 * kMsol;
-constexpr double kGM = kG * kM;
-constexpr double kTwoPi = 6.283185307179586476925286766559;
 
 constexpr int kWalkerOk = 0;
 constexpr int kWalkerPriorReject = 1;

@@ -1,4 +1,5 @@
-// magprop_kernels.cu -- sm_100a kernels and the C ABI of include/magprop_b200.h.
+// magprop_kernels.cu -- the evaluation pipeline: its sm_100a kernels, the likelihood handle and every entry point of
+// include/magprop_b200.h that launches the pipeline.
 //
 // FP64 throughout, no tensor cores -- the path is a scalar ODE solve per walker, not a contraction.
 // One likelihood evaluation runs as a short pipeline of launches on one stream (DESIGN.md section 3):
@@ -9,21 +10,25 @@
 //   reduce_*_kernel   luminosity -> interpolation -> chi-square -> lnprob (or model /  thread per walker, or a warp
 //                     light-curve output; or the stretch move's accept step)           per walker with a shuffle-
 //                                                                                       reduced chi-square
-// plus rhs_kernel (the coupled reference RHS for ODEs()/odes() callers), the ensemble-order and peer-barrier
-// helpers of the device-resident sampler, pt_swap_kernel (replica exchange of a parallel-tempered ensemble), and
-// dfma_peak_kernel (FP64 FMA roofline denominator).
+// plus the ensemble-order helpers of the device-resident sampler and pt_swap_kernel (replica exchange of a
+// parallel-tempered ensemble).  The rest of the library lives beside this file: magprop_chain.cu (posterior
+// summaries of a chain), magprop_models.cu (reference restatements of the model) and magprop_device.cu (IPC, the
+// peer barrier, the FP64 peak, version and errors).  Only this file includes magprop_core.cuh, so the disc tables
+// are compiled into the library once.
 #include <cuda_runtime.h>
 
 #include <cstddef>
 #include <cstdio>
 #include <cstring>
 #include <map>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <vector>
 
 #include "magprop_host.hpp"
 #include "magprop_rng.cuh"
+#include "magprop_abi.hpp"
 
 namespace mp {
 
@@ -816,425 +821,6 @@ __global__ void pt_swap_kernel(double* __restrict__ coords, double* __restrict__
   }
 }
 
-// ---- cross-GPU flag barrier over peer-mapped memory ---------------------------------------------
-// Thread p of the one block: raise flag[rank] = epoch in peer p's array (a system-scope release, after the
-// preceding kernel's peer stores -- stream order plus the fence make them visible first), then spin on
-// this rank's own array until peer p has raised its flag (system-scope acquire).  The spin is on LOCAL
-// memory; the only NVLink traffic is one 8-byte store per peer.
-struct PeerFlags {
-  uint64_t* p[MP_MAX_PEERS + 1];
-};
-__global__ void peer_barrier_kernel(uint64_t* my_flags, PeerFlags pf, int rank, int world, uint64_t epoch, int* error) {
-  const int p = threadIdx.x;
-  if (p >= world || p == rank) return;
-  __threadfence_system();
-  asm volatile("st.release.sys.global.u64 [%0], %1;" ::"l"(pf.p[p] + rank), "l"(epoch) : "memory");
-  unsigned long long t0, t1;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t0));
-  for (;;) {
-    uint64_t v;
-    asm volatile("ld.acquire.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(my_flags + p) : "memory");
-    if (v >= epoch) break;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t1));
-    if (t1 - t0 > 10000000000ull) {   // 10 s: a peer died -- report instead of hanging the GPU
-      if (error) *error = 1;
-      break;
-    }
-    __nanosleep(200);
-  }
-}
-
-// ---- posterior summaries of a device-resident chain (plot_synth.py:150-166) -------------------------------
-// Column means and the centred cross-products (for np.corrcoef), and exact order statistics by radix select
-// (for np.percentile): the chain never leaves the device, the host receives a few dozen numbers.
-// No floating-point atomics: every block writes its partial sums to part[block][q], and a one-block finish kernel adds
-// them in block order -- the result depends only on n and ndim, so two calls on one chain agree bit for bit.
-constexpr int kMomBlocks = 1184, kMomThreads = 256;
-
-__global__ void chain_mean_kernel(const double* __restrict__ x, long long n, int ndim, double* __restrict__ part) {
-  __shared__ double sh[MP_MAX_NDIM][8];
-  double acc[MP_MAX_NDIM];
-  for (int d = 0; d < MP_MAX_NDIM; ++d) acc[d] = 0.0;
-  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
-    for (int d = 0; d < ndim; ++d) acc[d] += x[i * ndim + d];
-  const int lane = threadIdx.x & 31, wrp = threadIdx.x >> 5;
-  for (int d = 0; d < ndim; ++d) {
-    double v = acc[d];
-    for (int off = 16; off > 0; off >>= 1) v += __shfl_xor_sync(kFull, v, off);
-    if (lane == 0) sh[d][wrp] = v;
-  }
-  __syncthreads();
-  if (threadIdx.x < ndim) {
-    double v = 0.0;
-    for (int w = 0; w < (int)(blockDim.x >> 5); ++w) v += sh[threadIdx.x][w];
-    part[blockIdx.x * ndim + threadIdx.x] = v;
-  }
-}
-
-// mean[d] = (sum of the blocks' partials in block order) / n
-__global__ void chain_mean_finish_kernel(const double* __restrict__ part, int blocks, long long n, int ndim,
-                                         double* __restrict__ mean) {
-  const int d = threadIdx.x;
-  if (d >= ndim) return;
-  double v = 0.0;
-  for (int b = 0; b < blocks; ++b) v += part[b * ndim + d];
-  mean[d] = v / (double)n;
-}
-
-__global__ void chain_cov_kernel(const double* __restrict__ x, long long n, int ndim, const double* __restrict__ mean,
-                                 double* __restrict__ part /*[block][npair], pairs (a <= b) row by row*/) {
-  __shared__ double sh[MP_MAX_NDIM * MP_MAX_NDIM][8];
-  double acc[MP_MAX_NDIM * (MP_MAX_NDIM + 1) / 2];
-  const int npair = ndim * (ndim + 1) / 2;
-  for (int q = 0; q < npair; ++q) acc[q] = 0.0;
-  double mu[MP_MAX_NDIM];
-  for (int d = 0; d < ndim; ++d) mu[d] = mean[d];
-  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
-    double c[MP_MAX_NDIM];
-    for (int d = 0; d < ndim; ++d) c[d] = x[i * ndim + d] - mu[d];
-    int q = 0;
-    for (int a = 0; a < ndim; ++a)
-      for (int b = a; b < ndim; ++b, ++q) acc[q] = fma(c[a], c[b], acc[q]);
-  }
-  const int lane = threadIdx.x & 31, wrp = threadIdx.x >> 5;
-  for (int q = 0; q < npair; ++q) {
-    double v = acc[q];
-    for (int off = 16; off > 0; off >>= 1) v += __shfl_xor_sync(kFull, v, off);
-    if (lane == 0) sh[q][wrp] = v;
-  }
-  __syncthreads();
-  if (threadIdx.x < npair) {
-    double v = 0.0;
-    for (int w = 0; w < (int)(blockDim.x >> 5); ++w) v += sh[threadIdx.x][w];
-    part[blockIdx.x * npair + threadIdx.x] = v;
-  }
-}
-
-// cov[a][b] = cov[b][a] = (sum of the blocks' partials of pair (a, b) in block order) / max(n - 1, 1)
-__global__ void chain_cov_finish_kernel(const double* __restrict__ part, int blocks, long long n, int ndim,
-                                        double* __restrict__ cov) {
-  const int npair = ndim * (ndim + 1) / 2, q = threadIdx.x;
-  if (q >= npair) return;
-  int a = 0, r = q;
-  while (r >= ndim - a) {   // row a of the upper triangle holds pairs (a, a..ndim-1)
-    r -= ndim - a;
-    ++a;
-  }
-  const int b = a + r;
-  double v = 0.0;
-  for (int k = 0; k < blocks; ++k) v += part[k * npair + q];
-  v /= (double)(n > 1 ? n - 1 : 1);
-  cov[a * ndim + b] = v;
-  cov[b * ndim + a] = v;
-}
-
-// IEEE doubles as unsigned keys in ascending order: -inf < ... < -0 < +0 < ... < +inf < every NaN.  A NaN's sign bit
-// is dropped, so a NaN made with the sign bit set (0/0 on x86) sorts last too, as np.sort puts it.
-__device__ __forceinline__ unsigned long long order_key(double v) {
-  unsigned long long b = (unsigned long long)__double_as_longlong(v);
-  if ((b & 0x7fffffffffffffffull) > 0x7ff0000000000000ull) b &= 0x7fffffffffffffffull;
-  return (b >> 63) ? ~b : (b | 0x8000000000000000ull);
-}
-// One pass of the radix select on column `col`: histogram of the 16-bit digit at `shift` over the elements whose
-// higher digits equal those of `prefix`.  64-bit bins, so a column of 2^32 or more equal digits cannot wrap one.  The
-// lanes of a warp that fall in the same bin add to it once (match + popc): a chain's ties (stuck walkers, a long
-// constant column) otherwise serialise on one address.
-__global__ void select_hist_kernel(const double* __restrict__ x, long long n, int ndim, int col, unsigned long long prefix,
-                                   int shift, unsigned long long* __restrict__ hist) {
-  const unsigned long long himask = (shift >= 48) ? 0ull : (~0ull << (shift + 16));
-  const int lane = threadIdx.x & 31;
-  const long long stride = (long long)gridDim.x * blockDim.x;
-  // base is the warp's first row: the loop condition is uniform over the warp, so every lane reaches the match
-  for (long long base = blockIdx.x * (long long)blockDim.x + (threadIdx.x & ~31); base < n; base += stride) {
-    const long long i = base + lane;
-    unsigned bin = 0xffffffffu;                          // no bin: past the end, or another prefix
-    if (i < n) {
-      const unsigned long long key = order_key(x[i * ndim + col]);
-      if ((key & himask) == (prefix & himask)) bin = (unsigned)((key >> shift) & 0xffffull);
-    }
-    const unsigned peers = __match_any_sync(kFull, bin);
-    if (bin != 0xffffffffu && lane == __ffs(peers) - 1) atomicAdd(hist + bin, (unsigned long long)__popc(peers));
-  }
-}
-
-// ---- walker-averaged autocorrelation function of a device-resident chain (emcee's integrated_time) ---------------
-// The chain [n_steps][nwalkers][ndim] is read as [n_steps][J], J = nwalkers*ndim: series j = w*ndim + d is column j,
-// retained rows first + t*thin, t in [0, n).  Three launches, no floating-point atomics -- the result depends only on
-// the shapes and the SM count, so two calls on one chain agree bit for bit:
-//   acf_center_kernel  one thread per series: shift x0 = first retained sample, mean m of (x - x0), and
-//                      C(0) = sum_t s_t^2 of the centred series s_t = (x_t - x0) - m
-//   acf_lag_kernel     a block owns kAcfKB lags (kAcfKR per warp) of 32 consecutive series (one per lane) for a group
-//                      of such series tiles and a range of time chunks.  Per chunk of kAcfT anchor rows it stages the
-//                      centred rows [t0, t0+T) and [t0+kbase, t0+kbase+T+KB) in shared memory (row reads coalesced
-//                      along the walker axis); every thread accumulates C(k) of its series for its kAcfKR lags in
-//                      registers through a sliding window of 2*kAcfKR lagged samples (2 shared loads per kAcfKR FMAs).
-//                      C(k)/C(0) is then summed per dimension in lane order, and over the group's tiles in tile order.
-//   acf_finish_kernel  one thread per (d, k): the blocks' partials in a fixed order, / nwalkers
-constexpr int kAcfKR = 16, kAcfWarps = 8, kAcfKB = kAcfKR * kAcfWarps, kAcfT = 128;
-constexpr int kAcfNQ = (MP_MAX_NDIM * kAcfKB + 32 * kAcfWarps - 1) / (32 * kAcfWarps);
-constexpr size_t kAcfSmem = (size_t)(2 * kAcfT + kAcfKB) * 32 * sizeof(double);
-
-struct AcfShape {
-  const double* x;
-  long long J;                  // nwalkers * ndim
-  long long first, thin, n;     // retained rows first + t*thin, t < n
-  long long lag_begin, nl;      // lags [lag_begin, lag_begin + nl)
-  long long n_tiles, n_groups;  // 32-series tiles; block group g takes tiles g, g + n_groups, ...
-  int ndim, n_lb;               // lag blocks of kAcfKB
-  int cps, nsplit;              // time chunks per split, splits
-};
-
-__global__ void acf_center_kernel(const AcfShape a, double* __restrict__ x0, double* __restrict__ mu,
-                                  double* __restrict__ c0) {
-  const long long stride = a.thin * a.J;
-  for (long long j = blockIdx.x * (long long)blockDim.x + threadIdx.x; j < a.J; j += (long long)gridDim.x * blockDim.x) {
-    const double* col = a.x + a.first * a.J + j;
-    const double s0 = col[0];
-    double sum = 0.0;
-    for (long long t = 0; t < a.n; ++t) sum += col[t * stride] - s0;
-    const double m = sum / (double)a.n;
-    double ss = 0.0;
-    for (long long t = 0; t < a.n; ++t) {
-      const double s = (col[t * stride] - s0) - m;
-      ss = fma(s, s, ss);
-    }
-    x0[j] = s0;
-    mu[j] = m;
-    c0[j] = ss;
-  }
-}
-
-__global__ void __launch_bounds__(32 * kAcfWarps, 2) acf_lag_kernel(const AcfShape a, const double* __restrict__ x0,
-                                                                    const double* __restrict__ mu,
-                                                                    const double* __restrict__ c0,
-                                                                    double* __restrict__ part /*[item][ndim][kAcfKB]*/) {
-  extern __shared__ double acf_sm[];
-  double* sa = acf_sm;                    // [kAcfT][32]          anchor rows
-  double* sb = acf_sm + kAcfT * 32;       // [kAcfT + kAcfKB][32] lagged rows
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  long long item = blockIdx.x;            // = (g * n_lb + lb) * nsplit + split
-  const int split = (int)(item % a.nsplit);
-  item /= a.nsplit;
-  const int lb = (int)(item % a.n_lb);
-  const long long g = item / a.n_lb;
-  const long long kbase = a.lag_begin + (long long)lb * kAcfKB;
-  const long long n_chunks = (a.n + kAcfT - 1) / kAcfT;
-  const long long c_lo = (long long)split * a.cps, c_hi = min(c_lo + a.cps, n_chunks);
-  const long long rstride = a.thin * a.J;
-  const double* rows = a.x + a.first * a.J;
-  double racc[kAcfNQ];
-#pragma unroll
-  for (int q = 0; q < kAcfNQ; ++q) racc[q] = 0.0;
-
-  for (long long tile = g; tile < a.n_tiles; tile += a.n_groups) {
-    const long long j = tile * 32 + lane;
-    const bool live = j < a.J;
-    const double sx0 = live ? x0[j] : 0.0, smu = live ? mu[j] : 0.0;
-    double acc[kAcfKR];
-#pragma unroll
-    for (int r = 0; r < kAcfKR; ++r) acc[r] = 0.0;
-    for (long long c = c_lo; c < c_hi; ++c) {
-      const long long t0 = c * kAcfT;
-      if (t0 + kbase >= a.n) break;       // every pair of this and later chunks reaches past the last row
-      __syncthreads();
-      // centred samples; zero past the last retained row, so pairs (t, t+k) with t+k >= n add nothing
-      for (int r = warp; r < kAcfT; r += kAcfWarps) {
-        const long long t = t0 + r;
-        sa[r * 32 + lane] = (live && t < a.n) ? (rows[t * rstride + j] - sx0) - smu : 0.0;
-      }
-      for (int r = warp; r < kAcfT + kAcfKB; r += kAcfWarps) {
-        const long long t = t0 + kbase + r;
-        sb[r * 32 + lane] = (live && t < a.n) ? (rows[t * rstride + j] - sx0) - smu : 0.0;
-      }
-      __syncthreads();
-      // lag kbase + warp*kAcfKR + r of anchor tb + i is sb row tb + warp*kAcfKR + i + r
-      const double* bw = sb + warp * kAcfKR * 32 + lane;
-      double b[2 * kAcfKR];
-#pragma unroll
-      for (int q = 0; q < kAcfKR; ++q) b[q] = bw[q * 32];
-#pragma unroll 1
-      for (int tb = 0; tb < kAcfT; tb += kAcfKR) {
-#pragma unroll
-        for (int q = 0; q < kAcfKR; ++q) b[kAcfKR + q] = bw[(tb + kAcfKR + q) * 32];
-#pragma unroll
-        for (int i = 0; i < kAcfKR; ++i) {
-          const double av = sa[(tb + i) * 32 + lane];
-#pragma unroll
-          for (int r = 0; r < kAcfKR; ++r) acc[r] = fma(av, b[i + r], acc[r]);
-        }
-#pragma unroll
-        for (int q = 0; q < kAcfKR; ++q) b[q] = b[kAcfKR + q];
-      }
-    }
-    // C(k)/C(0) of the tile's series, summed per dimension: lanes l with (tile*32 + l) % ndim == d, in lane order.
-    // A constant series has C(0) = 0 and gives NaN, as emcee's formula does.
-    const double cz = live ? c0[j] : 1.0;
-    __syncthreads();
-#pragma unroll
-    for (int r = 0; r < kAcfKR; ++r) sa[(warp * kAcfKR + r) * 32 + lane] = live ? acc[r] / cz : 0.0;
-    __syncthreads();
-    const int d0 = (int)((tile * 32) % a.ndim);
-#pragma unroll
-    for (int qi = 0; qi < kAcfNQ; ++qi) {
-      const int q = threadIdx.x + qi * 32 * kAcfWarps;
-      if (q < a.ndim * kAcfKB) {
-        const int d = q / kAcfKB, kk = q % kAcfKB;
-        double v = 0.0;
-        for (int l = (d - d0 + a.ndim) % a.ndim; l < 32; l += a.ndim) v += sa[kk * 32 + l];
-        racc[qi] += v;
-      }
-    }
-  }
-#pragma unroll
-  for (int qi = 0; qi < kAcfNQ; ++qi) {
-    const int q = threadIdx.x + qi * 32 * kAcfWarps;
-    if (q < a.ndim * kAcfKB) part[blockIdx.x * (long long)(a.ndim * kAcfKB) + q] = racc[qi];
-  }
-}
-
-__global__ void acf_finish_kernel(const AcfShape a, const double* __restrict__ part, int nwalkers, double* __restrict__ out) {
-  const long long q = blockIdx.x * (long long)blockDim.x + threadIdx.x;
-  if (q >= a.ndim * a.nl) return;
-  const int d = (int)(q / a.nl);
-  const long long kl = q % a.nl;
-  const int lb = (int)(kl / kAcfKB), kk = (int)(kl % kAcfKB);
-  double v = 0.0;
-  for (long long g = 0; g < a.n_groups; ++g)
-    for (int s = 0; s < a.nsplit; ++s)
-      v += part[((g * a.n_lb + lb) * a.nsplit + s) * (a.ndim * kAcfKB) + d * kAcfKB + kk];
-  out[q] = v / (double)nwalkers;
-}
-
-// ---- the coupled right-hand side, as ODEs()/odes() return it -----------------------
-// funcs.py:75-142 / magnetar/funcs.py:33-101, operation order kept.
-__global__ void rhs_kernel(double inertia_factor, double mdot_factor, double breakup, int dipole_torque,
-                           const double* __restrict__ y, const double* __restrict__ t,
-                           const double* __restrict__ pars, double n, double alpha, double cs7, double k,
-                           int W, double* __restrict__ dydt) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= W) return;
-  const double Mdisc = y[2 * i], omega = y[2 * i + 1], tt = t[i];
-  const double B = pars[5 * i], MdiscI = pars[5 * i + 1], RdiscI = pars[5 * i + 2];
-  const double epsilon = pars[5 * i + 3], delta = pars[5 * i + 4];
-  const double inertia = inertia_factor * kM * (kR * kR);
-  const double Rdisc = RdiscI * 1.0e5;
-  const double tvisc = Rdisc / (alpha * cs7 * 1.0e7);
-  const double mu = 1.0e15 * B * (kR * kR * kR);
-  const double M0 = delta * MdiscI * kMsol;
-  const double tfb = epsilon * tvisc;
-  double Rm = pow(mu, 4.0 / 7.0) * pow(kGM, -1.0 / 7.0) * pow((mdot_factor * Mdisc) / tvisc, -2.0 / 7.0);
-  const double Rc = pow(kGM / (omega * omega), 1.0 / 3.0);
-  const double Rlc = kC / omega;
-  if (Rm >= k * Rlc) Rm = k * Rlc;
-  const double w = pow(Rm / Rc, 1.5);
-  const double x = kGM / (kR * (kC * kC));
-  const double modW = 0.6 * kM * (kC * kC) * (x / (1.0 - 0.5 * x));
-  const double rot_param = (0.5 * inertia * (omega * omega)) / modW;
-  double Ndip = (-1.0 * (mu * mu) * (omega * omega * omega)) / (6.0 * (kC * kC * kC));
-  if (dipole_torque) {                                  // figure_3.py:142-143
-    const double q = Rlc / Rm;
-    Ndip = (-2.0 / 3.0) * (((mu * mu) * (omega * omega * omega)) / (kC * kC * kC)) * (q * q * q);
-  }
-  const double eta2 = 0.5 * (1.0 + tanh(n * (w - 1.0)));
-  const double eta1 = 1.0 - eta2;
-  const double Mdotprop = eta2 * (Mdisc / tvisc);
-  const double Mdotacc = eta1 * (Mdisc / tvisc);
-  const double Mdotfb = (M0 / tfb) * pow((tt + tfb) / tfb, -5.0 / 3.0);
-  double Nacc;
-  if (rot_param > breakup) Nacc = 0.0;
-  else if (Rm >= kR) Nacc = sqrt(kGM * Rm) * (Mdotacc - Mdotprop);
-  else Nacc = sqrt(kGM * kR) * (Mdotacc - Mdotprop);
-  dydt[2 * i] = Mdotfb - Mdotacc - Mdotprop;
-  dydt[2 * i + 1] = (Nacc + Ndip) / inertia;
-}
-
-// ---- the comparison model of code/figure_5.py:222-363 ("Ben's model") --------------------------------------
-// An accreting-mass magnetar with an exponentially draining disc, advanced by explicit Euler steps of 1 s (the
-// reference: a Python loop over 1e6 array elements per parameter set).  One parameter set per thread, the script's
-// operation order kept (fractional powers through pow, as NumPy's **); every `stride`-th step is stored.
-// out [W][3][n_out] = Ltot, Lprop, Ldip in units of 1e50 erg/s (figure_5.py:354-368).
-__global__ void gompertz_kernel(const double* __restrict__ pars, int W, double alpha, double cs7, double k, double omass,
-                                double dipeff, double propeff, long long n_steps, int stride, long long n_out,
-                                double* __restrict__ out) {
-  const int wi = blockIdx.x * blockDim.x + threadIdx.x;
-  if (wi >= W) return;
-  const double B = pars[6 * wi], P = pars[6 * wi + 1], MdiscI = pars[6 * wi + 2], RdiscI = pars[6 * wi + 3];
-  const double spin = P * 1.0e-3;                               // :224
-  const double Rdisc = RdiscI * 1.0e5;
-  const double visc = alpha * cs7 * 1.0e7 * Rdisc;
-  const double mu = 1.0e15 * B * (kR * kR * kR);
-  double omega = (2.0 * 3.141592653589793) / spin;             // :229
-  const double Mdisc0 = MdiscI * kMsol;
-  double M_bg = omass * kMsol;
-  const double Mdot0 = (3.0 * Mdisc0 * visc) / (Rdisc * Rdisc);  // :258
-  double Mdot = Mdot0, Msum = 0.0, tt = 1.0, omegadot = 0.0;
-  const double mu47 = pow(mu, 4.0 / 7.0), mu2 = mu * mu, c3 = kC * kC * kC, c2 = kC * kC, R2 = kR * kR, R3 = kR * kR * kR;
-  double* o = out + (size_t)wi * 3 * n_out;
-  for (long long i = 0; i < n_steps; ++i) {
-    if (i > 0) {                                                // :302-309
-      tt = tt + 1.0;
-      omega = omega + omegadot;
-      M_bg = M_bg + Msum;
-      Mdot = Mdot0 * exp((-3.0 * visc * tt) / (Rdisc * Rdisc));
-    }
-    const double GMb = kG * M_bg;
-    double Rm = mu47 * pow(GMb, -1.0 / 7.0) * pow(Mdot, -2.0 / 7.0);
-    const double Rc = pow(GMb / (omega * omega), 1.0 / 3.0);
-    const double light = kC / omega;
-    if (Rm >= (k * light)) Rm = k * light;
-    const double lr = light / Rm;
-    const double Ndip = (-2.0 / 3.0) * ((mu2 * (omega * omega * omega)) / c3) * (lr * lr * lr);
-    const double w = pow(Rm / Rc, 1.5);
-    const double nn = 1.0 - w;
-    const double inertia = 0.35 * M_bg * R2;
-    const double bigT = 0.5 * inertia * (omega * omega);
-    const double x = GMb / (kR * c2);
-    const double modW = 0.6 * M_bg * c2 * (x / (1.0 - 0.5 * x));
-    const double beta = bigT / modW;
-    double Nacc;
-    if (beta > 0.27) {
-      Nacc = 0.0;
-    } else if (Rm >= kR) {
-      Nacc = nn * sqrt(GMb * Rm) * Mdot;
-      if (!isfinite(Nacc)) Nacc = 0.0;
-    } else {
-      const double f = 1.0 - (omega / sqrt(GMb / R3));
-      Nacc = (i == 0) ? f / sqrt(GMb * kR) * Mdot : f * sqrt(GMb * kR) * Mdot;   // (:283-285 divides, :335-337 multiplies)
-      if (!isfinite(Nacc)) Nacc = 0.0;
-    }
-    if (Rc >= Rm) Msum = Mdot;                                  // :293-296, :341-344
-    else if (i == 0) Msum = 0.0;
-    omegadot = (Ndip + Nacc) / inertia;
-    if (i % stride == 0) {
-      double lp = (-1.0 * Nacc * omega) - ((GMb * Mdot) / Rm);
-      double ld = (mu2 * ((omega * omega) * (omega * omega))) / (6.0 * c3);
-      if (!isfinite(lp) || lp <= 0.0) lp = 0.0;                 // :354-361
-      if (!isfinite(ld) || ld <= 0.0) ld = 0.0;
-      const long long jo = i / stride;
-      o[jo] = ((propeff * lp) + (dipeff * ld)) * 1.0e-50;
-      o[n_out + jo] = lp * 1.0e-50;
-      o[2 * n_out + jo] = ld * 1.0e-50;
-    }
-  }
-}
-
-// ---- FP64 FMA peak: 8 independent chains per thread, 2 flop per DFMA ---------------
-__global__ void __launch_bounds__(256) dfma_peak_kernel(double* out, int iters, double seed) {
-  double a0 = seed + threadIdx.x, a1 = a0 + 1, a2 = a0 + 2, a3 = a0 + 3, a4 = a0 + 4, a5 = a0 + 5, a6 = a0 + 6,
-         a7 = a0 + 7;
-  const double m = 0.9999999, c = 1e-9;
-#pragma unroll 1
-  for (int i = 0; i < iters; ++i) {
-#pragma unroll
-    for (int u = 0; u < 8; ++u) {
-      a0 = fma(a0, m, c); a1 = fma(a1, m, c); a2 = fma(a2, m, c); a3 = fma(a3, m, c);
-      a4 = fma(a4, m, c); a5 = fma(a5, m, c); a6 = fma(a6, m, c); a7 = fma(a7, m, c);
-    }
-  }
-  const double s = a0 + a1 + a2 + a3 + a4 + a5 + a6 + a7;
-  if (s == 12345.678) out[0] = s;  // keep the chains alive
-}
-
 }  // namespace mp
 
 // =====================================================================================
@@ -1242,20 +828,8 @@ __global__ void __launch_bounds__(256) dfma_peak_kernel(double* out, int iters, 
 // =====================================================================================
 using namespace mp;
 
-static thread_local std::string g_err;
-static int fail(int code, const std::string& msg) {
-  g_err = msg;
-  return code;
-}
-#define MP_CUDA(call)                                                                     \
-  do {                                                                                    \
-    cudaError_t e_ = (call);                                                              \
-    if (e_ != cudaSuccess)                                                                \
-      return fail(MP_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_));       \
-  } while (0)
-
 struct DeviceNodes {
-  double* node_t = nullptr;
+  DevBuf<double> node_t;
   int n_nodes = 0;
 };
 
@@ -1269,14 +843,13 @@ struct mp_handle {
   int D = 0;
   NodeProgram np;
   DeviceNodes data_nodes;
-  double *d_y = nullptr, *d_yerr = nullptr, *d_dx = nullptr, *d_Dx = nullptr;   // y/yerr, 1e-50/yerr, dx, dx/Dx (DataView)
-  int *d_lo = nullptr, *d_orig = nullptr;
+  DevBuf<double> d_y, d_yerr, d_dx, d_Dx;   // y/yerr, 1e-50/yerr, dx, dx/Dx (DataView)
+  DevBuf<int> d_lo, d_orig;
   // curve node sets per stride
   std::map<int, DeviceNodes> curve_nodes;
   // staging for the host-pointer entry points
-  double *s_theta = nullptr, *s_out = nullptr, *s_state = nullptr, *s_lnp = nullptr;
-  int *s_status = nullptr, *s_nrhs = nullptr, *s_cstatus = nullptr;
-  size_t cap_theta = 0, cap_out = 0, cap_state = 0, cap_w = 0, cap_cstatus = 0;
+  DevBuf<double> s_theta, s_out, s_state, s_lnp;
+  DevBuf<int> s_status, s_nrhs, s_cstatus;
   // A lane = a stream plus the work space the stages of a launch hand to one another.  The handle owns two
   // pipeline lanes so that the host-pointer entry points can overlap the H2D copy of one chunk with the
   // kernels of the previous one.  Device-pointer entry points run on the caller's stream, and every such
@@ -1284,18 +857,19 @@ struct mp_handle {
   // ensembles on one dataset, a device call next to an mp_lnprob_batch_async in flight -- never share work
   // space; calls on ONE stream are ordered by the stream.
   struct Lane {
-    cudaStream_t stream = nullptr;
-    unsigned long long* recs = nullptr;
-    double* ybuf = nullptr;
-    int *status = nullptr, *n_rhs = nullptr, *work = nullptr, *counters = nullptr, *key = nullptr, *hist = nullptr,
-        *slot_wid = nullptr;
-    StiffRec* squeue = nullptr;
-    double* prop = nullptr;
-    size_t cap_walkers = 0, cap_ybuf = 0, cap_prop = 0;
-    double* betas = nullptr;     // the ladder of the tempered half-steps on this lane, and its host copy
+    cudaStream_t stream = nullptr;   // the handle's own lanes only (a caller's stream is never kept here, nor destroyed)
+    DevBuf<unsigned long long> recs;   // kRecWords rows, each as long as the lane's capacity in walkers
+    DevBuf<double> ybuf, prop;
+    DevBuf<int> status, n_rhs, work, counters, key, hist, slot_wid;
+    DevBuf<StiffRec> squeue;
+    DevBuf<double> betas;        // the ladder of the tempered half-steps on this lane, and its host copy
     std::vector<double> betas_host;
     int* hint_host = nullptr;    // mapped pinned int[4]: counters[4..7] of the last large launch on this lane (see launch_eval)
     int* hint_dev = nullptr;     // the device's pointer to it
+    ~Lane() {
+      if (hint_host) cudaFreeHost(hint_host);
+      if (stream) cudaStreamDestroy(stream);
+    }
   } lanes[2];
   std::map<cudaStream_t, Lane> user_lanes;
   std::mutex user_lanes_mu;
@@ -1304,41 +878,6 @@ struct mp_handle {
   Lane* last_lane = nullptr;       // work space of the most recent launch (mp_last_stiff_count)
   int64_t kernels_launched = 0;    // evaluation-pipeline kernels launched through this handle so far (mp_kernels_launched)
 };
-
-template <typename T>
-static int upload(T** dst, const std::vector<T>& v) {
-  *dst = nullptr;
-  if (v.empty()) return MP_OK;
-  MP_CUDA(cudaMalloc((void**)dst, v.size() * sizeof(T)));
-  MP_CUDA(cudaMemcpy(*dst, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice));
-  return MP_OK;
-}
-
-// Grow-only device buffer.  (cudaFree waits for the device, so a buffer an earlier launch still uses is
-// released only after that launch has finished.)
-template <typename T>
-static int ensure(T** p, size_t* cap, size_t need) {
-  if (need <= *cap) return MP_OK;
-  if (*p) cudaFree(*p);
-  *p = nullptr;
-  *cap = 0;
-  MP_CUDA(cudaMalloc((void**)p, need * sizeof(T)));
-  *cap = need;
-  return MP_OK;
-}
-
-extern "C" int mp_abi_version(void) { return MP_ABI_VERSION; }
-
-extern "C" int mp_device_count(void) {
-  int n = 0;
-  if (cudaGetDeviceCount(&n) != cudaSuccess) {
-    cudaGetLastError();
-    return 0;
-  }
-  return n;
-}
-
-extern "C" const char* mp_last_error(void) { return g_err.c_str(); }
 
 extern "C" int mp_create(const mp_model_spec* spec, const mp_prior_spec* prior, const double* grid,
                          int32_t G, const double* t, const double* y, const double* yerr, int32_t D,
@@ -1351,10 +890,8 @@ extern "C" int mp_create(const mp_model_spec* spec, const mp_prior_spec* prior, 
   if (rc == MP_ERR_BAD_GRID) return fail(rc, "mp_create: grid must be strictly increasing with >= 2 nodes");
   if (rc == MP_ERR_DATA_RANGE)
     return fail(rc, "A value in x_new is outside the interpolation range.");
-  if (mp_device_count() <= device || device < 0)
-    return fail(MP_ERR_CUDA, "mp_create: no such CUDA device (magprop_b200 has no CPU path)");
-  MP_CUDA(cudaSetDevice(device));
-  mp_handle* h = new mp_handle();
+  if ((rc = select_device(device, "mp_create"))) return rc;
+  std::unique_ptr<mp_handle> h(new mp_handle());
   h->device = device;
   h->model = *spec;
   h->spec = make_spec(*spec);
@@ -1365,24 +902,21 @@ extern "C" int mp_create(const mp_model_spec* spec, const mp_prior_spec* prior, 
     cudaDeviceProp prop;
     if (cudaGetDeviceProperties(&prop, device) == cudaSuccess) h->sm_count = prop.multiProcessorCount;
   }
-  for (auto& L : h->lanes) {
-    if (cudaStreamCreateWithFlags(&L.stream, cudaStreamNonBlocking) != cudaSuccess) {
-      mp_destroy(h);
+  for (auto& L : h->lanes)
+    if (cudaStreamCreateWithFlags(&L.stream, cudaStreamNonBlocking) != cudaSuccess)
       return fail(MP_ERR_CUDA, "mp_create: stream creation failed");
-    }
-  }
   h->stream = h->lanes[0].stream;
   h->D = D;
   h->np = np;
   h->data_nodes.n_nodes = (int)np.node_t.size();
-  if ((rc = upload(&h->data_nodes.node_t, np.node_t)) || (rc = upload(&h->d_y, np.ys)) ||
-      (rc = upload(&h->d_yerr, np.c)) || (rc = upload(&h->d_dx, np.dx)) ||
-      (rc = upload(&h->d_Dx, np.w)) || (rc = upload(&h->d_lo, np.lo)) ||
-      (rc = upload(&h->d_orig, np.order))) {
-    mp_destroy(h);
-    return rc;
-  }
-  *out = h;
+  MP_CUDA(h->data_nodes.node_t.upload(np.node_t));
+  MP_CUDA(h->d_y.upload(np.ys));
+  MP_CUDA(h->d_yerr.upload(np.c));
+  MP_CUDA(h->d_dx.upload(np.dx));
+  MP_CUDA(h->d_Dx.upload(np.w));
+  MP_CUDA(h->d_lo.upload(np.lo));
+  MP_CUDA(h->d_orig.upload(np.order));
+  *out = h.release();
   return MP_OK;
 }
 
@@ -1390,21 +924,6 @@ extern "C" void mp_destroy(mp_handle* h) {
   if (!h) return;
   cudaSetDevice(h->device);
   cudaDeviceSynchronize();
-  cudaFree(h->data_nodes.node_t);
-  cudaFree(h->d_y); cudaFree(h->d_yerr); cudaFree(h->d_dx); cudaFree(h->d_Dx);
-  cudaFree(h->d_lo); cudaFree(h->d_orig);
-  for (auto& kv : h->curve_nodes) cudaFree(kv.second.node_t);
-  cudaFree(h->s_theta); cudaFree(h->s_out); cudaFree(h->s_state); cudaFree(h->s_lnp);
-  cudaFree(h->s_status); cudaFree(h->s_nrhs); cudaFree(h->s_cstatus);
-  auto free_lane = [](mp_handle::Lane& L) {
-    if (L.hint_host) cudaFreeHost(L.hint_host);
-    cudaFree(L.recs); cudaFree(L.ybuf); cudaFree(L.status); cudaFree(L.n_rhs); cudaFree(L.work);
-    cudaFree(L.counters); cudaFree(L.squeue); cudaFree(L.prop); cudaFree(L.key); cudaFree(L.hist); cudaFree(L.slot_wid);
-    cudaFree(L.betas);
-    if (L.stream) cudaStreamDestroy(L.stream);
-  };
-  for (auto& L : h->lanes) free_lane(L);
-  for (auto& kv : h->user_lanes) free_lane(kv.second);     // (their .stream is null: the streams are the callers')
   delete h;
 }
 
@@ -1423,16 +942,16 @@ static int fill_problem(mp_handle* h, Problem& p, const DeviceNodes& nodes, bool
   std::memset(&p, 0, sizeof(p));
   p.sp = h->spec;
   p.dv.n_nodes = nodes.n_nodes;
-  p.dv.node_t = nodes.node_t;
+  p.dv.node_t = nodes.node_t.get();
   p.dv.t_start = h->grid[0];
   if (with_data) {
     p.dv.n_data = h->D;
-    p.dv.dat_ys = h->d_y;
-    p.dv.dat_c = h->d_yerr;
-    p.dv.dat_dx = h->d_dx;
-    p.dv.dat_w = h->d_Dx;
-    p.dv.dat_lo = h->d_lo;
-    p.dat_orig = h->d_orig;
+    p.dv.dat_ys = h->d_y.get();
+    p.dv.dat_c = h->d_yerr.get();
+    p.dv.dat_dx = h->d_dx.get();
+    p.dv.dat_w = h->d_Dx.get();
+    p.dv.dat_lo = h->d_lo.get();
+    p.dat_orig = h->d_orig.get();
   }
   p.prior_enabled = use_prior ? h->prior.enabled : 0;
   for (int i = 0; i < MP_MAX_NDIM; ++i) {
@@ -1463,34 +982,30 @@ static int slab_walkers(int Nn) {
   return (int)std::min<size_t>(std::max<size_t>(n, 4096), (size_t)1 << 22);
 }
 
+// The lane's work space for a slab of S walkers.  Every array grows only, so the stride of recs is the lane's
+// capacity in walkers, which an earlier launch of more walkers may have made larger than S (see Work).
 static int ensure_work(mp_handle::Lane& L, int S, int Nn, int ndim_prop, Work& k) {
-  int rc = MP_OK;
-  if ((size_t)S > L.cap_walkers) {
-    cudaFree(L.recs); cudaFree(L.status); cudaFree(L.n_rhs); cudaFree(L.work); cudaFree(L.squeue); cudaFree(L.key); cudaFree(L.slot_wid);
-    L.recs = nullptr; L.status = L.n_rhs = L.work = L.key = L.slot_wid = nullptr; L.squeue = nullptr; L.cap_walkers = 0;
-    MP_CUDA(cudaMalloc((void**)&L.recs, (size_t)S * sizeof(WalkerRec)));      // kRecWords rows of S words
-    MP_CUDA(cudaMalloc((void**)&L.status, (size_t)S * sizeof(int)));
-    MP_CUDA(cudaMalloc((void**)&L.n_rhs, (size_t)S * sizeof(int)));
-    MP_CUDA(cudaMalloc((void**)&L.work, (size_t)S * sizeof(int)));
-    MP_CUDA(cudaMalloc((void**)&L.key, (size_t)S * sizeof(int)));
-    MP_CUDA(cudaMalloc((void**)&L.slot_wid, (size_t)S * sizeof(int)));
-    MP_CUDA(cudaMalloc((void**)&L.squeue, (size_t)S * sizeof(StiffRec)));
-    L.cap_walkers = (size_t)S;
+  MP_CUDA(L.recs.ensure((size_t)S * kRecWords));
+  MP_CUDA(L.status.ensure(S));
+  MP_CUDA(L.n_rhs.ensure(S));
+  MP_CUDA(L.work.ensure(S));
+  MP_CUDA(L.key.ensure(S));
+  MP_CUDA(L.slot_wid.ensure(S));
+  MP_CUDA(L.squeue.ensure(S));
+  if (!L.counters.get()) {             // [8..11]: what the host was told last (never reset)
+    MP_CUDA(L.counters.ensure(12));
+    MP_CUDA(cudaMemset(L.counters.get(), 0, 12 * sizeof(int)));
   }
-  if (!L.counters) {             // [8..11]: what the host was told last (never reset)
-    MP_CUDA(cudaMalloc((void**)&L.counters, 12 * sizeof(int)));
-    MP_CUDA(cudaMemset(L.counters, 0, 12 * sizeof(int)));
-  }
-  if (!L.hist) MP_CUDA(cudaMalloc((void**)&L.hist, (kOrderBuckets + 3) * sizeof(int)));
+  MP_CUDA(L.hist.ensure(kOrderBuckets + 3));
   if (!L.hint_host && cudaHostAlloc((void**)&L.hint_host, 4 * sizeof(int), cudaHostAllocMapped) == cudaSuccess) {
     std::memset(L.hint_host, 0, 4 * sizeof(int));
     if (cudaHostGetDevicePointer((void**)&L.hint_dev, L.hint_host, 0) != cudaSuccess) L.hint_dev = nullptr;
   }
-  if ((rc = ensure(&L.ybuf, &L.cap_ybuf, (size_t)S * Nn))) return rc;
-  if (ndim_prop > 0 && (rc = ensure(&L.prop, &L.cap_prop, (size_t)S * ndim_prop))) return rc;
-  k.stride = (int)L.cap_walkers;
-  k.recs = L.recs; k.ybuf = L.ybuf; k.status = L.status; k.n_rhs = L.n_rhs; k.work = L.work;
-  k.squeue = L.squeue; k.counters = L.counters;
+  MP_CUDA(L.ybuf.ensure((size_t)S * Nn));
+  if (ndim_prop > 0) MP_CUDA(L.prop.ensure((size_t)S * ndim_prop));
+  k.stride = (int)(L.recs.size() / kRecWords);
+  k.recs = L.recs.get(); k.ybuf = L.ybuf.get(); k.status = L.status.get(); k.n_rhs = L.n_rhs.get(); k.work = L.work.get();
+  k.squeue = L.squeue.get(); k.counters = L.counters.get();
   return MP_OK;
 }
 
@@ -1526,7 +1041,7 @@ static int launch_eval(mp_handle* h, const Problem& p, const double* d_theta, in
       if (ms.active) ms.active += i0;
       else if (ms.betas) ms.mover0 += i0;     // (a tempered slab may span temperatures: offset the mover, not the position)
       else ms.pos0 += i0;
-      ms.prop = Lp->prop;
+      ms.prop = Lp->prop.get();
       if (ms.pack_out) ms.pack_out += (size_t)i0 * (ndim + 1);
     }
     Sink sk = sink;
@@ -1550,9 +1065,9 @@ static int launch_eval(mp_handle* h, const Problem& p, const double* d_theta, in
       if (e0 > 0 && e0 + e1 - 257 <= kTightMdBins && e2 + e3 - 33 <= kTightEpsBins) ordered = false;
     }
     const double* th0 = MOVE ? nullptr : d_theta + (size_t)i0 * ndim;
-    k.key = Lp->key;
-    k.hist = Lp->hist;
-    k.slot_wid = ordered ? Lp->slot_wid : nullptr;
+    k.key = Lp->key.get();
+    k.hist = Lp->hist.get();
+    k.slot_wid = ordered ? Lp->slot_wid.get() : nullptr;
     if (ordered) {
       // slots in key order: keys + histogram (MOVE: and the proposals), scan, scatter -- then the setup runs per slot
       MP_CUDA(cudaMemsetAsync(k.hist, 0, (kOrderBuckets + 3) * sizeof(int), stream));
@@ -1611,38 +1126,37 @@ extern "C" int mp_lnprob_batch_async(mp_handle* h, const double* theta, int32_t 
   if (ndim < 6 || ndim > MP_MAX_NDIM) return fail(MP_ERR_BAD_ARG, "ndim must be 6, 7, 8 or 9");
   if (W == 0) return MP_OK;
   MP_CUDA(cudaSetDevice(h->device));
-  int rc;
-  if ((rc = ensure(&h->s_theta, &h->cap_theta, (size_t)W * MP_MAX_NDIM))) return rc;
-  if (W > (int)h->cap_w) {
-    cudaFree(h->s_lnp); cudaFree(h->s_status); cudaFree(h->s_nrhs);
-    h->s_lnp = nullptr; h->s_status = nullptr; h->s_nrhs = nullptr; h->cap_w = 0;
-    MP_CUDA(cudaMalloc((void**)&h->s_lnp, (size_t)W * sizeof(double)));
-    MP_CUDA(cudaMalloc((void**)&h->s_status, (size_t)W * sizeof(int)));
-    MP_CUDA(cudaMalloc((void**)&h->s_nrhs, (size_t)W * sizeof(int)));
-    h->cap_w = W;
-  }
+  MP_CUDA(h->s_theta.ensure((size_t)W * MP_MAX_NDIM));
+  MP_CUDA(h->s_lnp.ensure(W));
+  MP_CUDA(h->s_status.ensure(W));
+  MP_CUDA(h->s_nrhs.ensure(W));
+  double* const s_theta = h->s_theta.get();
+  double* const s_lnp = h->s_lnp.get();
+  int* const s_status = h->s_status.get();
+  int* const s_nrhs = h->s_nrhs.get();
   // Large batches go through in chunks of a few waves on two alternating lanes: the H2D copy of chunk
   // k+1 and the D2H copy of chunk k-1 overlap the kernels of chunk k (when the caller's buffers are
   // pinned; pageable buffers still work, the copies just serialise).
   const int wave = 4 * wave_walkers(h);
   const int chunk = (W <= wave + wave / 2) ? W : wave;
   Problem p;
-  if ((rc = fill_problem(h, p, h->data_nodes, true, ndim, W, true))) return rc;
+  int rc = fill_problem(h, p, h->data_nodes, true, ndim, W, true);
+  if (rc) return rc;
   int k = 0;
   for (int c0 = 0; c0 < W; c0 += chunk, ++k) {
     const int lane = k & 1;
     cudaStream_t st = h->lanes[lane].stream;
     int n = W - c0;
     if (n > chunk + chunk / 2) n = chunk;          // the last chunk absorbs a remainder below half a chunk
-    MP_CUDA(cudaMemcpyAsync(h->s_theta + (size_t)c0 * ndim, theta + (size_t)c0 * ndim, (size_t)n * ndim * sizeof(double),
+    MP_CUDA(cudaMemcpyAsync(s_theta + (size_t)c0 * ndim, theta + (size_t)c0 * ndim, (size_t)n * ndim * sizeof(double),
                             cudaMemcpyHostToDevice, st));
-    if ((rc = launch_eval<kModeLnprob, false>(h, p, h->s_theta + (size_t)c0 * ndim, n,
-                                              Sink{h->s_lnp + c0, h->s_status + c0, h->s_nrhs + c0}, nullptr, nullptr, nullptr,
+    if ((rc = launch_eval<kModeLnprob, false>(h, p, s_theta + (size_t)c0 * ndim, n,
+                                              Sink{s_lnp + c0, s_status + c0, s_nrhs + c0}, nullptr, nullptr, nullptr,
                                               st, lane)))
       return rc;
-    MP_CUDA(cudaMemcpyAsync(lnp + c0, h->s_lnp + c0, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (status) MP_CUDA(cudaMemcpyAsync(status + c0, h->s_status + c0, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, st));
-    if (n_rhs) MP_CUDA(cudaMemcpyAsync(n_rhs + c0, h->s_nrhs + c0, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, st));
+    MP_CUDA(cudaMemcpyAsync(lnp + c0, s_lnp + c0, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (status) MP_CUDA(cudaMemcpyAsync(status + c0, s_status + c0, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, st));
+    if (n_rhs) MP_CUDA(cudaMemcpyAsync(n_rhs + c0, s_nrhs + c0, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, st));
     if (n != chunk) break;
   }
   return MP_OK;
@@ -1673,15 +1187,15 @@ extern "C" int mp_model_at_data(mp_handle* h, const double* pars, int32_t W, int
   int rc = fill_problem(h, p, h->data_nodes, true, ndim, W, false);
   if (rc) return rc;
   p.sp.unlog_mask = 0;  // model_lum takes physical parameters
-  if ((rc = ensure(&h->s_theta, &h->cap_theta, (size_t)W * MP_MAX_NDIM))) return rc;
-  if ((rc = ensure(&h->s_out, &h->cap_out, (size_t)W * h->D))) return rc;
-  if ((rc = ensure(&h->s_cstatus, &h->cap_cstatus, (size_t)W))) return rc;
-  MP_CUDA(cudaMemcpyAsync(h->s_theta, pars, (size_t)W * ndim * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-  if ((rc = launch_eval<kModeModelAtData, false>(h, p, h->s_theta, W, Sink{nullptr, h->s_cstatus, nullptr}, h->s_out, nullptr,
-                                                 nullptr, h->stream, 0)))
+  MP_CUDA(h->s_theta.ensure((size_t)W * MP_MAX_NDIM));
+  MP_CUDA(h->s_out.ensure((size_t)W * h->D));
+  MP_CUDA(h->s_cstatus.ensure(W));
+  MP_CUDA(cudaMemcpyAsync(h->s_theta.get(), pars, (size_t)W * ndim * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+  if ((rc = launch_eval<kModeModelAtData, false>(h, p, h->s_theta.get(), W, Sink{nullptr, h->s_cstatus.get(), nullptr},
+                                                 h->s_out.get(), nullptr, nullptr, h->stream, 0)))
     return rc;
-  MP_CUDA(cudaMemcpyAsync(out, h->s_out, (size_t)W * h->D * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-  if (status) MP_CUDA(cudaMemcpyAsync(status, h->s_cstatus, (size_t)W * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+  MP_CUDA(cudaMemcpyAsync(out, h->s_out.get(), (size_t)W * h->D * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  if (status) MP_CUDA(cudaMemcpyAsync(status, h->s_cstatus.get(), (size_t)W * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
   MP_CUDA(cudaStreamSynchronize(h->stream));
   return MP_OK;
 }
@@ -1695,9 +1209,8 @@ static int curve_node_set(mp_handle* h, int stride, DeviceNodes** out) {
     build_curve_nodes(h->grid.data(), (int)h->grid.size(), stride, nt, gi);
     DeviceNodes dn;
     dn.n_nodes = (int)nt.size();
-    int rc = upload(&dn.node_t, nt);
-    if (rc) return rc;
-    it = h->curve_nodes.emplace(stride, dn).first;
+    MP_CUDA(dn.node_t.upload(nt));
+    it = h->curve_nodes.emplace(stride, std::move(dn)).first;
   }
   *out = &it->second;
   return MP_OK;
@@ -1738,50 +1251,25 @@ extern "C" int mp_model_curves(mp_handle* h, const double* pars, int32_t W, int3
   if (W == 0) return MP_OK;
   MP_CUDA(cudaSetDevice(h->device));
   const size_t Gs = (size_t)mp_curve_nodes(h, node_stride);
-  int rc;
-  if ((rc = ensure(&h->s_theta, &h->cap_theta, (size_t)W * MP_MAX_NDIM))) return rc;
-  if ((rc = ensure(&h->s_out, &h->cap_out, (size_t)W * 3 * Gs))) return rc;
-  if (state && (rc = ensure(&h->s_state, &h->cap_state, (size_t)W * 2 * Gs))) return rc;
+  MP_CUDA(h->s_theta.ensure((size_t)W * MP_MAX_NDIM));
+  MP_CUDA(h->s_out.ensure((size_t)W * 3 * Gs));
+  if (state) MP_CUDA(h->s_state.ensure((size_t)W * 2 * Gs));
   int* d_status = nullptr;
   if (status) {
-    if ((rc = ensure(&h->s_cstatus, &h->cap_cstatus, (size_t)W))) return rc;
-    d_status = h->s_cstatus;
+    MP_CUDA(h->s_cstatus.ensure(W));
+    d_status = h->s_cstatus.get();
   }
-  MP_CUDA(cudaMemcpyAsync(h->s_theta, pars, (size_t)W * ndim * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-  rc = curves_on(h, h->s_theta, W, ndim, node_stride, h->s_out, state ? h->s_state : nullptr, d_status, h->stream, 0);
+  MP_CUDA(cudaMemcpyAsync(h->s_theta.get(), pars, (size_t)W * ndim * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+  int rc = curves_on(h, h->s_theta.get(), W, ndim, node_stride, h->s_out.get(), state ? h->s_state.get() : nullptr, d_status,
+                     h->stream, 0);
   if (!rc) {
-    cudaMemcpyAsync(out, h->s_out, (size_t)W * 3 * Gs * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
-    if (state) cudaMemcpyAsync(state, h->s_state, (size_t)W * 2 * Gs * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
+    cudaMemcpyAsync(out, h->s_out.get(), (size_t)W * 3 * Gs * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
+    if (state) cudaMemcpyAsync(state, h->s_state.get(), (size_t)W * 2 * Gs * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
     if (status) cudaMemcpyAsync(status, d_status, (size_t)W * sizeof(int), cudaMemcpyDeviceToHost, h->stream);
     cudaError_t e = cudaStreamSynchronize(h->stream);
     if (e != cudaSuccess) rc = fail(MP_ERR_CUDA, std::string("mp_model_curves: ") + cudaGetErrorString(e));
   }
   return rc;
-}
-
-extern "C" int mp_rhs_batch(const mp_model_spec* spec, const double* y, const double* t, const double* pars,
-                            const double* knobs, int32_t W, double* dydt, int32_t device) {
-  if (!spec || !y || !t || !pars || !knobs || !dydt || W < 0) return fail(MP_ERR_BAD_ARG, "mp_rhs_batch: null pointer");
-  if (W == 0) return MP_OK;
-  if (mp_device_count() <= device || device < 0)
-    return fail(MP_ERR_CUDA, "mp_rhs_batch: no such CUDA device (magprop_b200 has no CPU path)");
-  MP_CUDA(cudaSetDevice(device));
-  // one allocation for the four arrays (y[2W] t[W] pars[5W] dydt[2W]), released on every path
-  double* d_all = nullptr;
-  MP_CUDA(cudaMalloc((void**)&d_all, (size_t)W * 10 * sizeof(double)));
-  double *d_y = d_all, *d_t = d_all + (size_t)2 * W, *d_p = d_all + (size_t)3 * W, *d_o = d_all + (size_t)8 * W;
-  cudaError_t e = cudaMemcpy(d_y, y, (size_t)W * 2 * sizeof(double), cudaMemcpyHostToDevice);
-  if (e == cudaSuccess) e = cudaMemcpy(d_t, t, (size_t)W * sizeof(double), cudaMemcpyHostToDevice);
-  if (e == cudaSuccess) e = cudaMemcpy(d_p, pars, (size_t)W * 5 * sizeof(double), cudaMemcpyHostToDevice);
-  if (e == cudaSuccess) {
-    rhs_kernel<<<(W + 127) / 128, 128>>>(spec->inertia_factor, spec->mdot_factor, spec->breakup_rhs, spec->dipole_torque, d_y, d_t, d_p,
-                                         knobs[0], knobs[1], knobs[2], knobs[3], W, d_o);
-    e = cudaGetLastError();
-  }
-  if (e == cudaSuccess) e = cudaMemcpy(dydt, d_o, (size_t)W * 2 * sizeof(double), cudaMemcpyDeviceToHost);
-  cudaFree(d_all);
-  if (e != cudaSuccess) return fail(MP_ERR_CUDA, std::string("mp_rhs_batch: ") + cudaGetErrorString(e));
-  return MP_OK;
 }
 
 static int fill_move_problem(mp_handle* h, Problem& p, int ndim, int n_active) {
@@ -1923,9 +1411,9 @@ static int check_tempered(const mp_ensemble* e, int32_t ntemps, const double* be
 // The ladder a lane's tempered half-steps read: copied in stream order, and only when it differs from the last one.
 static int upload_ladder(mp_handle::Lane& L, int ntemps, const double* betas, cudaStream_t stream) {
   if (L.betas_host.size() == (size_t)ntemps && std::equal(betas, betas + ntemps, L.betas_host.begin())) return MP_OK;
-  if (!L.betas) MP_CUDA(cudaMalloc((void**)&L.betas, MP_MAX_TEMPS * sizeof(double)));
+  MP_CUDA(L.betas.ensure(MP_MAX_TEMPS));
   L.betas_host.clear();
-  MP_CUDA(cudaMemcpyAsync(L.betas, betas, (size_t)ntemps * sizeof(double), cudaMemcpyHostToDevice, stream));
+  MP_CUDA(cudaMemcpyAsync(L.betas.get(), betas, (size_t)ntemps * sizeof(double), cudaMemcpyHostToDevice, stream));
   L.betas_host.assign(betas, betas + ntemps);
   return MP_OK;
 }
@@ -1948,7 +1436,7 @@ extern "C" int mp_tempered_half_step(mp_handle* h, const mp_ensemble* e, int32_t
   fill_ensemble_move(e, step, split, m);
   m.rank = 0;
   m.half = m.n_mine = half;
-  m.betas = L->betas;
+  m.betas = L->betas.get();
   return launch_eval<kModeLnprob, true>(h, p, nullptr, n_movers, Sink{nullptr, nullptr, nullptr}, nullptr, nullptr, &m, s);
 }
 
@@ -1986,245 +1474,12 @@ extern "C" int mp_ensemble_order(int32_t nwalkers, uint64_t seed, uint64_t step,
   return MP_OK;
 }
 
-// ---- peer-mapped replicas (CUDA IPC) -------------------------------------------------------------
-static_assert(sizeof(cudaIpcMemHandle_t) == 64, "the C ABI carries IPC handles as 64 bytes");
-
-extern "C" int mp_peer_alloc(int32_t device, uint64_t bytes, void** d_ptr, unsigned char handle[64]) {
-  if (!d_ptr || !handle || bytes == 0) return fail(MP_ERR_BAD_ARG, "mp_peer_alloc: bad argument");
-  if (mp_device_count() <= device || device < 0) return fail(MP_ERR_CUDA, "mp_peer_alloc: no such CUDA device");
-  MP_CUDA(cudaSetDevice(device));
-  void* p = nullptr;
-  MP_CUDA(cudaMalloc(&p, bytes));
-  cudaError_t e = cudaMemset(p, 0, bytes);
-  cudaIpcMemHandle_t hd;
-  if (e == cudaSuccess) e = cudaIpcGetMemHandle(&hd, p);
-  if (e != cudaSuccess) {
-    cudaFree(p);
-    return fail(MP_ERR_CUDA, std::string("mp_peer_alloc: ") + cudaGetErrorString(e));
-  }
-  std::memcpy(handle, &hd, 64);
-  *d_ptr = p;
-  return MP_OK;
-}
-
-extern "C" int mp_peer_open(int32_t device, const unsigned char handle[64], void** d_ptr) {
-  if (!d_ptr || !handle) return fail(MP_ERR_BAD_ARG, "mp_peer_open: null pointer");
-  MP_CUDA(cudaSetDevice(device));
-  cudaIpcMemHandle_t hd;
-  std::memcpy(&hd, handle, 64);
-  MP_CUDA(cudaIpcOpenMemHandle(d_ptr, hd, cudaIpcMemLazyEnablePeerAccess));
-  return MP_OK;
-}
-
-extern "C" int mp_peer_close(int32_t device, void* d_ptr) {
-  if (!d_ptr) return MP_OK;
-  MP_CUDA(cudaSetDevice(device));
-  MP_CUDA(cudaIpcCloseMemHandle(d_ptr));
-  return MP_OK;
-}
-
-extern "C" int mp_peer_free(int32_t device, void* d_ptr) {
-  if (!d_ptr) return MP_OK;
-  MP_CUDA(cudaSetDevice(device));
-  MP_CUDA(cudaFree(d_ptr));
-  return MP_OK;
-}
-
-extern "C" int mp_peer_barrier(int32_t device, uint64_t* d_my_flags, uint64_t* const* peer_flags, int32_t rank,
-                               int32_t world, uint64_t epoch, int32_t* d_error, void* stream) {
-  if (!d_my_flags || !peer_flags || world < 1 || world > MP_MAX_PEERS + 1 || rank < 0 || rank >= world)
-    return fail(MP_ERR_BAD_ARG, "mp_peer_barrier: bad argument");
-  if (world == 1) return MP_OK;
-  MP_CUDA(cudaSetDevice(device));
-  PeerFlags pf;
-  std::memset(&pf, 0, sizeof(pf));
-  for (int p = 0; p < world; ++p) {
-    if (p != rank && !peer_flags[p]) return fail(MP_ERR_BAD_ARG, "mp_peer_barrier: null peer flag array");
-    pf.p[p] = peer_flags[p];
-  }
-  peer_barrier_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(d_my_flags, pf, rank, world, epoch, d_error);
-  MP_CUDA(cudaGetLastError());
-  return MP_OK;
-}
-
-// ---- posterior summaries on the device ---------------------------------------------------------------------
-extern "C" int mp_chain_moments(const double* d_chain, int64_t n, int32_t ndim, double* mean, double* cov, int32_t device,
-                                void* stream) {
-  if (!d_chain || !mean || !cov || n < 1 || ndim < 1 || ndim > MP_MAX_NDIM) return fail(MP_ERR_BAD_ARG, "mp_chain_moments: bad argument");
-  if (mp_device_count() <= device || device < 0) return fail(MP_ERR_CUDA, "mp_chain_moments: no such CUDA device");
-  MP_CUDA(cudaSetDevice(device));
-  cudaStream_t st = (cudaStream_t)stream;
-  const int blocks = (int)std::min<int64_t>((n + kMomThreads - 1) / kMomThreads, kMomBlocks);
-  const int npair = ndim * (ndim + 1) / 2;
-  const size_t n_out = (size_t)ndim + (size_t)ndim * ndim;
-  double* d_buf = nullptr;
-  MP_CUDA(cudaMallocAsync((void**)&d_buf, (n_out + (size_t)blocks * npair) * sizeof(double), st));
-  double *d_mean = d_buf, *d_cov = d_mean + ndim, *d_part = d_cov + (size_t)ndim * ndim;   // part: [blocks][ndim or npair]
-  chain_mean_kernel<<<blocks, kMomThreads, 0, st>>>(d_chain, n, ndim, d_part);
-  chain_mean_finish_kernel<<<1, 32, 0, st>>>(d_part, blocks, n, ndim, d_mean);
-  chain_cov_kernel<<<blocks, kMomThreads, 0, st>>>(d_chain, n, ndim, d_mean, d_part);
-  chain_cov_finish_kernel<<<1, 64, 0, st>>>(d_part, blocks, n, ndim, d_cov);
-  std::vector<double> h(n_out);
-  cudaError_t e = cudaGetLastError();
-  if (e == cudaSuccess) e = cudaMemcpyAsync(h.data(), d_buf, n_out * sizeof(double), cudaMemcpyDeviceToHost, st);
-  const cudaError_t ef = cudaFreeAsync(d_buf, st);
-  if (e == cudaSuccess) e = ef;
-  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-  if (e != cudaSuccess) return fail(MP_ERR_CUDA, std::string("mp_chain_moments: ") + cudaGetErrorString(e));
-  std::memcpy(mean, h.data(), ndim * sizeof(double));
-  std::memcpy(cov, h.data() + ndim, (size_t)ndim * ndim * sizeof(double));
-  return MP_OK;
-}
-
-extern "C" int mp_chain_order_statistics(const double* d_chain, int64_t n, int32_t ndim, int32_t col, const int64_t* ranks,
-                                         int32_t n_ranks, double* values, int32_t device, void* stream) {
-  if (!d_chain || !ranks || !values || n < 1 || ndim < 1 || col < 0 || col >= ndim || n_ranks < 0)
-    return fail(MP_ERR_BAD_ARG, "mp_chain_order_statistics: bad argument");
-  for (int r = 0; r < n_ranks; ++r)
-    if (ranks[r] < 0 || ranks[r] >= n) return fail(MP_ERR_BAD_ARG, "mp_chain_order_statistics: rank outside [0, n)");
-  if (mp_device_count() <= device || device < 0) return fail(MP_ERR_CUDA, "mp_chain_order_statistics: no such CUDA device");
-  MP_CUDA(cudaSetDevice(device));
-  cudaStream_t st = (cudaStream_t)stream;
-  unsigned long long* d_hist = nullptr;
-  MP_CUDA(cudaMallocAsync((void**)&d_hist, 65536 * sizeof(unsigned long long), st));
-  std::vector<unsigned long long> hist(65536);
-  const int blocks = (int)std::min<int64_t>((n + 255) / 256, 1184);
-  cudaError_t e = cudaSuccess;
-  for (int r = 0; r < n_ranks && e == cudaSuccess; ++r) {
-    unsigned long long k = (unsigned long long)ranks[r];
-    unsigned long long prefix = 0ull;
-    for (int shift = 48; shift >= 0; shift -= 16) {
-      e = cudaMemsetAsync(d_hist, 0, 65536 * sizeof(unsigned long long), st);
-      if (e == cudaSuccess) {
-        select_hist_kernel<<<blocks, 256, 0, st>>>(d_chain, n, ndim, col, prefix, shift, d_hist);
-        e = cudaGetLastError();
-      }
-      if (e == cudaSuccess)
-        e = cudaMemcpyAsync(hist.data(), d_hist, 65536 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st);
-      if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-      if (e != cudaSuccess) break;
-      unsigned digit = 0;
-      for (; digit < 65535u && k >= hist[digit]; ++digit) k -= hist[digit];
-      prefix |= (unsigned long long)digit << shift;
-    }
-    // key -> double
-    const unsigned long long b = (prefix >> 63) ? (prefix & 0x7fffffffffffffffull) : ~prefix;
-    std::memcpy(values + r, &b, sizeof(double));
-  }
-  const cudaError_t ef = cudaFreeAsync(d_hist, st);
-  if (e == cudaSuccess) e = ef;
-  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-  if (e != cudaSuccess) return fail(MP_ERR_CUDA, std::string("mp_chain_order_statistics: ") + cudaGetErrorString(e));
-  return MP_OK;
-}
-
-extern "C" int mp_chain_autocorr(const double* d_chain, int64_t n_steps, int32_t nwalkers, int32_t ndim, int64_t first,
-                                 int64_t thin, int64_t lag_begin, int64_t lag_end, double* acf, int32_t device, void* stream) {
-  if (!d_chain || !acf || nwalkers < 1 || ndim < 1 || ndim > MP_MAX_NDIM || thin < 1 || first < 0 || first >= n_steps ||
-      lag_begin < 0 || lag_end <= lag_begin)
-    return fail(MP_ERR_BAD_ARG, "mp_chain_autocorr: bad argument");
-  const int64_t n = (n_steps - first + thin - 1) / thin;
-  if (lag_end > n) return fail(MP_ERR_BAD_ARG, "mp_chain_autocorr: lag_end exceeds the number of retained rows");
-  if (mp_device_count() <= device || device < 0) return fail(MP_ERR_CUDA, "mp_chain_autocorr: no such CUDA device");
-  MP_CUDA(cudaSetDevice(device));
-  int sms = 0;
-  MP_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
-  MP_CUDA(cudaFuncSetAttribute(acf_lag_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kAcfSmem));
-  cudaStream_t st = (cudaStream_t)stream;
-
-  AcfShape a;
-  a.x = d_chain;
-  a.J = (long long)nwalkers * ndim;
-  a.first = first, a.thin = thin, a.n = n;
-  a.lag_begin = lag_begin, a.nl = lag_end - lag_begin;
-  a.ndim = ndim;
-  a.n_lb = (int)((a.nl + kAcfKB - 1) / kAcfKB);
-  a.n_tiles = (a.J + 31) / 32;
-  // One wave of acf_lag_kernel (two blocks per SM): tiles are dealt out over the blocks; when there are fewer tiles x lag
-  // blocks than that (few walkers), the time axis is split as well and the splits' partials are summed by the last pass.
-  const long long wave = 2LL * sms;
-  const long long n_chunks = (n + kAcfT - 1) / kAcfT;
-  a.n_groups = std::min<long long>(a.n_tiles, std::max<long long>(1, wave / a.n_lb));
-  long long nsplit = 1;
-  if (a.n_groups == a.n_tiles) nsplit = std::min<long long>(n_chunks, std::max<long long>(1, wave / (a.n_tiles * a.n_lb)));
-  a.cps = (int)((n_chunks + nsplit - 1) / nsplit);
-  a.nsplit = (int)((n_chunks + a.cps - 1) / a.cps);
-  const long long items = a.n_groups * a.n_lb * a.nsplit;
-
-  const size_t n_part = (size_t)items * ndim * kAcfKB, n_out = (size_t)ndim * a.nl;
-  double* d_buf = nullptr;
-  MP_CUDA(cudaMallocAsync((void**)&d_buf, (3 * (size_t)a.J + n_part + n_out) * sizeof(double), st));
-  double *d_x0 = d_buf, *d_mu = d_x0 + a.J, *d_c0 = d_mu + a.J, *d_part = d_c0 + a.J, *d_out = d_part + n_part;
-  acf_center_kernel<<<(int)std::min<long long>((a.J + 255) / 256, 8LL * sms), 256, 0, st>>>(a, d_x0, d_mu, d_c0);
-  acf_lag_kernel<<<(unsigned)items, 32 * kAcfWarps, kAcfSmem, st>>>(a, d_x0, d_mu, d_c0, d_part);
-  acf_finish_kernel<<<(unsigned)((n_out + 255) / 256), 256, 0, st>>>(a, d_part, nwalkers, d_out);
-  cudaError_t e = cudaGetLastError();
-  if (e == cudaSuccess) e = cudaMemcpyAsync(acf, d_out, n_out * sizeof(double), cudaMemcpyDeviceToHost, st);
-  const cudaError_t ef = cudaFreeAsync(d_buf, st);
-  if (e == cudaSuccess) e = ef;
-  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-  if (e != cudaSuccess) return fail(MP_ERR_CUDA, std::string("mp_chain_autocorr: ") + cudaGetErrorString(e));
-  return MP_OK;
-}
-
-extern "C" int mp_gompertz_curves(const double* pars, int32_t W, const double* knobs, int64_t n_steps, int32_t stride,
-                                  double* out, int32_t device) {
-  if (!pars || !knobs || !out || W < 0 || n_steps < 1 || stride < 1) return fail(MP_ERR_BAD_ARG, "mp_gompertz_curves: bad argument");
-  if (W == 0) return MP_OK;
-  if (mp_device_count() <= device || device < 0)
-    return fail(MP_ERR_CUDA, "mp_gompertz_curves: no such CUDA device (magprop_b200 has no CPU path)");
-  MP_CUDA(cudaSetDevice(device));
-  const long long n_out = (n_steps + stride - 1) / stride;
-  double *d_p = nullptr, *d_o = nullptr;
-  MP_CUDA(cudaMalloc((void**)&d_p, (size_t)W * 6 * sizeof(double)));
-  cudaError_t e = cudaMalloc((void**)&d_o, (size_t)W * 3 * n_out * sizeof(double));
-  if (e == cudaSuccess) e = cudaMemcpy(d_p, pars, (size_t)W * 6 * sizeof(double), cudaMemcpyHostToDevice);
-  if (e == cudaSuccess) {
-    gompertz_kernel<<<(W + 31) / 32, 32>>>(d_p, W, knobs[0], knobs[1], knobs[2], knobs[3], knobs[4], knobs[5], n_steps, stride, n_out, d_o);
-    e = cudaGetLastError();
-  }
-  if (e == cudaSuccess) e = cudaMemcpy(out, d_o, (size_t)W * 3 * n_out * sizeof(double), cudaMemcpyDeviceToHost);
-  cudaFree(d_p);
-  cudaFree(d_o);
-  if (e != cudaSuccess) return fail(MP_ERR_CUDA, std::string("mp_gompertz_curves: ") + cudaGetErrorString(e));
-  return MP_OK;
-}
-
 extern "C" int mp_last_stiff_count(mp_handle* h, int32_t* count) {
   if (!h || !count) return fail(MP_ERR_BAD_ARG, "mp_last_stiff_count: null pointer");
   MP_CUDA(cudaSetDevice(h->device));
   MP_CUDA(cudaDeviceSynchronize());
   *count = 0;
-  if (h->last_lane && h->last_lane->counters)
-    MP_CUDA(cudaMemcpy(count, h->last_lane->counters + 2, sizeof(int), cudaMemcpyDeviceToHost));
-  return MP_OK;
-}
-
-extern "C" int mp_fp64_peak_tflops(int32_t device, double* tflops) {
-  if (!tflops) return fail(MP_ERR_BAD_ARG, "mp_fp64_peak_tflops: null pointer");
-  if (mp_device_count() <= device || device < 0) return fail(MP_ERR_CUDA, "no such CUDA device");
-  MP_CUDA(cudaSetDevice(device));
-  cudaDeviceProp prop;
-  MP_CUDA(cudaGetDeviceProperties(&prop, device));
-  double* d = nullptr;
-  MP_CUDA(cudaMalloc((void**)&d, 8));
-  const int blocks = prop.multiProcessorCount * 8, iters = 4096;
-  cudaEvent_t e0, e1;
-  MP_CUDA(cudaEventCreate(&e0));
-  MP_CUDA(cudaEventCreate(&e1));
-  double best = 0.0;
-  for (int rep = 0; rep < 6; ++rep) {
-    MP_CUDA(cudaEventRecord(e0));
-    dfma_peak_kernel<<<blocks, 256>>>(d, iters, 1.0 + rep);
-    MP_CUDA(cudaEventRecord(e1));
-    MP_CUDA(cudaEventSynchronize(e1));
-    float ms = 0;
-    MP_CUDA(cudaEventElapsedTime(&ms, e0, e1));
-    const double flops = 2.0 * 64.0 * iters * 256.0 * blocks;
-    if (rep > 0) best = std::max(best, flops / (ms * 1e-3) / 1e12);
-  }
-  cudaEventDestroy(e0); cudaEventDestroy(e1);
-  cudaFree(d);
-  *tflops = best;
+  if (h->last_lane && h->last_lane->counters.get())
+    MP_CUDA(cudaMemcpy(count, h->last_lane->counters.get() + 2, sizeof(int), cudaMemcpyDeviceToHost));
   return MP_OK;
 }
