@@ -255,6 +255,48 @@ int mp_tempered_half_step(mp_handle* h, const mp_ensemble* e, int32_t ntemps, co
 int mp_tempered_swap(const mp_ensemble* e, int32_t ntemps, const double* betas, uint64_t step,
                      int32_t* d_swap_accepted, void* stream);
 
+/* ---- emcee 3's moves= (StretchMove, DEMove, DESnookerMove) --------------------------------------------------
+ * The half-steps above with a weighted mix of moves instead of the stretch move of e->a.  Per half-step, with the
+ * existing split: mover x is moved against the complement half C, |C| = Nc (in a tempered ensemble, the complement
+ * within the mover's own temperature).  hs = 2*step + split is the half-step counter, me the mover's row, and
+ * idx(u, m) = min((int)(u*m), m-1) the partner rule.
+ *   Random draws: two Philox4x32-10 blocks per mover beyond the stretch move's, A = counter (hs, me, 4) and
+ *     B = counter (hs, me, 5), keyed by the seed; words 0-3 keep their meaning, so the stretch move's stream does not
+ *     change.
+ *   MP_MOVE_DE (gamma0, sigma; Nelson et al. 2014): uj = u01(A0,A1), uk = u01(A2,A3), ug = u01(B0,B1),
+ *     ua = u01(B2,B3).  Partners are an ordered pair of distinct positions: j = idx(uj, Nc), then k = idx(uk, Nc-1),
+ *     and k += 1 if k >= j.  g = gamma0 * (1 + s3*(2*ug - 1)) with s3 = sigma*sqrt(3) (host); gamma0 = 0 means
+ *     2.38/sqrt(2*ndim).  q_c = x_c + g*(c_j,c - c_k,c), every operation rounded on its own.  ln f = 0.  Unlike
+ *     emcee the jitter on gamma is uniform with standard deviation sigma, not Gaussian (no log/cos: positions stay
+ *     reproducible bit for bit on the host).
+ *   MP_MOVE_DE_SNOOKER (gammas; ter Braak & Vrugt 2008): uz = u01(A0,A1), u1 = u01(A2,A3), u2 = u01(B0,B1),
+ *     ua = u01(B2,B3).  Three distinct positions: z = idx(uz, Nc); r1 = idx(u1, Nc-1), moved up past z;
+ *     r2 = idx(u2, Nc-2), moved up past z and r1 in ascending order.  e = x - z, ee = sum_c e_c^2,
+ *     dd = sum_c (r1_c - r2_c)*e_c (ascending c, rounded term by term); q = x + (gammas*dd/ee)*e;
+ *     ln f = (0.5*(ndim-1)) * log(sum_c (q_c - z_c)^2 / ee).  ee == 0: q = x and ln f = 0; a zero numerator gives
+ *     ln f = -inf (rejected).
+ *   MP_MOVE_STRETCH (a): exactly the stretch move of mp_ensemble_half_step.
+ *   Accept: ((ln f + lq) - lx) > log(ua), lq and lx weighted by beta_t in a tempered ensemble.  Status, bad_rows,
+ *     counters and pack_out as for the stretch move.
+ *   Which move runs: one per MCMC step, for both half-steps and every temperature.  u = u01 of Philox counter
+ *     (step, 0, 6); the move is the first k with u*W < cum_k, W and cum_k the sequential sums of the weights.
+ * Checked on the host before any device work (MP_ERR_BAD_ARG): moves non-null, 1 <= n_moves <= MP_MAX_MOVES, known
+ * kinds, weights finite and >= 0 with a positive sum, stretch a > 1, DE 0 <= sigma < 1 and gamma0 >= 0, snooker
+ * gammas > 0, and a half (per temperature) of at least 2 walkers for DE and 3 for snooker when they have weight.   */
+#define MP_MOVE_STRETCH 0
+#define MP_MOVE_DE 1
+#define MP_MOVE_DE_SNOOKER 2
+#define MP_MAX_MOVES 8
+typedef struct mp_move {
+  int32_t kind;
+  int32_t pad;
+  double weight, a, gamma0, sigma, gammas;
+} mp_move;
+int mp_ensemble_moves_half_step(mp_handle* h, const mp_ensemble* e, const mp_move* moves, int32_t n_moves,
+                                uint64_t step, int32_t split, void* stream);
+int mp_tempered_moves_half_step(mp_handle* h, const mp_ensemble* e, int32_t ntemps, const double* betas,
+                                const mp_move* moves, int32_t n_moves, uint64_t step, int32_t split, void* stream);
+
 /* Peer-mappable device memory for the replicas (CUDA IPC; one process per GPU on one node).
  * mp_peer_alloc: cudaMalloc + export a 64-byte handle other processes pass to mp_peer_open, which maps the
  * block into the caller's address space on `device` (NVLink peer access).  mp_peer_barrier: every rank calls

@@ -15,6 +15,8 @@ MP_MAX_NDIM = 9
 MP_ABI_VERSION = 2
 MP_MAX_PEERS = 15
 MP_MAX_TEMPS = 256
+MP_MOVE_STRETCH, MP_MOVE_DE, MP_MOVE_DE_SNOOKER = range(3)
+MP_MAX_MOVES = 8
 
 MP_OK, MP_ERR_BAD_ARG, MP_ERR_DATA_RANGE, MP_ERR_CUDA, MP_ERR_BAD_GRID, MP_ERR_NO_DATA = range(6)
 
@@ -55,6 +57,12 @@ class Ensemble(C.Structure):
                 ("synced_step", C.c_uint64),
                 ("pack_out", C.c_void_p), ("bad_rows", C.c_void_p), ("bad_count", C.c_void_p),
                 ("bad_capacity", C.c_int32)]
+
+
+class Move(C.Structure):
+    """mp_move (include/magprop_b200.h): one entry of a weighted list of ensemble moves."""
+    _fields_ = [("kind", C.c_int32), ("pad", C.c_int32), ("weight", C.c_double), ("a", C.c_double),
+                ("gamma0", C.c_double), ("sigma", C.c_double), ("gammas", C.c_double)]
 
 
 def script_model_spec(n=10.0, alpha=0.1, cs7=1.0, k=0.9, dipeff=1.0, propeff=1.0, f_beam=1.0,
@@ -140,6 +148,9 @@ def declare(lib):
     lib.mp_ensemble_unpack.argtypes = [C.POINTER(Ensemble), C.c_uint64, C.c_int32, vp, vp]
     lib.mp_ensemble_order.argtypes = [C.c_int32, C.c_uint64, C.c_uint64, C.c_int32, vp, vp]
     lib.mp_tempered_half_step.argtypes = [vp, C.POINTER(Ensemble), C.c_int32, vp, C.c_uint64, C.c_int32, vp]
+    lib.mp_ensemble_moves_half_step.argtypes = [vp, C.POINTER(Ensemble), vp, C.c_int32, C.c_uint64, C.c_int32, vp]
+    lib.mp_tempered_moves_half_step.argtypes = [vp, C.POINTER(Ensemble), C.c_int32, vp, vp, C.c_int32, C.c_uint64,
+                                                C.c_int32, vp]
     lib.mp_tempered_swap.argtypes = [C.POINTER(Ensemble), C.c_int32, vp, C.c_uint64, vp, vp]
     lib.mp_peer_alloc.argtypes = [C.c_int32, C.c_uint64, C.POINTER(vp), C.c_char_p]
     lib.mp_peer_open.argtypes = [C.c_int32, C.c_char_p, C.POINTER(vp)]
@@ -163,7 +174,7 @@ EXPORTS = ["mp_abi_version", "mp_device_count", "mp_last_error", "mp_create", "m
            "mp_curve_nodes", "mp_model_curves", "mp_model_curves_device", "mp_rhs_batch",
            "mp_stretch_half_step", "mp_fp64_peak_tflops", "mp_last_stiff_count",
            "mp_ensemble_half_step", "mp_ensemble_sync", "mp_ensemble_unpack", "mp_ensemble_order",
-           "mp_tempered_half_step", "mp_tempered_swap",
+           "mp_tempered_half_step", "mp_tempered_swap", "mp_ensemble_moves_half_step", "mp_tempered_moves_half_step",
            "mp_chain_moments", "mp_chain_order_statistics", "mp_chain_autocorr", "mp_gompertz_curves", "mp_kernels_launched",
            "mp_peer_alloc", "mp_peer_open", "mp_peer_close", "mp_peer_free", "mp_peer_barrier"]
 

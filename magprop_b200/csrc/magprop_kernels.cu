@@ -203,9 +203,12 @@ __global__ void order_scatter_kernel(int W, const int* __restrict__ key, int* __
   if (kk >= 0) slot_wid[pos] = i;
 }
 
-// The stretch move wrapped around an evaluation (mp_stretch_half_step / mp_ensemble_half_step):
+// The ensemble move wrapped around an evaluation (mp_stretch_half_step / mp_ensemble_half_step / the *_moves_ entry
+// points).  The stretch move:
 //   z = ((a-1) u + 1)^2 / a ; q = c - (c - s) z ; accept iff (ndim-1) ln z + lp(q) - lp(s) > ln u'
-// (Goodman & Weare 2010; emcee's RedBlueMove); tempered: beta_t lp(q) - beta_t lp(s).  setup_kernel forms the proposals, the reduce kernels accept.
+// (Goodman & Weare 2010; emcee's RedBlueMove); tempered: beta_t lp(q) - beta_t lp(s).  `kind` may instead be
+// differential evolution or its snooker update (include/magprop_b200.h, mp_move), whose proposals leave the log of
+// their Hastings factor in `lnf`.  One kind per launch.  setup_kernel forms the proposals, the reduce kernels accept.
 struct Move {
   double* coords;        // [nwalkers][ndim], updated in place
   double* lnp;           // [nwalkers]
@@ -244,6 +247,9 @@ struct Move {
   double* bad_rows;      // proposals whose likelihood was not finite ({GRB}_bad.csv, mcmc_eqns.py:72-79)
   int* bad_count;
   int bad_capacity;
+  int kind;              // MP_MOVE_STRETCH (a above), MP_MOVE_DE (g0 = gamma0, s3 = sigma sqrt 3), MP_MOVE_DE_SNOOKER (gammas)
+  double g0, s3, gammas;
+  double* lnf;           // [n_active] ln of each proposal's Hastings factor (DE, snooker; work space next to prop)
 };
 
 struct Draw {
@@ -261,17 +267,25 @@ __device__ __forceinline__ const double* replica_coords(const Move& m, int home)
 __device__ __forceinline__ const double* replica_lnp(const Move& m, int home) {
   return home == m.rank ? m.lnp : m.peer_lnp[home < m.rank ? home : home - 1];
 }
+// The row mover i moves, and its temperature (0 unless tempered).
+__device__ __forceinline__ int mover_row(const Move& m, int i, int& t) {
+  t = 0;
+  if (m.betas) {
+    const TemperedMover tm = tempered_mover(m.perm, (uint32_t)m.pos0, (uint32_t)(m.mover0 + i));
+    t = (int)tm.t;
+    return (int)tm.row;
+  }
+  return m.active ? m.active[i] : (int)perm_at(m.perm, (uint32_t)(m.pos0 + i));
+}
+// The row at position pj of the complement of a mover of temperature t.
+__device__ __forceinline__ int partner_row(const Move& m, int t, int pj) {
+  if (m.betas) return (int)tempered_partner(m.perm, (uint32_t)m.cpos0, (uint32_t)t, (uint32_t)pj);
+  return m.complement ? m.complement[pj] : (int)perm_at(m.perm, (uint32_t)(m.cpos0 + pj));
+}
 // counter = (half-step, walker); two Philox blocks give u_z, u_partner, u_accept.  (Tempered: walker = global row.)
 __device__ __forceinline__ Draw draw_for(const Move& m, int i) {
   Draw d;
-  d.t = 0;
-  if (m.betas) {
-    const TemperedMover tm = tempered_mover(m.perm, (uint32_t)m.pos0, (uint32_t)(m.mover0 + i));
-    d.t = (int)tm.t;
-    d.me = (int)tm.row;
-  } else {
-    d.me = m.active ? m.active[i] : (int)perm_at(m.perm, (uint32_t)(m.pos0 + i));
-  }
+  d.me = mover_row(m, i, d.t);
   const Philox r0 = philox4x32_10((uint32_t)m.step, (uint32_t)(m.step >> 32), (uint32_t)d.me, 0u,
                                   (uint32_t)m.seed, (uint32_t)(m.seed >> 32));
   const Philox r1 = philox4x32_10((uint32_t)m.step, (uint32_t)(m.step >> 32), (uint32_t)d.me, 1u,
@@ -283,8 +297,7 @@ __device__ __forceinline__ Draw draw_for(const Move& m, int i) {
   d.z = __ddiv_rn(__dmul_rn(zr, zr), m.a);
   int pj = (int)(up * m.n_complement);
   if (pj >= m.n_complement) pj = m.n_complement - 1;
-  if (m.betas) d.partner = (int)tempered_partner(m.perm, (uint32_t)m.cpos0, (uint32_t)d.t, (uint32_t)pj);
-  else d.partner = m.complement ? m.complement[pj] : (int)perm_at(m.perm, (uint32_t)(m.cpos0 + pj));
+  d.partner = partner_row(m, d.t, pj);
   d.pj = pj;
   return d;
 }
@@ -326,17 +339,77 @@ __device__ __forceinline__ void rec_load_lum(const Work& k, int i, Walker& w) {
 // The stretch proposal of mover i (see Move): q = c - (c - s) z, kept in m.prop[i] for the accept step.  With
 // peer-mapped replicas the mover's current row is first brought into the local replica (it is about to be moved
 // here) and the partner's row is read from its home.
+__device__ __forceinline__ void fetch_mover(const Move& m, int me, int ndim) {
+  const int hm = home_before_this_step(m, me);
+  if (hm != m.rank) {
+    const double* src = replica_coords(m, hm);
+    for (int c = 0; c < ndim; ++c) m.coords[(size_t)me * ndim + c] = src[(size_t)me * ndim + c];
+    m.lnp[me] = replica_lnp(m, hm)[me];
+  }
+}
+// The replica that holds the current row of the walker at complement position pj (row `row`).
+__device__ __forceinline__ const double* partner_replica(const Move& m, int pj, int row) {
+  if (m.n_peers == 0) return m.coords;
+  return replica_coords(m, m.split == 1 ? pj / m.n_mine : home_before_this_step(m, row));
+}
+// The differential-evolution proposals of mover i (Move::kind MP_MOVE_DE or MP_MOVE_DE_SNOOKER; the formulas are those
+// of include/magprop_b200.h, mp_move): q in th and m.prop[i], ln f in m.lnf[i].  No FMA contraction, as in propose().
+__device__ __noinline__ void propose_de(const Move& m, int i, int ndim, double* th) {
+  int t;
+  const int me = mover_row(m, i, t);
+  const MoveDraws u = move_draws(m.seed, m.step, (uint32_t)me);
+  if (m.n_peers > 0) fetch_mover(m, me, ndim);
+  const double* x = m.coords + (size_t)me * ndim;
+  const uint32_t nc = (uint32_t)m.n_complement;
+  double lnf = 0.0;
+  if (m.kind == MP_MOVE_DE) {
+    uint32_t j, k;
+    de_pair(u.u[0], u.u[1], nc, &j, &k);
+    const int rj = partner_row(m, t, (int)j), rk = partner_row(m, t, (int)k);
+    const double* cj = partner_replica(m, (int)j, rj) + (size_t)rj * ndim;
+    const double* ck = partner_replica(m, (int)k, rk) + (size_t)rk * ndim;
+    const double g = __dmul_rn(m.g0, __dadd_rn(1.0, __dmul_rn(m.s3, __dadd_rn(__dmul_rn(2.0, u.u[2]), -1.0))));
+    for (int c = 0; c < ndim; ++c) th[c] = __dadd_rn(x[c], __dmul_rn(g, __dadd_rn(cj[c], -ck[c])));
+  } else {
+    uint32_t jz, j1, j2;
+    snooker_triple(u.u[0], u.u[1], u.u[2], nc, &jz, &j1, &j2);
+    const int rz = partner_row(m, t, (int)jz), r1 = partner_row(m, t, (int)j1), r2 = partner_row(m, t, (int)j2);
+    const double* z = partner_replica(m, (int)jz, rz) + (size_t)rz * ndim;
+    const double* c1 = partner_replica(m, (int)j1, r1) + (size_t)r1 * ndim;
+    const double* c2 = partner_replica(m, (int)j2, r2) + (size_t)r2 * ndim;
+    double ee = 0.0, dd = 0.0;
+    for (int c = 0; c < ndim; ++c) {
+      const double e = __dadd_rn(x[c], -z[c]);
+      ee = __dadd_rn(ee, __dmul_rn(e, e));
+      dd = __dadd_rn(dd, __dmul_rn(__dadd_rn(c1[c], -c2[c]), e));
+    }
+    if (ee == 0.0) {
+      for (int c = 0; c < ndim; ++c) th[c] = x[c];
+    } else {
+      const double f = __ddiv_rn(__dmul_rn(m.gammas, dd), ee);
+      double nq = 0.0;
+      for (int c = 0; c < ndim; ++c) {
+        th[c] = __dadd_rn(x[c], __dmul_rn(f, __dadd_rn(x[c], -z[c])));
+        const double w = __dadd_rn(th[c], -z[c]);
+        nq = __dadd_rn(nq, __dmul_rn(w, w));
+      }
+      lnf = nq == 0.0 ? -INFINITY : __dmul_rn(0.5 * (ndim - 1.0), log(__ddiv_rn(nq, ee)));
+    }
+  }
+  for (int c = 0; c < ndim; ++c) m.prop[(size_t)i * ndim + c] = th[c];
+  m.lnf[i] = lnf;
+}
+
 __device__ __forceinline__ void propose(const Move& m, int i, int ndim, double* th) {
+  if (m.kind != MP_MOVE_STRETCH) {
+    propose_de(m, i, ndim, th);
+    return;
+  }
   const Draw d = draw_for(m, i);
   const double* pc = m.coords;
   if (m.n_peers > 0) {
-    const int hm = home_before_this_step(m, d.me);
-    if (hm != m.rank) {
-      const double* src = replica_coords(m, hm);
-      for (int c = 0; c < ndim; ++c) m.coords[(size_t)d.me * ndim + c] = src[(size_t)d.me * ndim + c];
-      m.lnp[d.me] = replica_lnp(m, hm)[d.me];
-    }
-    pc = replica_coords(m, m.split == 1 ? d.pj / m.n_mine : home_before_this_step(m, d.partner));
+    fetch_mover(m, d.me, ndim);
+    pc = partner_replica(m, d.pj, d.partner);
   }
   for (int c = 0; c < ndim; ++c) {
     const double cc = pc[(size_t)d.partner * ndim + c];
@@ -610,18 +683,27 @@ __device__ __forceinline__ void deliver(const Problem& p, const Work& k, const S
     return;
   }
   const int ndim = p.ndim;
-  const Draw d = draw_for(m, i);
-  const int me = d.me;
+  int me, t;
+  double lnf, ua;                            // ln of the Hastings factor, the accept draw
+  if (m.kind == MP_MOVE_STRETCH) {
+    const Draw d = draw_for(m, i);
+    me = d.me; t = d.t; ua = d.ua;
+    lnf = __dmul_rn(ndim - 1.0, log(d.z));
+  } else {
+    me = mover_row(m, i, t);
+    ua = move_draws(m.seed, m.step, (uint32_t)me).u[3];
+    lnf = m.lnf[i];
+  }
   const double* q = m.prop + (size_t)i * ndim;
   const double lp_old = m.lnp[me];
   double lq = lp_new, lx = lp_old;           // tempered: beta_t lp (lnp stays untempered)
   if (m.betas) {
-    const double b = m.betas[d.t];
+    const double b = m.betas[t];
     lq = __dmul_rn(b, lp_new);
     lx = __dmul_rn(b, lp_old);
   }
-  const double lnpdiff = __dadd_rn(__dadd_rn(__dmul_rn(ndim - 1.0, log(d.z)), lq), -lx);
-  const bool accept = lnpdiff > log(d.ua);
+  const double lnpdiff = __dadd_rn(__dadd_rn(lnf, lq), -lx);
+  const bool accept = lnpdiff > log(ua);
   if (accept) {
     for (int c = 0; c < ndim; ++c) m.coords[(size_t)me * ndim + c] = q[c];
     m.lnp[me] = lp_new;
@@ -859,7 +941,7 @@ struct mp_handle {
   struct Lane {
     cudaStream_t stream = nullptr;   // the handle's own lanes only (a caller's stream is never kept here, nor destroyed)
     DevBuf<unsigned long long> recs;   // kRecWords rows, each as long as the lane's capacity in walkers
-    DevBuf<double> ybuf, prop;
+    DevBuf<double> ybuf, prop, lnf;  // lnf: ln of each proposal's Hastings factor (the DE moves), indexed as prop
     DevBuf<int> status, n_rhs, work, counters, key, hist, slot_wid;
     DevBuf<StiffRec> squeue;
     DevBuf<double> betas;        // the ladder of the tempered half-steps on this lane, and its host copy
@@ -1002,7 +1084,10 @@ static int ensure_work(mp_handle::Lane& L, int S, int Nn, int ndim_prop, Work& k
     if (cudaHostGetDevicePointer((void**)&L.hint_dev, L.hint_host, 0) != cudaSuccess) L.hint_dev = nullptr;
   }
   MP_CUDA(L.ybuf.ensure((size_t)S * Nn));
-  if (ndim_prop > 0) MP_CUDA(L.prop.ensure((size_t)S * ndim_prop));
+  if (ndim_prop > 0) {
+    MP_CUDA(L.prop.ensure((size_t)S * ndim_prop));
+    MP_CUDA(L.lnf.ensure(S));
+  }
   k.stride = (int)(L.recs.size() / kRecWords);
   k.recs = L.recs.get(); k.ybuf = L.ybuf.get(); k.status = L.status.get(); k.n_rhs = L.n_rhs.get(); k.work = L.work.get();
   k.squeue = L.squeue.get(); k.counters = L.counters.get();
@@ -1042,6 +1127,7 @@ static int launch_eval(mp_handle* h, const Problem& p, const double* d_theta, in
       else if (ms.betas) ms.mover0 += i0;     // (a tempered slab may span temperatures: offset the mover, not the position)
       else ms.pos0 += i0;
       ms.prop = Lp->prop.get();
+      ms.lnf = Lp->lnf.get();
       if (ms.pack_out) ms.pack_out += (size_t)i0 * (ndim + 1);
     }
     Sink sk = sink;
@@ -1346,8 +1432,55 @@ extern "C" int mp_ensemble_sync(const mp_ensemble* e, uint64_t step, void* strea
   return MP_OK;
 }
 
+// The stretch move of scale a as an mp_move (the move of mp_ensemble_half_step / mp_tempered_half_step).
+static mp_move stretch_move(double a) {
+  mp_move mv;
+  std::memset(&mv, 0, sizeof(mv));
+  mv.kind = MP_MOVE_STRETCH;
+  mv.weight = 1.0;
+  mv.a = a;
+  return mv;
+}
+
+// The host-side checks of a list of moves for halves (per temperature) of `half` walkers (see mp_move).
+static int check_moves(const mp_move* moves, int32_t n_moves, int half, const char* who) {
+  const std::string w(who);
+  if (!moves || n_moves < 1 || n_moves > MP_MAX_MOVES)
+    return fail(MP_ERR_BAD_ARG, w + ": moves must be non-null and n_moves in [1, MP_MAX_MOVES]");
+  double total = 0.0;
+  for (int k = 0; k < n_moves; ++k) {
+    const mp_move& mv = moves[k];
+    if (!(mv.weight >= 0.0 && std::isfinite(mv.weight))) return fail(MP_ERR_BAD_ARG, w + ": move weights must be finite and >= 0");
+    total += mv.weight;
+    int need = 1;
+    if (mv.kind == MP_MOVE_STRETCH) {
+      if (!(mv.a > 1.0 && std::isfinite(mv.a))) return fail(MP_ERR_BAD_ARG, w + ": stretch move needs a > 1");
+    } else if (mv.kind == MP_MOVE_DE) {
+      if (!(mv.sigma >= 0.0 && mv.sigma < 1.0)) return fail(MP_ERR_BAD_ARG, w + ": DE move needs 0 <= sigma < 1");
+      if (!(mv.gamma0 >= 0.0 && std::isfinite(mv.gamma0))) return fail(MP_ERR_BAD_ARG, w + ": DE move needs gamma0 >= 0");
+      need = 2;
+    } else if (mv.kind == MP_MOVE_DE_SNOOKER) {
+      if (!(mv.gammas > 0.0 && std::isfinite(mv.gammas))) return fail(MP_ERR_BAD_ARG, w + ": snooker move needs gammas > 0");
+      need = 3;
+    } else {
+      return fail(MP_ERR_BAD_ARG, w + ": unknown move kind");
+    }
+    if (mv.weight > 0.0 && half < need)
+      return fail(MP_ERR_BAD_ARG, w + ": a half of the ensemble holds fewer walkers than the move's partners");
+  }
+  if (!(total > 0.0 && std::isfinite(total))) return fail(MP_ERR_BAD_ARG, w + ": move weights must have a positive, finite sum");
+  return MP_OK;
+}
+
+// The move MCMC step `step` runs (choose_move: one per step, the same for both half-steps and every temperature).
+static const mp_move& pick_move(const mp_move* moves, int32_t n_moves, uint64_t seed, uint64_t step) {
+  double w[MP_MAX_MOVES];
+  for (int k = 0; k < n_moves; ++k) w[k] = moves[k].weight;
+  return moves[choose_move(seed, step, w, n_moves)];
+}
+
 // The move of this rank's share of half `split` at MCMC step `step` (everything but the pull side).
-static void fill_ensemble_move(const mp_ensemble* e, uint64_t step, int split, Move& m) {
+static void fill_ensemble_move(const mp_ensemble* e, uint64_t step, int split, const mp_move& mv, Move& m) {
   const int half = e->nwalkers / 2, n_mine = half / e->world;
   std::memset(&m, 0, sizeof(m));
   m.coords = e->coords;
@@ -1356,7 +1489,11 @@ static void fill_ensemble_move(const mp_ensemble* e, uint64_t step, int split, M
   m.pos0 = split * half + e->rank * n_mine;
   m.cpos0 = (1 - split) * half;
   m.n_complement = half;
-  m.a = e->a;
+  m.kind = mv.kind;
+  m.a = mv.a;
+  m.g0 = mv.gamma0 > 0.0 ? mv.gamma0 : 2.38 / std::sqrt(2.0 * e->ndim);
+  m.s3 = mv.sigma * std::sqrt(3.0);
+  m.gammas = mv.gammas;
   m.seed = e->seed;
   m.step = 2 * step + (uint64_t)split;
   m.accepted = e->accepted;
@@ -1371,20 +1508,38 @@ static void fill_ensemble_move(const mp_ensemble* e, uint64_t step, int split, M
   }
 }
 
+// One half-step of a (checked) ensemble with move `mv`: mp_ensemble_half_step and mp_ensemble_moves_half_step.
+static int ensemble_half_step(mp_handle* h, const mp_ensemble* e, const mp_move& mv, uint64_t step, int32_t split,
+                              void* stream, const char* who) {
+  MP_CUDA(cudaSetDevice(h->device));
+  const int n_mine = e->nwalkers / 2 / e->world;
+  Problem p;
+  int rc = fill_move_problem(h, p, e->ndim, n_mine);
+  if (rc) return rc;
+  Move m;
+  fill_ensemble_move(e, step, split, mv, m);
+  if ((rc = fill_pull(e, step, m, who))) return rc;
+  return launch_eval<kModeLnprob, true>(h, p, nullptr, n_mine, Sink{nullptr, nullptr, nullptr}, nullptr, nullptr, &m,
+                                        (cudaStream_t)stream);
+}
+
 extern "C" int mp_ensemble_half_step(mp_handle* h, const mp_ensemble* e, uint64_t step, int32_t split, void* stream) {
   if (!h) return fail(MP_ERR_BAD_ARG, "mp_ensemble_half_step: null handle");
   int rc = check_ensemble(e, "mp_ensemble_half_step");
   if (rc) return rc;
   if (split != 0 && split != 1) return fail(MP_ERR_BAD_ARG, "mp_ensemble_half_step: split must be 0 or 1");
-  MP_CUDA(cudaSetDevice(h->device));
-  const int n_mine = e->nwalkers / 2 / e->world;
-  Problem p;
-  if ((rc = fill_move_problem(h, p, e->ndim, n_mine))) return rc;
-  Move m;
-  fill_ensemble_move(e, step, split, m);
-  if ((rc = fill_pull(e, step, m, "mp_ensemble_half_step"))) return rc;
-  return launch_eval<kModeLnprob, true>(h, p, nullptr, n_mine, Sink{nullptr, nullptr, nullptr}, nullptr, nullptr, &m,
-                                        (cudaStream_t)stream);
+  return ensemble_half_step(h, e, stretch_move(e->a), step, split, stream, "mp_ensemble_half_step");
+}
+
+extern "C" int mp_ensemble_moves_half_step(mp_handle* h, const mp_ensemble* e, const mp_move* moves, int32_t n_moves,
+                                           uint64_t step, int32_t split, void* stream) {
+  const char* who = "mp_ensemble_moves_half_step";
+  int rc = check_ensemble(e, who);
+  if (rc) return rc;
+  if (split != 0 && split != 1) return fail(MP_ERR_BAD_ARG, std::string(who) + ": split must be 0 or 1");
+  if ((rc = check_moves(moves, n_moves, e->nwalkers / 2, who))) return rc;
+  if (!h) return fail(MP_ERR_BAD_ARG, std::string(who) + ": null handle");
+  return ensemble_half_step(h, e, pick_move(moves, n_moves, e->seed, step), step, split, stream, who);
 }
 
 // ---- parallel tempering ----------------------------------------------------------------------------
@@ -1418,12 +1573,11 @@ static int upload_ladder(mp_handle::Lane& L, int ntemps, const double* betas, cu
   return MP_OK;
 }
 
-extern "C" int mp_tempered_half_step(mp_handle* h, const mp_ensemble* e, int32_t ntemps, const double* betas, uint64_t step,
-                                     int32_t split, void* stream) {
-  int rc = check_tempered(e, ntemps, betas, "mp_tempered_half_step");
-  if (rc) return rc;
-  if (!h) return fail(MP_ERR_BAD_ARG, "mp_tempered_half_step: null handle");
-  if (split != 0 && split != 1) return fail(MP_ERR_BAD_ARG, "mp_tempered_half_step: split must be 0 or 1");
+// One half-step of every temperature of a (checked) tempered ensemble with move `mv`: mp_tempered_half_step and
+// mp_tempered_moves_half_step.
+static int tempered_half_step(mp_handle* h, const mp_ensemble* e, int32_t ntemps, const double* betas, const mp_move& mv,
+                              uint64_t step, int32_t split, void* stream) {
+  int rc;
   MP_CUDA(cudaSetDevice(h->device));
   const cudaStream_t s = (cudaStream_t)stream;
   const int half = e->nwalkers / 2, n_movers = ntemps * half;
@@ -1433,11 +1587,31 @@ extern "C" int mp_tempered_half_step(mp_handle* h, const mp_ensemble* e, int32_t
   lane_for(h, s, -1, &L);
   if ((rc = upload_ladder(*L, ntemps, betas, s))) return rc;
   Move m;
-  fill_ensemble_move(e, step, split, m);
+  fill_ensemble_move(e, step, split, mv, m);
   m.rank = 0;
   m.half = m.n_mine = half;
   m.betas = L->betas.get();
   return launch_eval<kModeLnprob, true>(h, p, nullptr, n_movers, Sink{nullptr, nullptr, nullptr}, nullptr, nullptr, &m, s);
+}
+
+extern "C" int mp_tempered_half_step(mp_handle* h, const mp_ensemble* e, int32_t ntemps, const double* betas, uint64_t step,
+                                     int32_t split, void* stream) {
+  int rc = check_tempered(e, ntemps, betas, "mp_tempered_half_step");
+  if (rc) return rc;
+  if (!h) return fail(MP_ERR_BAD_ARG, "mp_tempered_half_step: null handle");
+  if (split != 0 && split != 1) return fail(MP_ERR_BAD_ARG, "mp_tempered_half_step: split must be 0 or 1");
+  return tempered_half_step(h, e, ntemps, betas, stretch_move(e->a), step, split, stream);
+}
+
+extern "C" int mp_tempered_moves_half_step(mp_handle* h, const mp_ensemble* e, int32_t ntemps, const double* betas,
+                                           const mp_move* moves, int32_t n_moves, uint64_t step, int32_t split, void* stream) {
+  const char* who = "mp_tempered_moves_half_step";
+  int rc = check_tempered(e, ntemps, betas, who);
+  if (rc) return rc;
+  if (split != 0 && split != 1) return fail(MP_ERR_BAD_ARG, std::string(who) + ": split must be 0 or 1");
+  if ((rc = check_moves(moves, n_moves, e->nwalkers / 2, who))) return rc;
+  if (!h) return fail(MP_ERR_BAD_ARG, std::string(who) + ": null handle");
+  return tempered_half_step(h, e, ntemps, betas, pick_move(moves, n_moves, e->seed, step), step, split, stream);
 }
 
 extern "C" int mp_tempered_swap(const mp_ensemble* e, int32_t ntemps, const double* betas, uint64_t step,

@@ -126,4 +126,60 @@ MP_RNG_HD bool pt_swap_accept(uint64_t seed, uint64_t step, uint32_t row_hot, do
   return log(u01(r.c[0], r.c[1])) < (beta_cold - beta_hot) * (lnp_hot - lnp_cold);
 }
 
+// ---- the differential-evolution moves (mp_ensemble_moves_half_step) -------------------------------------
+// The partner rule of every move: position min(floor(u m), m-1) of m.
+MP_RNG_HD uint32_t pick_index(double u, uint32_t m) {
+  const uint32_t i = (uint32_t)(u * m);
+  return i < m ? i : m - 1u;
+}
+// The four uniforms of a DE or snooker mover: Philox blocks A = counter (hs, me, 4) and B = (hs, me, 5); u[0] from
+// A0,A1, u[1] from A2,A3, u[2] from B0,B1, u[3] from B2,B3 (the accept draw).  Words 0-3 stay the stretch move's.
+struct MoveDraws {
+  double u[4];
+};
+MP_RNG_HD MoveDraws move_draws(uint64_t seed, uint64_t hs, uint32_t me) {
+  const Philox a = philox4x32_10((uint32_t)hs, (uint32_t)(hs >> 32), me, 4u, (uint32_t)seed, (uint32_t)(seed >> 32));
+  const Philox b = philox4x32_10((uint32_t)hs, (uint32_t)(hs >> 32), me, 5u, (uint32_t)seed, (uint32_t)(seed >> 32));
+  MoveDraws d;
+  d.u[0] = u01(a.c[0], a.c[1]);
+  d.u[1] = u01(a.c[2], a.c[3]);
+  d.u[2] = u01(b.c[0], b.c[1]);
+  d.u[3] = u01(b.c[2], b.c[3]);
+  return d;
+}
+// DE: an ordered pair of distinct positions of the complement (nc >= 2).
+MP_RNG_HD void de_pair(double uj, double uk, uint32_t nc, uint32_t* j, uint32_t* k) {
+  *j = pick_index(uj, nc);
+  *k = pick_index(uk, nc - 1u);
+  if (*k >= *j) *k += 1u;
+}
+// Snooker: three distinct positions z, r1, r2 of the complement (nc >= 3), each uniform over the positions left.
+MP_RNG_HD void snooker_triple(double uz, double u1, double u2, uint32_t nc, uint32_t* z, uint32_t* r1, uint32_t* r2) {
+  *z = pick_index(uz, nc);
+  *r1 = pick_index(u1, nc - 1u);
+  if (*r1 >= *z) *r1 += 1u;
+  const uint32_t lo = *z < *r1 ? *z : *r1, hi = *z < *r1 ? *r1 : *z;
+  *r2 = pick_index(u2, nc - 2u);
+  if (*r2 >= lo) *r2 += 1u;
+  if (*r2 >= hi) *r2 += 1u;
+}
+// Which of n moves MCMC step `step` runs (one move per step, as emcee picks one per iteration): u from Philox counter
+// (step, 0, word 6); the first k with u W < cum_k, W and cum_k the sequential sums of the weights.  (Should rounding
+// leave no such k, the last move of positive weight.)
+MP_RNG_HD int choose_move(uint64_t seed, uint64_t step, const double* weights, int n) {
+  const Philox r = philox4x32_10((uint32_t)step, (uint32_t)(step >> 32), 0u, 6u, (uint32_t)seed, (uint32_t)(seed >> 32));
+  const double u = u01(r.c[0], r.c[1]);
+  double W = 0.0;
+  for (int k = 0; k < n; ++k) W += weights[k];
+  const double uw = u * W;
+  double cum = 0.0;
+  int last = 0;
+  for (int k = 0; k < n; ++k) {
+    cum += weights[k];
+    if (weights[k] > 0.0) last = k;
+    if (uw < cum) return k;
+  }
+  return last;
+}
+
 }  // namespace mp

@@ -25,6 +25,9 @@ so this module carries the minimum needed to run and measure the path:
                         per half-step (``mp_tempered_half_step``), then one swap
                         pass per step (``mp_tempered_swap``).
 ``thermodynamic_log_evidence``  ln Z by thermodynamic integration over the ladder.
+``StretchMove``, ``DEMove``, ``DESnookerMove``  emcee 3's ``moves=``: both ensembles take a move, a list of
+                        moves or a list of ``(move, weight)`` and run one of them per step
+                        (``mp_ensemble_moves_half_step`` / ``mp_tempered_moves_half_step``).
 
 Move semantics (Goodman & Weare 2010, as emcee's RedBlueMove implements them;
 SURVEY.md appendix C): every step the walkers are split into two halves at random
@@ -109,6 +112,114 @@ class EnsembleSampler:
         return self.naccepted / max(1, self.iteration)
 
 
+# ---- emcee 3's moves= ------------------------------------------------------------------------------------
+class StretchMove:
+    """emcee's ``StretchMove(a=2.0)``: the affine-invariant stretch move (Goodman & Weare 2010), scale ``a`` > 1."""
+    kind = 0
+
+    def __init__(self, a=2.0):
+        self.a = float(a)
+
+    def _check(self):
+        if not (np.isfinite(self.a) and self.a > 1.0):
+            raise ValueError("StretchMove needs a > 1")
+
+    def _fill(self, m):
+        m.a = self.a
+
+    def __repr__(self):
+        return f"StretchMove(a={self.a})"
+
+
+class DEMove:
+    """emcee's ``DEMove(sigma=1e-5, gamma0=None)``: differential evolution (Nelson et al. 2014),
+    q = x + g (c_j - c_k) for an ordered pair of distinct walkers j, k of the complement.  g is ``gamma0`` (None:
+    2.38 / sqrt(2 ndim)) times 1 + a jitter of standard deviation ``sigma`` -- uniform here, Gaussian in emcee
+    (include/magprop_b200.h, mp_move, says why)."""
+    kind = 1
+
+    def __init__(self, sigma=1.0e-5, gamma0=None):
+        self.sigma = float(sigma)
+        self.gamma0 = None if gamma0 is None else float(gamma0)
+
+    def _check(self):
+        if not 0.0 <= self.sigma < 1.0:
+            raise ValueError("DEMove needs 0 <= sigma < 1")
+        if self.gamma0 is not None and not (np.isfinite(self.gamma0) and self.gamma0 > 0.0):
+            raise ValueError("DEMove needs gamma0 > 0 (or None for 2.38 / sqrt(2 ndim))")
+
+    def _fill(self, m):
+        m.sigma, m.gamma0 = self.sigma, 0.0 if self.gamma0 is None else self.gamma0
+
+    def __repr__(self):
+        return f"DEMove(sigma={self.sigma}, gamma0={self.gamma0})"
+
+
+class DESnookerMove:
+    """emcee's ``DESnookerMove(gammas=1.7)``: the snooker update of ter Braak & Vrugt (2008) -- x moves along the line
+    through a third walker z by ``gammas`` times the projection of the difference of two more onto it, with the
+    Hastings factor (|q - z| / |x - z|)^(ndim - 1)."""
+    kind = 2
+
+    def __init__(self, gammas=1.7):
+        self.gammas = float(gammas)
+
+    def _check(self):
+        if not (np.isfinite(self.gammas) and self.gammas > 0.0):
+            raise ValueError("DESnookerMove needs gammas > 0")
+
+    def _fill(self, m):
+        m.gammas = self.gammas
+
+    def __repr__(self):
+        return f"DESnookerMove(gammas={self.gammas})"
+
+
+_PARTNERS = {0: 1, 1: 2, 2: 3}        # distinct complement walkers a move needs
+
+
+def move_table(moves, half=None):
+    """``moves`` as emcee accepts it -- a move, a list of moves (equal weights) or a list of ``(move, weight)`` --
+    checked (``ValueError``) and returned as ``(list of (move, weight), ctypes array of mp_move)``.  ``half``: the
+    walkers in a half of the ensemble (per temperature), which must hold every partner a weighted move draws."""
+    from . import _capi as A
+    single = (StretchMove, DEMove, DESnookerMove)
+    if isinstance(moves, single):
+        moves = [moves]
+    try:
+        items = list(moves)
+    except TypeError:
+        raise ValueError("moves must be a move, a list of moves or a list of (move, weight)") from None
+    if not 1 <= len(items) <= A.MP_MAX_MOVES:
+        raise ValueError(f"between 1 and {A.MP_MAX_MOVES} moves")
+    table = []
+    for it in items:
+        if isinstance(it, single):
+            mv, w = it, 1.0
+        elif isinstance(it, (tuple, list)) and len(it) == 2 and isinstance(it[0], single):
+            mv, w = it
+        else:
+            raise ValueError(f"not a move or (move, weight): {it!r}")
+        try:
+            w = float(w)
+        except (TypeError, ValueError):
+            raise ValueError(f"bad move weight: {it!r}") from None
+        if not (np.isfinite(w) and w >= 0.0):
+            raise ValueError("move weights must be finite and >= 0")
+        mv._check()
+        if half is not None and w > 0.0 and half < _PARTNERS[mv.kind]:
+            raise ValueError(f"{mv!r} needs at least {_PARTNERS[mv.kind]} walkers in each half of the ensemble")
+        table.append((mv, w))
+    total = sum(w for _, w in table)
+    if not (np.isfinite(total) and total > 0.0):
+        raise ValueError("move weights must have a positive, finite sum")
+    arr = (A.Move * len(table))()
+    for m, (mv, w) in zip(arr, table):
+        m.kind, m.weight = mv.kind, w
+        mv._fill(m)
+    return table, arr
+
+
 def rank_slice(n_items: int, rank: int, world: int):
     """Contiguous equal share of n_items for `rank`; n_items must divide evenly."""
     if n_items % world:
@@ -165,7 +276,11 @@ class CudaBackend:
         self._own = []
 
     def half_step(self, ens, step, split):
-        self.A.check(self.lib.mp_ensemble_half_step(self.lik._h, C.byref(ens.desc), step, split, self.stream() or None))
+        if ens.moves is None:
+            self.A.check(self.lib.mp_ensemble_half_step(self.lik._h, C.byref(ens.desc), step, split, self.stream() or None))
+        else:
+            self.A.check(self.lib.mp_ensemble_moves_half_step(self.lik._h, C.byref(ens.desc), C.addressof(ens._moves_c),
+                                                              len(ens._moves_c), step, split, self.stream() or None))
 
     def unpack(self, ens, step, split, gathered):
         self.A.check(self.lib.mp_ensemble_unpack(C.byref(ens.desc), step, split, gathered.data_ptr(), self.stream() or None))
@@ -181,8 +296,13 @@ class CudaBackend:
         self.lik.lnprob_device(ens.coords.data_ptr(), ens.coords.shape[0], ens.ndim, ens.lnp.data_ptr(), 0, 0, self.stream())
 
     def tempered_half_step(self, ens, step, split):
-        self.A.check(self.lib.mp_tempered_half_step(self.lik._h, C.byref(ens.desc), ens.ntemps, self.A.ptr(ens.betas), step,
-                                                    split, self.stream() or None))
+        if ens.moves is None:
+            self.A.check(self.lib.mp_tempered_half_step(self.lik._h, C.byref(ens.desc), ens.ntemps, self.A.ptr(ens.betas),
+                                                        step, split, self.stream() or None))
+        else:
+            self.A.check(self.lib.mp_tempered_moves_half_step(self.lik._h, C.byref(ens.desc), ens.ntemps,
+                                                              self.A.ptr(ens.betas), C.addressof(ens._moves_c),
+                                                              len(ens._moves_c), step, split, self.stream() or None))
 
     def tempered_swap(self, ens, step):
         self.A.check(self.lib.mp_tempered_swap(C.byref(ens.desc), ens.ntemps, self.A.ptr(ens.betas), step,
@@ -194,6 +314,9 @@ class DeviceEnsemble:
 
     ``backend`` performs the half-steps: ``CudaBackend`` on a GPU (see ``from_likelihood``); the tests inject a
     NumPy double so the sharding / exchange logic runs under gloo on the CPU.
+
+    ``moves`` (emcee 3's argument, see ``move_table``): None runs the stretch move of scale ``a``; otherwise one of the
+    given moves per step, chosen by weight from the seed, and ``a`` is unused.
     """
 
     BAD_CAPACITY = 4096
@@ -201,11 +324,12 @@ class DeviceEnsemble:
     ntemps = 1                  # rows = ntemps * nwalkers (TemperedEnsemble)
 
     def __init__(self, backend, nwalkers, ndim, a=2.0, seed=0, device="cuda", dist=None, randomize_split=True,
-                 exchange="auto"):
+                 exchange="auto", moves=None):
         import torch
         from . import _capi as A
         if nwalkers % 2 or nwalkers < 2 * ndim:
             raise ValueError("nwalkers must be even and at least 2*ndim")
+        self.moves, self._moves_c = (None, None) if moves is None else move_table(moves, nwalkers // 2)
         self.torch, self.backend = torch, backend
         self.nwalkers, self.ndim, self.a, self.seed = nwalkers, ndim, float(a), int(seed)
         self.randomize_split = bool(randomize_split)
@@ -303,10 +427,11 @@ class DeviceEnsemble:
         return "peer"
 
     @classmethod
-    def from_likelihood(cls, lik, nwalkers, ndim, a=2.0, seed=0, dist=None, randomize_split=True, exchange="auto"):
+    def from_likelihood(cls, lik, nwalkers, ndim, a=2.0, seed=0, dist=None, randomize_split=True, exchange="auto",
+                        moves=None):
         import torch
         ens = cls(CudaBackend(lik), nwalkers, ndim, a=a, seed=seed, device=torch.device("cuda", lik.device), dist=dist,
-                  randomize_split=randomize_split, exchange=exchange)
+                  randomize_split=randomize_split, exchange=exchange, moves=moves)
         ens._lik = lik
         return ens
 
@@ -517,10 +642,12 @@ class TemperedEnsemble(DeviceEnsemble):
     temperature is an ensemble moved as ``DeviceEnsemble`` moves one, accepting on ``beta_t * lnp``; all temperatures
     move in one launch per half-step, and once per step walker j of each temperature may swap places with walker j
     of the next colder one, from the hottest pair down (semantics: ``mp_tempered_half_step`` / ``mp_tempered_swap``
-    in include/magprop_b200.h).  ``lnp`` is untempered.  One device only: ``dist`` raises ``ValueError``.
+    in include/magprop_b200.h).  ``lnp`` is untempered.  One device only: ``dist`` raises ``ValueError``.  ``moves`` as
+    for ``DeviceEnsemble``: the step's move is the same for every temperature.
     ``backend`` as for ``DeviceEnsemble``, with ``tempered_half_step`` and ``tempered_swap``."""
 
-    def __init__(self, backend, nwalkers, ndim, betas, a=2.0, seed=0, device="cuda", randomize_split=True, dist=None):
+    def __init__(self, backend, nwalkers, ndim, betas, a=2.0, seed=0, device="cuda", randomize_split=True, dist=None,
+                 moves=None):
         import torch
         if dist is not None:
             raise ValueError("a tempered ensemble runs on one device: dist is not supported")
@@ -528,14 +655,15 @@ class TemperedEnsemble(DeviceEnsemble):
         self.ntemps = self.betas.size
         if self.ntemps * nwalkers >= 1 << 31:
             raise ValueError("ntemps * nwalkers must be below 2^31")
-        super().__init__(backend, nwalkers, ndim, a=a, seed=seed, device=device, randomize_split=randomize_split)
+        super().__init__(backend, nwalkers, ndim, a=a, seed=seed, device=device, randomize_split=randomize_split,
+                         moves=moves)
         self.swap_accepted = torch.zeros(self.ntemps - 1, dtype=torch.int32, device=self.device)
 
     @classmethod
-    def from_likelihood(cls, lik, nwalkers, ndim, betas, a=2.0, seed=0, randomize_split=True, dist=None):
+    def from_likelihood(cls, lik, nwalkers, ndim, betas, a=2.0, seed=0, randomize_split=True, dist=None, moves=None):
         import torch
         ens = cls(CudaBackend(lik), nwalkers, ndim, betas, a=a, seed=seed, device=torch.device("cuda", lik.device),
-                  randomize_split=randomize_split, dist=dist)
+                  randomize_split=randomize_split, dist=dist, moves=moves)
         ens._lik = lik
         return ens
 

@@ -58,9 +58,10 @@ class RunResult:
         return integrated_time(self._chain, **kw)
 
 
-def run(grb, x, y, yerr, n_walk, n_step, seed=0, p0=None, device=0, dist=None, fbad=None):
+def run(grb, x, y, yerr, n_walk, n_step, seed=0, p0=None, device=0, dist=None, fbad=None, moves=None):
     """One chain of ``n_step`` stretch-move steps for ``n_walk`` walkers, positions resident on the GPU
-    (one fused launch per half-step; with ``dist`` the ensemble is sharded over the ranks).  ``fbad``: the
+    (one fused launch per half-step; with ``dist`` the ensemble is sharded over the ranks).  ``moves``: emcee 3's
+    argument (``DeviceEnsemble``), e.g. ``[(DEMove(), 0.8), (DESnookerMove(), 0.2)]``; None is the stretch move.  ``fbad``: the
     reference's bad-parameter file (``synth_mcmc.py:159,181``, ``mcmc_eqns.py:72-79``) -- proposals whose likelihood
     was not finite are logged on the device and appended to it after the run (by rank 0)."""
     from .. import _capi as A
@@ -74,7 +75,7 @@ def run(grb, x, y, yerr, n_walk, n_step, seed=0, p0=None, device=0, dist=None, f
     p0 = np.asarray(p0, dtype=np.float64)
     lk = Likelihood(A.script_model_spec(), time_grid(None), x, y, yerr, lower, upper, device=device)
     try:
-        ens = DeviceEnsemble.from_likelihood(lk, n_walk, p0.shape[1], a=2.0, seed=seed, dist=dist)
+        ens = DeviceEnsemble.from_likelihood(lk, n_walk, p0.shape[1], a=2.0, seed=seed, dist=dist, moves=moves)
         ens.initialise(p0)
         chain, lnp = ens.run(n_step, store=True)
         ens.check_peers()
@@ -90,14 +91,14 @@ def run(grb, x, y, yerr, n_walk, n_step, seed=0, p0=None, device=0, dist=None, f
     return res
 
 
-def run_tempered(grb, x, y, yerr, n_walk, ntemps, n_step, beta_min, seed=0, discard=None, device=0):
+def run_tempered(grb, x, y, yerr, n_walk, ntemps, n_step, beta_min, seed=0, discard=None, device=0, moves=None):
     """A parallel-tempered run (``TemperedEnsemble``): ``ntemps`` temperatures on a geometric ladder from 1 down to
     ``beta_min``, ``n_walk`` walkers each, every temperature started from ``initial_ball``.  Returns the ``RunResult``
     of the cold chain (``write_outputs`` and ``posterior_summary_device`` take it as they take ``run``'s) with
     ``log_evidence`` / ``log_evidence_err`` (``thermodynamic_log_evidence`` over the steps after ``discard``; None:
     the first half), ``betas``, ``swap_acceptance`` [ntemps - 1] and the device-resident cold chain and lnp of every
     temperature (``chain_device``, ``lnp_device``) attached.  The ladder should reach the prior:
-    ``beta_min * <lnL>_{beta_min}`` is the part of ln Z the hottest temperature stands for."""
+    ``beta_min * <lnL>_{beta_min}`` is the part of ln Z the hottest temperature stands for.  ``moves`` as for ``run``."""
     from .. import _capi as A
     from ..engine import Likelihood, time_grid
     from ..sampler import TemperedEnsemble, geometric_betas, thermodynamic_log_evidence
@@ -109,7 +110,7 @@ def run_tempered(grb, x, y, yerr, n_walk, ntemps, n_step, beta_min, seed=0, disc
     p0 = np.stack([initial_ball(grb, n_walk, rng=rng) for _ in range(ntemps)])
     lk = Likelihood(A.script_model_spec(), time_grid(None), x, y, yerr, lower, upper, device=device)
     try:
-        ens = TemperedEnsemble.from_likelihood(lk, n_walk, p0.shape[2], betas, a=2.0, seed=seed)
+        ens = TemperedEnsemble.from_likelihood(lk, n_walk, p0.shape[2], betas, a=2.0, seed=seed, moves=moves)
         ens.initialise(p0)
         chain, lnp = ens.run(n_step, store=True)
         log_z, dlog_z = thermodynamic_log_evidence(betas, lnp, discard=discard)
