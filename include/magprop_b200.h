@@ -256,13 +256,16 @@ int mp_tempered_swap(const mp_ensemble* e, int32_t ntemps, const double* betas, 
                      int32_t* d_swap_accepted, void* stream);
 
 /* ---- emcee 3's moves= (StretchMove, DEMove, DESnookerMove) --------------------------------------------------
- * The half-steps above with a weighted mix of moves instead of the stretch move of e->a.  Per half-step, with the
- * existing split: mover x is moved against the complement half C, |C| = Nc (in a tempered ensemble, the complement
- * within the mover's own temperature).  hs = 2*step + split is the half-step counter, me the mover's row, and
- * idx(u, m) = min((int)(u*m), m-1) the partner rule.
- *   Random draws: two Philox4x32-10 blocks per mover beyond the stretch move's, A = counter (hs, me, 4) and
- *     B = counter (hs, me, 5), keyed by the seed; words 0-3 keep their meaning, so the stretch move's stream does not
- *     change.
+ * The half-steps above with a weighted mix of moves; mp_ensemble_half_step and mp_tempered_half_step are these with
+ * the one move MP_MOVE_STRETCH of e->a.  Per half-step, with the existing split: mover x is moved against the
+ * complement half C, |C| = Nc (in a tempered ensemble, the complement within the mover's own temperature).
+ * hs = 2*step + split is the half-step counter, me the mover's row, and idx(u, m) = min((int)(u*m), m-1) the partner
+ * rule.  Every move proposes q with the log of its Hastings factor, ln f, and draws its accept uniform ua from
+ * Philox4x32-10 blocks keyed by the seed: the stretch move from counter (hs, me, 0) and (hs, me, 1), the others from
+ * A = counter (hs, me, 4) and B = counter (hs, me, 5).
+ *   MP_MOVE_STRETCH (a; Goodman & Weare 2010): uz = u01(S0,S1), up = u01(S2,S3) of block S = (hs, me, 0),
+ *     ua = u01 of words 0,1 of (hs, me, 1).  z = ((a-1)*uz + 1)^2 / a, partner c = C[idx(up, Nc)],
+ *     q_c = c_c - (c_c - x_c)*z, ln f = (ndim-1) * log(z).
  *   MP_MOVE_DE (gamma0, sigma; Nelson et al. 2014): uj = u01(A0,A1), uk = u01(A2,A3), ug = u01(B0,B1),
  *     ua = u01(B2,B3).  Partners are an ordered pair of distinct positions: j = idx(uj, Nc), then k = idx(uk, Nc-1),
  *     and k += 1 if k >= j.  g = gamma0 * (1 + s3*(2*ug - 1)) with s3 = sigma*sqrt(3) (host); gamma0 = 0 means
@@ -275,9 +278,8 @@ int mp_tempered_swap(const mp_ensemble* e, int32_t ntemps, const double* betas, 
  *     dd = sum_c (r1_c - r2_c)*e_c (ascending c, rounded term by term); q = x + (gammas*dd/ee)*e;
  *     ln f = (0.5*(ndim-1)) * log(sum_c (q_c - z_c)^2 / ee).  ee == 0: q = x and ln f = 0; a zero numerator gives
  *     ln f = -inf (rejected).
- *   MP_MOVE_STRETCH (a): exactly the stretch move of mp_ensemble_half_step.
  *   Accept: ((ln f + lq) - lx) > log(ua), lq and lx weighted by beta_t in a tempered ensemble.  Status, bad_rows,
- *     counters and pack_out as for the stretch move.
+ *     counters and pack_out as described for mp_ensemble.
  *   Which move runs: one per MCMC step, for both half-steps and every temperature.  u = u01 of Philox counter
  *     (step, 0, 6); the move is the first k with u*W < cum_k, W and cum_k the sequential sums of the weights.
  * Checked on the host before any device work (MP_ERR_BAD_ARG): moves non-null, 1 <= n_moves <= MP_MAX_MOVES, known

@@ -204,26 +204,25 @@ __global__ void order_scatter_kernel(int W, const int* __restrict__ key, int* __
 }
 
 // The ensemble move wrapped around an evaluation (mp_stretch_half_step / mp_ensemble_half_step / the *_moves_ entry
-// points).  The stretch move:
-//   z = ((a-1) u + 1)^2 / a ; q = c - (c - s) z ; accept iff (ndim-1) ln z + lp(q) - lp(s) > ln u'
-// (Goodman & Weare 2010; emcee's RedBlueMove); tempered: beta_t lp(q) - beta_t lp(s).  `kind` may instead be
-// differential evolution or its snooker update (include/magprop_b200.h, mp_move), whose proposals leave the log of
-// their Hastings factor in `lnf`.  One kind per launch.  setup_kernel forms the proposals, the reduce kernels accept.
+// points).  `kind` is the stretch move (Goodman & Weare 2010; emcee's RedBlueMove), differential evolution or its
+// snooker update (include/magprop_b200.h, mp_move); one kind per launch.  Every kind has one contract: the proposal
+// (setup_kernel, or order_key_kernel on an ordered launch) leaves q in `prop` and ln f, the log of its Hastings
+// factor, in `lnf`; the accept step (the reduce kernels, deliver) takes
+//   accept iff ln f + lp(q) - lp(s) > ln u,  u = accept_uniform(kind, ...)
+// tempered: beta_t lp(q) - beta_t lp(s).
 struct Move {
   double* coords;        // [nwalkers][ndim], updated in place
   double* lnp;           // [nwalkers]
   // who moves against whom: explicit index lists (mp_stretch_half_step) ...
   const int* active;     // [n_active] walkers to move (disjoint from complement), or null
   const int* complement; // [n_complement]
-  // ... or positions of the ensemble order (mp_ensemble_half_step): mover i is walker P(pos0 + i), its
-  // partner is drawn from P(cpos0 + [0, n_complement))
+  // ... or positions of the ensemble order, with T temperatures of n walkers (T = 1 without a ladder): mover
+  // mover0 + i is the tempered_mover of positions pos0 + [0, n/2), its partner is drawn from its own temperature's
+  // P(cpos0 + [0, n_complement))
   SplitPerm perm;
   int pos0, cpos0;
   int n_complement;
-  // ... or a tempered ensemble (mp_tempered_half_step; null on every other path): mover mover0 + i is the
-  // tempered_mover of the positions above, its partner comes from its own temperature, and the accept test
-  // weighs the log-probabilities by betas[t]
-  const double* betas;
+  const double* betas;   // [T] the accept test weighs the log-probabilities by betas[t] (null: untempered)
   int mover0;
   double a;
   uint64_t seed, step;   // step: the half-step counter (RNG counter word)
@@ -249,13 +248,9 @@ struct Move {
   int bad_capacity;
   int kind;              // MP_MOVE_STRETCH (a above), MP_MOVE_DE (g0 = gamma0, s3 = sigma sqrt 3), MP_MOVE_DE_SNOOKER (gammas)
   double g0, s3, gammas;
-  double* lnf;           // [n_active] ln of each proposal's Hastings factor (DE, snooker; work space next to prop)
+  double* lnf;           // [n_active] ln of each proposal's Hastings factor (work space next to prop)
 };
 
-struct Draw {
-  double z, ua;
-  int me, partner, pj, t;
-};
 // Which rank's replica holds walker w's current row (see Move).
 __device__ __forceinline__ int home_before_this_step(const Move& m, int w) {
   if (m.synced) return m.rank;
@@ -267,39 +262,18 @@ __device__ __forceinline__ const double* replica_coords(const Move& m, int home)
 __device__ __forceinline__ const double* replica_lnp(const Move& m, int home) {
   return home == m.rank ? m.lnp : m.peer_lnp[home < m.rank ? home : home - 1];
 }
-// The row mover i moves, and its temperature (0 unless tempered).
+// The row mover i moves, and its temperature (0 without a ladder).
 __device__ __forceinline__ int mover_row(const Move& m, int i, int& t) {
   t = 0;
-  if (m.betas) {
-    const TemperedMover tm = tempered_mover(m.perm, (uint32_t)m.pos0, (uint32_t)(m.mover0 + i));
-    t = (int)tm.t;
-    return (int)tm.row;
-  }
-  return m.active ? m.active[i] : (int)perm_at(m.perm, (uint32_t)(m.pos0 + i));
+  if (m.active) return m.active[i];
+  const TemperedMover tm = tempered_mover(m.perm, (uint32_t)m.pos0, (uint32_t)(m.mover0 + i));
+  t = (int)tm.t;
+  return (int)tm.row;
 }
 // The row at position pj of the complement of a mover of temperature t.
 __device__ __forceinline__ int partner_row(const Move& m, int t, int pj) {
-  if (m.betas) return (int)tempered_partner(m.perm, (uint32_t)m.cpos0, (uint32_t)t, (uint32_t)pj);
-  return m.complement ? m.complement[pj] : (int)perm_at(m.perm, (uint32_t)(m.cpos0 + pj));
-}
-// counter = (half-step, walker); two Philox blocks give u_z, u_partner, u_accept.  (Tempered: walker = global row.)
-__device__ __forceinline__ Draw draw_for(const Move& m, int i) {
-  Draw d;
-  d.me = mover_row(m, i, d.t);
-  const Philox r0 = philox4x32_10((uint32_t)m.step, (uint32_t)(m.step >> 32), (uint32_t)d.me, 0u,
-                                  (uint32_t)m.seed, (uint32_t)(m.seed >> 32));
-  const Philox r1 = philox4x32_10((uint32_t)m.step, (uint32_t)(m.step >> 32), (uint32_t)d.me, 1u,
-                                  (uint32_t)m.seed, (uint32_t)(m.seed >> 32));
-  const double uz = u01(r0.c[0], r0.c[1]);
-  const double up = u01(r0.c[2], r0.c[3]);
-  d.ua = u01(r1.c[0], r1.c[1]);
-  const double zr = __dadd_rn(__dmul_rn(m.a - 1.0, uz), 1.0);
-  d.z = __ddiv_rn(__dmul_rn(zr, zr), m.a);
-  int pj = (int)(up * m.n_complement);
-  if (pj >= m.n_complement) pj = m.n_complement - 1;
-  d.partner = partner_row(m, d.t, pj);
-  d.pj = pj;
-  return d;
+  if (m.complement) return m.complement[pj];
+  return (int)tempered_partner(m.perm, (uint32_t)m.cpos0, (uint32_t)t, (uint32_t)pj);
 }
 
 constexpr int kRecWords = (int)(sizeof(WalkerRec) / 8);
@@ -400,23 +374,33 @@ __device__ __noinline__ void propose_de(const Move& m, int i, int ndim, double* 
   m.lnf[i] = lnf;
 }
 
+// The proposal of mover i: q in th and m.prop[i], ln f in m.lnf[i].  The stretch move draws u_z and u_partner from
+// Philox counter (half-step, row, 0):  z = ((a-1) u_z + 1)^2 / a,  q = c - (c - s) z,  ln f = (ndim-1) ln z.
 __device__ __forceinline__ void propose(const Move& m, int i, int ndim, double* th) {
   if (m.kind != MP_MOVE_STRETCH) {
     propose_de(m, i, ndim, th);
     return;
   }
-  const Draw d = draw_for(m, i);
+  int t;
+  const int me = mover_row(m, i, t);
+  const Philox r = philox4x32_10((uint32_t)m.step, (uint32_t)(m.step >> 32), (uint32_t)me, 0u,
+                                 (uint32_t)m.seed, (uint32_t)(m.seed >> 32));
+  const double zr = __dadd_rn(__dmul_rn(m.a - 1.0, u01(r.c[0], r.c[1])), 1.0);
+  const double z = __ddiv_rn(__dmul_rn(zr, zr), m.a);
+  const int pj = (int)pick_index(u01(r.c[2], r.c[3]), (uint32_t)m.n_complement);
+  const int partner = partner_row(m, t, pj);
   const double* pc = m.coords;
   if (m.n_peers > 0) {
-    fetch_mover(m, d.me, ndim);
-    pc = partner_replica(m, d.pj, d.partner);
+    fetch_mover(m, me, ndim);
+    pc = partner_replica(m, pj, partner);
   }
   for (int c = 0; c < ndim; ++c) {
-    const double cc = pc[(size_t)d.partner * ndim + c];
-    const double x = m.coords[(size_t)d.me * ndim + c];
-    th[c] = __dadd_rn(cc, -__dmul_rn(__dadd_rn(cc, -x), d.z));   // no FMA contraction: reproducible on the host
+    const double cc = pc[(size_t)partner * ndim + c];
+    const double x = m.coords[(size_t)me * ndim + c];
+    th[c] = __dadd_rn(cc, -__dmul_rn(__dadd_rn(cc, -x), z));   // no FMA contraction: reproducible on the host
     m.prop[(size_t)i * ndim + c] = th[c];
   }
+  m.lnf[i] = __dmul_rn(ndim - 1.0, log(z));
 }
 
 // Large launches, before the setup: every walker's bucket key and the bucket histogram (MOVE: the proposals are
@@ -447,7 +431,7 @@ __global__ void __launch_bounds__(128) order_key_kernel(const __grid_constant__ 
   }
 }
 
-// MOVE = false: walker i's parameters are theta[i][:].  MOVE = true: walker i is mover i of a stretch-move
+// MOVE = false: walker i's parameters are theta[i][:].  MOVE = true: walker i is mover i of an ensemble-move
 // half-step and its parameters are the proposal q.  One thread per SLOT (= walker unless the launch is ordered).
 template <bool MOVE>
 __global__ void __launch_bounds__(128, 4) setup_kernel(const __grid_constant__ Problem p, const __grid_constant__ Work k,
@@ -664,7 +648,7 @@ __device__ __forceinline__ bool stage_data(const DataView& g, DataView& s, doubl
   return true;
 }
 
-// Where a finished evaluation goes: the caller's arrays, or the accept step of the stretch move.
+// Where a finished evaluation goes: the caller's arrays, or the accept step of the ensemble move.
 struct Sink {
   double* lnp;     // [W]
   int* status;     // [W] or null
@@ -683,17 +667,9 @@ __device__ __forceinline__ void deliver(const Problem& p, const Work& k, const S
     return;
   }
   const int ndim = p.ndim;
-  int me, t;
-  double lnf, ua;                            // ln of the Hastings factor, the accept draw
-  if (m.kind == MP_MOVE_STRETCH) {
-    const Draw d = draw_for(m, i);
-    me = d.me; t = d.t; ua = d.ua;
-    lnf = __dmul_rn(ndim - 1.0, log(d.z));
-  } else {
-    me = mover_row(m, i, t);
-    ua = move_draws(m.seed, m.step, (uint32_t)me).u[3];
-    lnf = m.lnf[i];
-  }
+  int t;
+  const int me = mover_row(m, i, t);
+  const double ua = accept_uniform(m.kind, m.seed, m.step, (uint32_t)me);
   const double* q = m.prop + (size_t)i * ndim;
   const double lp_old = m.lnp[me];
   double lq = lp_new, lx = lp_old;           // tempered: beta_t lp (lnp stays untempered)
@@ -702,7 +678,7 @@ __device__ __forceinline__ void deliver(const Problem& p, const Work& k, const S
     lq = __dmul_rn(b, lp_new);
     lx = __dmul_rn(b, lp_old);
   }
-  const double lnpdiff = __dadd_rn(__dadd_rn(lnf, lq), -lx);
+  const double lnpdiff = __dadd_rn(__dadd_rn(m.lnf[i], lq), -lx);
   const bool accept = lnpdiff > log(ua);
   if (accept) {
     for (int c = 0; c < ndim; ++c) m.coords[(size_t)me * ndim + c] = q[c];
@@ -1097,7 +1073,7 @@ static int ensure_work(mp_handle::Lane& L, int S, int Nn, int ndim_prop, Work& k
 // One evaluation of W walkers: setup -> advance (explicit, then the stiff queue) -> reduce, slab by slab.
 //   MOVE = false: parameters from d_theta [W][ndim]; results to `sink` (lnprob), `out` (model at data
 //                 [W][D], or curves [W][3][Nn]) and `state` (curves, optional)
-//   MOVE = true : the W movers of a stretch-move half-step described by `mv`
+//   MOVE = true : the W movers of an ensemble-move half-step described by `mv`
 template <int MODE, bool MOVE>
 static int launch_eval(mp_handle* h, const Problem& p, const double* d_theta, int W, Sink sink, double* out, double* state,
                        const Move* mv, cudaStream_t stream, int lane = -1) {
@@ -1124,8 +1100,7 @@ static int launch_eval(mp_handle* h, const Problem& p, const double* d_theta, in
     Move ms = m;
     if (MOVE) {
       if (ms.active) ms.active += i0;
-      else if (ms.betas) ms.mover0 += i0;     // (a tempered slab may span temperatures: offset the mover, not the position)
-      else ms.pos0 += i0;
+      else ms.mover0 += i0;     // (a tempered slab may span temperatures: offset the mover, not the position)
       ms.prop = Lp->prop.get();
       ms.lnf = Lp->lnf.get();
       if (ms.pack_out) ms.pack_out += (size_t)i0 * (ndim + 1);

@@ -147,6 +147,13 @@ MP_RNG_HD MoveDraws move_draws(uint64_t seed, uint64_t hs, uint32_t me) {
   d.u[3] = u01(b.c[2], b.c[3]);
   return d;
 }
+// The accept draw u of mover `me` (row) at half-step hs, ln u compared with ln f + lp(q) - lp(s): the stretch move's
+// (kind 0) from Philox counter (hs, me, 1), words 0-1; DE's and snooker's from block B of move_draws, = u[3].
+MP_RNG_HD double accept_uniform(int kind, uint64_t seed, uint64_t hs, uint32_t me) {
+  const Philox r = philox4x32_10((uint32_t)hs, (uint32_t)(hs >> 32), me, kind == 0 ? 1u : 5u, (uint32_t)seed,
+                                 (uint32_t)(seed >> 32));
+  return kind == 0 ? u01(r.c[0], r.c[1]) : u01(r.c[2], r.c[3]);
+}
 // DE: an ordered pair of distinct positions of the complement (nc >= 2).
 MP_RNG_HD void de_pair(double uj, double uk, uint32_t nc, uint32_t* j, uint32_t* k) {
   *j = pick_index(uj, nc);

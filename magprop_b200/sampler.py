@@ -276,11 +276,8 @@ class CudaBackend:
         self._own = []
 
     def half_step(self, ens, step, split):
-        if ens.moves is None:
-            self.A.check(self.lib.mp_ensemble_half_step(self.lik._h, C.byref(ens.desc), step, split, self.stream() or None))
-        else:
-            self.A.check(self.lib.mp_ensemble_moves_half_step(self.lik._h, C.byref(ens.desc), C.addressof(ens._moves_c),
-                                                              len(ens._moves_c), step, split, self.stream() or None))
+        self.A.check(self.lib.mp_ensemble_moves_half_step(self.lik._h, C.byref(ens.desc), C.addressof(ens._moves_c),
+                                                          len(ens._moves_c), step, split, self.stream() or None))
 
     def unpack(self, ens, step, split, gathered):
         self.A.check(self.lib.mp_ensemble_unpack(C.byref(ens.desc), step, split, gathered.data_ptr(), self.stream() or None))
@@ -296,13 +293,9 @@ class CudaBackend:
         self.lik.lnprob_device(ens.coords.data_ptr(), ens.coords.shape[0], ens.ndim, ens.lnp.data_ptr(), 0, 0, self.stream())
 
     def tempered_half_step(self, ens, step, split):
-        if ens.moves is None:
-            self.A.check(self.lib.mp_tempered_half_step(self.lik._h, C.byref(ens.desc), ens.ntemps, self.A.ptr(ens.betas),
-                                                        step, split, self.stream() or None))
-        else:
-            self.A.check(self.lib.mp_tempered_moves_half_step(self.lik._h, C.byref(ens.desc), ens.ntemps,
-                                                              self.A.ptr(ens.betas), C.addressof(ens._moves_c),
-                                                              len(ens._moves_c), step, split, self.stream() or None))
+        self.A.check(self.lib.mp_tempered_moves_half_step(self.lik._h, C.byref(ens.desc), ens.ntemps, self.A.ptr(ens.betas),
+                                                          C.addressof(ens._moves_c), len(ens._moves_c), step, split,
+                                                          self.stream() or None))
 
     def tempered_swap(self, ens, step):
         self.A.check(self.lib.mp_tempered_swap(C.byref(ens.desc), ens.ntemps, self.A.ptr(ens.betas), step,
@@ -315,8 +308,8 @@ class DeviceEnsemble:
     ``backend`` performs the half-steps: ``CudaBackend`` on a GPU (see ``from_likelihood``); the tests inject a
     NumPy double so the sharding / exchange logic runs under gloo on the CPU.
 
-    ``moves`` (emcee 3's argument, see ``move_table``): None runs the stretch move of scale ``a``; otherwise one of the
-    given moves per step, chosen by weight from the seed, and ``a`` is unused.
+    ``moves`` (emcee 3's argument, see ``move_table``): one of the given moves per step, chosen by weight from the
+    seed; None is ``StretchMove(a)``, and otherwise ``a`` is unused.
     """
 
     BAD_CAPACITY = 4096
@@ -329,7 +322,7 @@ class DeviceEnsemble:
         from . import _capi as A
         if nwalkers % 2 or nwalkers < 2 * ndim:
             raise ValueError("nwalkers must be even and at least 2*ndim")
-        self.moves, self._moves_c = (None, None) if moves is None else move_table(moves, nwalkers // 2)
+        self.moves, self._moves_c = move_table(StretchMove(a) if moves is None else moves, nwalkers // 2)
         self.torch, self.backend = torch, backend
         self.nwalkers, self.ndim, self.a, self.seed = nwalkers, ndim, float(a), int(seed)
         self.randomize_split = bool(randomize_split)
@@ -491,14 +484,18 @@ class DeviceEnsemble:
             self.backend.unpack(self, self.step, split, self.gathered)
 
     def run(self, nsteps, store=False):
-        """nsteps stretch-move steps (2 half-steps each).  Returns the chain
+        """nsteps steps (2 half-steps each).  Returns the chain
         [nsteps, nwalkers, ndim] and lnprob [nsteps, nwalkers] when store=True."""
-        t = self.torch
-        chain = t.empty((nsteps, self.nwalkers, self.ndim), dtype=t.float64, device=self.device) if store else None
-        lps = t.empty((nsteps, self.nwalkers), dtype=t.float64, device=self.device) if store else None
+        chain, lps = self._buffers(nsteps) if store else (None, None)
         self._advance(nsteps, chain, lps, 0)
         self.sync()
         return (chain, lps) if store else None
+
+    def _buffers(self, nsteps):
+        """Empty chain and lnprob buffers of ``nsteps`` steps, in the shapes ``run`` returns."""
+        t = self.torch
+        return (t.empty((nsteps, self.nwalkers, self.ndim), dtype=t.float64, device=self.device),
+                t.empty((nsteps, self.nwalkers), dtype=t.float64, device=self.device))
 
     def _advance(self, nsteps, chain=None, lps=None, row=0):
         """nsteps steps; with ``chain``, rows row, row + 1, ... of chain / lps receive the state after each step."""
@@ -526,8 +523,7 @@ class DeviceEnsemble:
         if max_steps < 1 or check_every < 1:
             raise ValueError("max_steps and check_every must be positive")
         t = self.torch
-        chain = t.empty((max_steps, self.nwalkers, self.ndim), dtype=t.float64, device=self.device)
-        lps = t.empty((max_steps, self.nwalkers), dtype=t.float64, device=self.device)
+        chain, lps = self._buffers(max_steps)
         history, tau_prev, converged, n = [], np.full(self.ndim, np.inf), False, 0
         while n < max_steps and not converged:
             k = min(check_every, max_steps - n)
@@ -681,11 +677,13 @@ class TemperedEnsemble(DeviceEnsemble):
         """nsteps tempered steps: half-steps 0 and 1 of every temperature, then the swaps.  With ``store`` returns the
         cold chain [nsteps, nwalkers, ndim] and the lnp of every temperature [nsteps, ntemps, nwalkers], both as they
         stand after the step's swaps."""
-        t = self.torch
-        chain = t.empty((nsteps, self.nwalkers, self.ndim), dtype=t.float64, device=self.device) if store else None
-        lps = t.empty((nsteps, self.ntemps, self.nwalkers), dtype=t.float64, device=self.device) if store else None
+        chain, lps = self._buffers(nsteps) if store else (None, None)
         self._advance(nsteps, chain, lps, 0)
         return (chain, lps) if store else None
+
+    def _buffers(self, nsteps):
+        chain, _ = super()._buffers(nsteps)
+        return chain, self.torch.empty((nsteps, self.ntemps, self.nwalkers), dtype=self.torch.float64, device=self.device)
 
     def _advance(self, nsteps, chain=None, lps=None, row=0):
         for it in range(nsteps):
@@ -720,21 +718,11 @@ def run_concurrently(ensembles, nsteps, store=False):
     streams = [torch.cuda.Stream(device=e.device) for e in ensembles]
     for e, st in zip(ensembles, streams):
         st.wait_stream(torch.cuda.current_stream(e.device))
-    out = []
-    if store:
-        for e in ensembles:
-            out.append((torch.empty((nsteps, e.nwalkers, e.ndim), dtype=torch.float64, device=e.device),
-                        torch.empty((nsteps, e.nwalkers), dtype=torch.float64, device=e.device)))
+    out = [e._buffers(nsteps) if store else (None, None) for e in ensembles]
     for it in range(nsteps):
-        for k, (e, st) in enumerate(zip(ensembles, streams)):
+        for e, st, (chain, lps) in zip(ensembles, streams, out):
             with torch.cuda.stream(st):
-                e._half(0)
-                e._half(1)
-                e.step += 1
-                if store:
-                    e.sync()
-                    out[k][0][it].copy_(e.coords)
-                    out[k][1][it].copy_(e.lnp)
+                e._advance(1, chain, lps, it)
     for e, st in zip(ensembles, streams):
         torch.cuda.current_stream(e.device).wait_stream(st)
     return out if store else None

@@ -11,7 +11,7 @@ import numpy as np
 import pytest
 
 from conftest import has_gpu, relerr
-import stretch_ref as R
+import ensemble_ref as E
 from magprop_b200.sampler import DeviceEnsemble
 from magprop_b200.synthetic import synth_mcmc as S
 
@@ -132,7 +132,7 @@ def test_window_driver_matches_integrated_time_bit_for_bit():
 def _converging(dist=None, max_steps=3000):
     rng = np.random.RandomState(5)
     p0 = rng.randn(32, 3)
-    ens = DeviceEnsemble(R.NumpyBackend(gauss_lnprob), 32, 3, a=2.0, seed=11, device="cpu", dist=dist)
+    ens = DeviceEnsemble(E.NumpyBackend(gauss_lnprob), 32, 3, a=2.0, seed=11, device="cpu", dist=dist)
     ens.set_state(p0, gauss_lnprob(p0))
     chain, lps, hist, conv = ens.run_until_converged(max_steps, check_every=50, n_tau=10, tau_rtol=0.1)
     return chain.numpy(), lps.numpy(), hist, conv, ens.step
@@ -141,7 +141,7 @@ def _converging(dist=None, max_steps=3000):
 def _fresh_run(nsteps):
     rng = np.random.RandomState(5)
     p0 = rng.randn(32, 3)
-    ens = DeviceEnsemble(R.NumpyBackend(gauss_lnprob), 32, 3, a=2.0, seed=11, device="cpu")
+    ens = DeviceEnsemble(E.NumpyBackend(gauss_lnprob), 32, 3, a=2.0, seed=11, device="cpu")
     ens.set_state(p0, gauss_lnprob(p0))
     chain, lps = ens.run(nsteps, store=True)
     return chain.numpy(), lps.numpy()

@@ -16,8 +16,7 @@ import numpy as np
 import pytest
 
 from conftest import relerr
-import stretch_ref as R
-import tempered_ref as TR
+import ensemble_ref as E
 from magprop_b200 import _capi as A
 from magprop_b200.engine import Likelihood, time_grid
 from oracle import magprop_oracle as O
@@ -318,7 +317,7 @@ def test_ensemble_half_steps_across_slabs(built, wide):
     """A 65 536-walker ensemble on the wide dataset moves 32 768 walkers per half-step: 2 slabs.  Two steps equal
     the restatement driven by single-slab host batches, bit for bit; fixed halves equal the explicit-list call."""
     import torch
-    from magprop_b200.sampler import DeviceEnsemble
+    from magprop_b200.sampler import DeviceEnsemble, StretchMove
     lk = script_handle(*wide)
     rng = np.random.RandomState(404)
     n = 65536
@@ -337,10 +336,11 @@ def test_ensemble_half_steps_across_slabs(built, wide):
     torch.cuda.synchronize()
     assert lk.kernels_launched() - k0 >= 4 * 8
     for it in range(2):
-        order = R.ensemble_order(n, 99, it)
+        order = E.ensemble_order(n, 99, it)
         for split in (0, 1):
-            R.half_step(coords, lnp, order[split * half:(split + 1) * half], order[(1 - split) * half:(2 - split) * half],
-                        2.0, 99, 2 * it + split, fn, acc)
+            E.half_step(coords, lnp, order[split * half:(split + 1) * half], np.zeros(half, np.int64),
+                        order[None, (1 - split) * half:(2 - split) * half], StretchMove(2.0), 99, 2 * it + split, fn,
+                        accepted=acc)
         assert np.array_equal(chain[it].cpu().numpy(), coords)
         assert same(lps[it].cpu().numpy(), lnp)
     assert np.array_equal(ens.accepted.cpu().numpy(), acc)
@@ -363,7 +363,7 @@ def test_tempered_half_steps_across_slabs(built, wide):
     """T = 3 x n = 16 384 on the wide dataset: 24 576 movers per half-step, so the slab boundary falls inside the
     hottest temperature.  Two steps with swaps equal the restatement driven by single-slab host batches."""
     import torch
-    from magprop_b200.sampler import TemperedEnsemble, geometric_betas
+    from magprop_b200.sampler import StretchMove, TemperedEnsemble, geometric_betas
     lk = script_handle(*wide)
     T, n = 3, 16384
     assert slab_bound(10001) < T * n // 2
@@ -383,10 +383,11 @@ def test_tempered_half_steps_across_slabs(built, wide):
             k0 = lk.kernels_launched()
             ens.backend.tempered_half_step(ens, step, split)
             assert lk.kernels_launched() - k0 >= 8
-            TR.half_step(coords, lnp, betas, n, split, 2.0, 21, step, fn, acc)
+            t, rows, comp = E.tempered_rows(n, T, 21, step, split)
+            E.half_step(coords, lnp, rows, t, comp, StretchMove(2.0), 21, 2 * step + split, fn, betas=betas, accepted=acc)
             assert np.array_equal(ens.coords.cpu().numpy(), coords) and same(ens.lnp.cpu().numpy(), lnp)
         ens.backend.tempered_swap(ens, step)
-        TR.swap(coords, lnp, betas, n, 21, step, swaps)
+        E.swap(coords, lnp, betas, n, 21, step, swaps)
         ens.step += 1
         torch.cuda.synchronize()
         assert np.array_equal(ens.coords.cpu().numpy(), coords) and same(ens.lnp.cpu().numpy(), lnp)

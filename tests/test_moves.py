@@ -1,23 +1,21 @@
 """emcee 3's moves on the device ensembles: the NumPy restatement of the DE and snooker moves samples known Gaussians,
 the host-compiled draws, partner picks and move choice equal it, the mp_move layout and every argument check of the
 two entry points hold without a GPU, and a sharded run equals a single one under gloo (CPU); the kernels equal the
-restatement bit for bit across the launch paths, a one-stretch-move list equals the default call, streams do not
-matter, and stretch and the mix agree on the Humped posterior (GPU)."""
+restatement bit for bit across the launch paths, the plain stretch-move entry points equal the sampler's default
+ensembles, streams do not matter, and stretch and the mix agree on the Humped posterior (GPU)."""
 import ctypes as C
 import os
 
 import numpy as np
 import pytest
 
-import moves_ref as MR
-import stretch_ref as R
-import tempered_ref as TR
+import ensemble_ref as E
 from conftest import ROOT
 from magprop_b200.sampler import DEMove, DESnookerMove, DeviceEnsemble, StretchMove, TemperedEnsemble, move_table
 from magprop_b200.synthetic.synth_mcmc import integrated_time
 
 MIX = [(DEMove(), 0.8), (DESnookerMove(), 0.2)]
-KINDS = {"de": DEMove(), "snooker": DESnookerMove(), "mix": MIX}
+KINDS = {"stretch": None, "de": DEMove(), "snooker": DESnookerMove(), "mix": MIX}
 
 
 # ---- the restatement samples known Gaussians ---------------------------------------------------------------
@@ -40,7 +38,7 @@ def sample_gaussian(d, moves, nsteps=6000, nwalkers=32, seed=1):
     mu, cov, lnprob = gaussian(d)
     rng = np.random.RandomState(seed)
     p0 = mu + 0.1 * rng.multivariate_normal(np.zeros(d), cov, size=nwalkers)
-    ens = DeviceEnsemble(MR.NumpyMovesBackend(lnprob), nwalkers, d, seed=seed, device="cpu", moves=moves)
+    ens = DeviceEnsemble(E.NumpyBackend(lnprob), nwalkers, d, seed=seed, device="cpu", moves=moves)
     ens.set_state(p0, lnprob(p0))
     chain, _ = ens.run(nsteps, store=True)
     return mu, cov, chain.numpy()[nsteps // 4:], ens
@@ -68,21 +66,6 @@ def test_restatement_samples_correlated_gaussians(kind, d):
     assert 0.05 < acc < 0.95, acc
 
 
-def test_restatement_of_the_stretch_move_in_a_list_is_the_stretch_move():
-    """[StretchMove(a)] through the moves restatement == the stretch restatement (moves=None), plain and tempered."""
-    _, _, lnprob = gaussian(3)
-    p0 = np.random.RandomState(2).randn(16, 3) * [1.0, 30.0, 1000.0]
-    out = []
-    for moves in (None, StretchMove(2.5)):
-        e = DeviceEnsemble(MR.NumpyMovesBackend(lnprob), 16, 3, a=2.5, seed=4, device="cpu", moves=moves)
-        e.set_state(p0, lnprob(p0))
-        t = TemperedEnsemble(MR.NumpyMovesBackend(lnprob), 16, 3, [1.0, 0.3, 0.1], a=2.5, seed=4, device="cpu", moves=moves)
-        t.initialise(p0)
-        out.append((e.run(30, store=True)[0].numpy(), e.accepted.numpy().copy(), t.run(30)[1].numpy()))
-    for a, b in zip(*out):
-        assert np.array_equal(a, b)
-
-
 # ---- host-compiled helpers == the restatement --------------------------------------------------------------
 @pytest.fixture(scope="module")
 def moves_rng(tmp_path_factory):
@@ -94,6 +77,8 @@ def moves_rng(tmp_path_factory):
     lib = C.CDLL(so)
     vp = C.c_void_p
     lib.mr_move_draws.argtypes = [C.c_ulonglong, C.c_ulonglong, C.c_uint, vp]
+    lib.mr_accept_uniform.argtypes = [C.c_int, C.c_ulonglong, C.c_ulonglong, C.c_uint]
+    lib.mr_accept_uniform.restype = C.c_double
     lib.mr_de_pair.argtypes = [C.c_double, C.c_double, C.c_uint, vp]
     lib.mr_snooker_triple.argtypes = [C.c_double, C.c_double, C.c_double, C.c_uint, vp]
     lib.mr_choose_move.argtypes = [C.c_ulonglong, C.c_ulonglong, vp, C.c_int]
@@ -109,21 +94,25 @@ def test_host_compiled_draws_and_partner_picks_match_the_restatement(moves_rng):
         if it % 3 == 0:
             seed, hs = it, it // 3
         moves_rng.mr_move_draws(seed, hs, row, u4.ctypes.data)
-        want = [float(w[0]) for w in MR.move_draws(seed, hs, np.array([row]))]
+        want = [float(w[0]) for w in E.move_draws(seed, hs, np.array([row]))]
         assert u4.tolist() == want, (seed, hs, row)
+        for kind in (E.STRETCH, E.DE, E.SNOOKER):
+            ua = moves_rng.mr_accept_uniform(kind, seed, hs, row)
+            assert ua == float(E.accept_uniform(kind, seed, hs, np.array([row]))[0]), (kind, seed, hs, row)
+            assert (ua == u4[3]) == (kind != E.STRETCH), (kind, seed, hs, row)
         for nc in (2, 3, 4, 7, 1000, 1 << 20):
             moves_rng.mr_de_pair(u4[0], u4[1], nc, jk.ctypes.data)
-            j, k = MR.de_pair(np.array([u4[0]]), np.array([u4[1]]), nc)
+            j, k = E.de_pair(np.array([u4[0]]), np.array([u4[1]]), nc)
             assert (int(jk[0]), int(jk[1])) == (int(j[0]), int(k[0])) and jk[0] != jk[1] and jk.max() < nc
             if nc >= 3:
                 moves_rng.mr_snooker_triple(u4[0], u4[1], u4[2], nc, zr.ctypes.data)
-                want = [int(v[0]) for v in MR.snooker_triple(np.array([u4[0]]), np.array([u4[1]]), np.array([u4[2]]), nc)]
+                want = [int(v[0]) for v in E.snooker_triple(np.array([u4[0]]), np.array([u4[1]]), np.array([u4[2]]), nc)]
                 assert zr.tolist() == want and len(set(want)) == 3 and max(want) < nc
     # the picks cover their ranges uniformly: every ordered pair of 3, every ordered triple of 4
     u = [rng.rand(60000) for _ in range(3)]
-    j, k = MR.de_pair(u[0], u[1], 3)
+    j, k = E.de_pair(u[0], u[1], 3)
     assert np.abs(np.bincount(j * 3 + k, minlength=9)[[1, 2, 3, 5, 6, 7]] / 10000.0 - 1.0).max() < 0.06
-    z, r1, r2 = MR.snooker_triple(u[0], u[1], u[2], 4)
+    z, r1, r2 = E.snooker_triple(u[0], u[1], u[2], 4)
     counts = np.bincount(z * 16 + r1 * 4 + r2, minlength=64)
     assert (counts > 0).sum() == 24 and np.abs(counts[counts > 0] / 2500.0 - 1.0).max() < 0.12
 
@@ -136,7 +125,7 @@ def test_host_compiled_move_choice_matches_the_restatement(moves_rng):
         picks = []
         for step in list(range(500)) + [int(s) for s in rng.randint(0, 1 << 62, size=100)]:
             got = moves_rng.mr_choose_move(77, step, wa.ctypes.data, len(w))
-            assert got == MR.choose_move(77, step, w), (w, step)
+            assert got == E.choose_move(77, step, w), (w, step)
             assert w[got] > 0.0
             picks.append(got)
         freq = np.bincount(picks[:500], minlength=len(w)) / 500.0
@@ -231,12 +220,12 @@ def test_bad_moves_raise_value_error():
         with pytest.raises(ValueError):
             move_table(moves)
         with pytest.raises(ValueError):
-            DeviceEnsemble(MR.NumpyMovesBackend(lnprob), 8, 3, device="cpu", moves=moves)
+            DeviceEnsemble(E.NumpyBackend(lnprob), 8, 3, device="cpu", moves=moves)
     with pytest.raises(ValueError):
-        DeviceEnsemble(MR.NumpyMovesBackend(lnprob), 4, 2, device="cpu", moves=DESnookerMove())     # half of 2 < 3
+        DeviceEnsemble(E.NumpyBackend(lnprob), 4, 2, device="cpu", moves=DESnookerMove())     # half of 2 < 3
     with pytest.raises(ValueError):
-        TemperedEnsemble(MR.NumpyMovesBackend(lnprob), 4, 2, [1.0, 0.5], device="cpu", moves=[DEMove(), DESnookerMove()])
-    DeviceEnsemble(MR.NumpyMovesBackend(lnprob), 4, 2, device="cpu", moves=[DEMove(), (DESnookerMove(), 0.0)])
+        TemperedEnsemble(E.NumpyBackend(lnprob), 4, 2, [1.0, 0.5], device="cpu", moves=[DEMove(), DESnookerMove()])
+    DeviceEnsemble(E.NumpyBackend(lnprob), 4, 2, device="cpu", moves=[DEMove(), (DESnookerMove(), 0.0)])
     table, arr = move_table([DEMove(0.1, 1.5), (DESnookerMove(2.0), 3.0), StretchMove(3.0)])
     assert [w for _, w in table] == [1.0, 3.0, 1.0]
     assert [(m.kind, m.weight, m.a, m.gamma0, m.sigma, m.gammas) for m in arr] == [
@@ -248,7 +237,7 @@ def test_bad_moves_raise_value_error():
 def _run_mix(dist, nsteps=25):
     _, _, lnprob = gaussian(3)
     p0 = gaussian(3)[0] + np.random.RandomState(5).randn(32, 3) * [1.0, 30.0, 1000.0]
-    ens = DeviceEnsemble(MR.NumpyMovesBackend(lnprob), 32, 3, seed=11, device="cpu", dist=dist, moves=MIX)
+    ens = DeviceEnsemble(E.NumpyBackend(lnprob), 32, 3, seed=11, device="cpu", dist=dist, moves=MIX)
     ens.set_state(p0, lnprob(p0))
     chain, lps = ens.run(nsteps, store=True)
     return chain.numpy(), lps.numpy(), ens.acceptance_fraction().numpy(), ens.exchange
@@ -275,7 +264,7 @@ def test_two_rank_mix_matches_single_rank(tmp_path):
     assert str(two["exchange"]) == "allgather" and single[3] == "none"
     assert np.array_equal(two["chain"], single[0]) and np.array_equal(two["lps"], single[1])
     assert np.array_equal(two["acc"], single[2])
-    kinds = {MR.choose_move(11, s, [0.8, 0.2]) for s in range(25)}
+    kinds = {E.choose_move(11, s, [0.8, 0.2]) for s in range(25)}
     assert kinds == {0, 1}                                              # both moves ran
     assert 0.05 < single[2].mean() < 0.95
 
@@ -317,22 +306,38 @@ def _state(ens):
 @pytest.mark.gpu
 @pytest.mark.parametrize("case", ["ball64", "prior16k", "tempered"])
 def test_one_stretch_move_equals_the_default_call(built, golden, case):
-    """[StretchMove(a)] through the moves entry points == moves=None (mp_ensemble_half_step / mp_tempered_half_step),
-    bit for bit in coords, lnp, accepted, status and n_rhs."""
+    """The plain entry points mp_ensemble_half_step / mp_tempered_half_step (the stretch move of e->a), driven on an
+    ensemble's descriptor, == that ensemble run by the sampler (moves=None: [StretchMove(a)] through the moves entry
+    points), bit for bit in coords, lnp, accepted, status and n_rhs."""
     import torch
+    from magprop_b200 import _capi as A
+    from magprop_b200.sampler import geometric_betas
+    lib = A.load()
     lk = _humped(golden)
     out = []
-    for moves in (None, [StretchMove(2.0)]):
+    for plain in (False, True):
         if case == "tempered":
-            from magprop_b200.sampler import geometric_betas
-            ens = _with_n_rhs(TemperedEnsemble.from_likelihood(lk, 256, 6, geometric_betas(4, 1e-2), seed=3, moves=moves))
+            ens = _with_n_rhs(TemperedEnsemble.from_likelihood(lk, 256, 6, geometric_betas(4, 1e-2), seed=3))
             ens.initialise(np.stack([_ball(256, 1), _ball(256, 2, 0.05), _prior_wide(256, 3), _prior_wide(256, 4)]))
-            ens.run(4, store=False)
+            nsteps = 4
         else:
             n, p0 = (64, _ball(64, 1)) if case == "ball64" else (16384, _prior_wide(16384, 2))
-            ens = _with_n_rhs(DeviceEnsemble.from_likelihood(lk, n, 6, seed=3, moves=moves))
+            ens = _with_n_rhs(DeviceEnsemble.from_likelihood(lk, n, 6, seed=3))
             ens.initialise(p0)
-            ens.run(4 if n == 64 else 2)
+            nsteps = 4 if n == 64 else 2
+        if not plain:
+            ens.run(nsteps, store=False)
+        else:
+            stream = torch.cuda.current_stream().cuda_stream or None
+            for step in range(nsteps):
+                for split in (0, 1):
+                    if case == "tempered":
+                        A.check(lib.mp_tempered_half_step(lk._h, C.byref(ens.desc), ens.ntemps, A.ptr(ens.betas), step,
+                                                          split, stream))
+                    else:
+                        A.check(lib.mp_ensemble_half_step(lk._h, C.byref(ens.desc), step, split, stream))
+                if case == "tempered":
+                    ens.backend.tempered_swap(ens, step)
         torch.cuda.synchronize()
         out.append(_state(ens))
     for a, b in zip(*out):
@@ -371,29 +376,29 @@ def _check_against_restatement(lk, fn, n, p0, moves, seed, nsteps, ntemps=1, bet
     stiff, kinds = [], []
     half = n // 2
     for step in range(nsteps):
-        mv = MR.step_move(table, seed, step)
+        mv = E.step_move(table, seed, step)
         kinds.append(mv.kind)
         for split in (0, 1):
             x0 = coords.copy()
             if betas is None:
                 ens.backend.half_step(ens, step, split)
                 stiff.append(lk.last_stiff_count())          # (synchronises: the launch is complete)
-                order = R.ensemble_order(n, seed, step)
+                order = E.ensemble_order(n, seed, step)
                 rows = order[split * half:(split + 1) * half]
                 comp = order[(1 - split) * half:(2 - split) * half][None, :]
-                q, a = MR.half_step(coords, lnp, rows, np.zeros(half, np.int64), comp, mv, seed, 2 * step + split, fn,
+                q, a = E.half_step(coords, lnp, rows, np.zeros(half, np.int64), comp, mv, seed, 2 * step + split, fn,
                                     accepted=acc)
             else:
                 ens.backend.tempered_half_step(ens, step, split)
                 stiff.append(lk.last_stiff_count())
-                t, rows, comp = TR.tempered_rows(n, ntemps, seed, step, split)
-                q, a = MR.half_step(coords, lnp, rows, t, comp, mv, seed, 2 * step + split, fn, betas=betas, accepted=acc)
+                t, rows, comp = E.tempered_rows(n, ntemps, seed, step, split)
+                q, a = E.half_step(coords, lnp, rows, t, comp, mv, seed, 2 * step + split, fn, betas=betas, accepted=acc)
             got = ens.coords.cpu().numpy()
             assert np.array_equal(got, coords), (step, split, _mismatch(got, coords, x0, rows, q, a, n))
             assert np.array_equal(ens.lnp.cpu().numpy(), lnp), (step, split)
         if betas is not None:
             ens.backend.tempered_swap(ens, step)
-            TR.swap(coords, lnp, betas, n, seed, step)
+            E.swap(coords, lnp, betas, n, seed, step)
         ens.step += 1
     torch.cuda.synchronize()
     assert np.array_equal(ens.coords.cpu().numpy(), coords) and np.array_equal(ens.accepted.cpu().numpy(), acc)
@@ -402,7 +407,7 @@ def _check_against_restatement(lk, fn, n, p0, moves, seed, nsteps, ntemps=1, bet
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("kind", ["de", "snooker", "mix"])
+@pytest.mark.parametrize("kind", ["stretch", "de", "snooker", "mix"])
 def test_moves_match_the_restatement_small(built, golden, kind):
     """64 walkers from the ball (small launches: the ordered warp-per-walker reduce)."""
     lk = _humped(golden)
@@ -413,7 +418,7 @@ def test_moves_match_the_restatement_small(built, golden, kind):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("kind", ["de", "snooker", "mix"])
+@pytest.mark.parametrize("kind", ["stretch", "de", "snooker", "mix"])
 def test_moves_match_the_restatement_ordered(built, golden, kind):
     """16 384 walkers from a prior-wide start: 8192 movers per half-step, so the work list is ordered and the proposals
     are formed in order_key_kernel; the spread walkers feed the stiff queue."""
@@ -438,7 +443,7 @@ def test_moves_match_the_restatement_across_slabs(built):
     p0 = np.concatenate([LP.ball(rng, n // 2, 3e-2), LP.ball(rng, n // 2, 0.3)])[rng.permutation(n)]
     fn = lambda q: LP.host_batched(lk, q)[0]
     # steps 0 and 1 of seed 4 run DE then snooker under the mix
-    assert [MR.choose_move(4, s, [0.8, 0.2]) for s in (0, 1)] == [0, 1]
+    assert [E.choose_move(4, s, [0.8, 0.2]) for s in (0, 1)] == [0, 1]
     _, kinds = _check_against_restatement(lk, fn, n, p0, MIX, 4, 2)
     assert kinds == [1, 2]
     lk.close()

@@ -7,18 +7,19 @@ import numpy as np
 import pytest
 
 from conftest import ROOT, relerr
-import stretch_ref as R
-from magprop_b200.sampler import DeviceEnsemble, EnsembleSampler, rank_slice
+import ensemble_ref as E
+from magprop_b200.sampler import DeviceEnsemble, EnsembleSampler, StretchMove, rank_slice
 
 
 def test_philox_known_answers():
     # Random123 kat_vectors, philox4x32 10 rounds
-    f = lambda c, k: tuple(int(v) for v in R.philox4x32_10(*[np.uint64(x) for x in c], *k))
+    f = lambda c, k: tuple(int(v) for v in E.philox4x32_10(*[np.uint64(x) for x in c], *k))
     assert f((0, 0, 0, 0), (0, 0)) == (0x6627e8d5, 0xe169c58d, 0xbc57ac4c, 0x9b00dbd8)
     assert f((0xffffffff,) * 4, (0xffffffff,) * 2) == (0x408f276d, 0x41c83b0e, 0xa20bc7c6, 0x6d5451fd)
     assert f((0x243f6a88, 0x85a308d3, 0x13198a2e, 0x03707344), (0xa4093822, 0x299f31d0)) == \
         (0xd16cfe09, 0x94fdcceb, 0x5001e420, 0x24126ea1)
-    u = np.concatenate(R.draws(7, 3, np.arange(20000)))
+    rows = np.arange(20000)
+    u = np.concatenate(E.stretch_draws(7, 3, rows) + (E.accept_uniform(E.STRETCH, 7, 3, rows),))
     assert 0.0 < u.min() and u.max() < 1.0 and abs(u.mean() - 0.5) < 0.01
 
 
@@ -55,7 +56,7 @@ def test_ensemble_order_is_a_keyed_permutation(hostsim):
         got = np.empty(n, dtype=np.int32)
         for step in (0, 1, 12345):
             hostsim.hs_ensemble_order(n, C.c_ulonglong(17), C.c_ulonglong(step), 1, got.ctypes.data_as(C.c_void_p))
-            want = R.ensemble_order(n, 17, step)
+            want = E.ensemble_order(n, 17, step)
             assert (got == want).all()
             assert np.array_equal(np.sort(got), np.arange(n))
         hostsim.hs_ensemble_order(n, C.c_ulonglong(17), C.c_ulonglong(5), 0, got.ctypes.data_as(C.c_void_p))
@@ -65,7 +66,7 @@ def test_ensemble_order_is_a_keyed_permutation(hostsim):
         assert hostsim.hs_ensemble_order_roundtrip(n, C.c_ulonglong(17), C.c_ulonglong(3)) == 0
     # over many steps every walker lands in half 0 about half of the time, and pairs decorrelate
     n = 64
-    in0 = np.array([R.ensemble_order(n, 3, s)[: n // 2] for s in range(400)])
+    in0 = np.array([E.ensemble_order(n, 3, s)[: n // 2] for s in range(400)])
     freq = np.array([(in0 == w).any(axis=1).mean() for w in range(n)])
     assert np.abs(freq - 0.5).max() < 0.1
     both = np.mean([(0 in r) and (1 in r) for r in in0])
@@ -75,7 +76,7 @@ def test_ensemble_order_is_a_keyed_permutation(hostsim):
 def _run_ensemble(dist, nsteps=25, randomize=True):
     rng = np.random.RandomState(5)
     p0 = rng.randn(32, 3)
-    ens = DeviceEnsemble(R.NumpyBackend(gauss_lnprob), 32, 3, a=2.0, seed=11, device="cpu", dist=dist,
+    ens = DeviceEnsemble(E.NumpyBackend(gauss_lnprob), 32, 3, a=2.0, seed=11, device="cpu", dist=dist,
                          randomize_split=randomize)
     ens.set_state(p0, gauss_lnprob(p0))
     chain, lps = ens.run(nsteps, store=True)
@@ -123,7 +124,7 @@ def test_device_ensemble_and_host_sampler_agree_statistically():
     hflat = host.get_chain()[500:].reshape(-1, 3)
     res = {}
     for randomize in (True, False):
-        ens = DeviceEnsemble(R.NumpyBackend(gauss_lnprob), 40, 3, a=2.0, seed=2, device="cpu", randomize_split=randomize)
+        ens = DeviceEnsemble(E.NumpyBackend(gauss_lnprob), 40, 3, a=2.0, seed=2, device="cpu", randomize_split=randomize)
         ens.set_state(p0, gauss_lnprob(p0))
         chain, _ = ens.run(2000, store=True)
         flat = chain.numpy()[500:].reshape(-1, 3)
@@ -162,13 +163,14 @@ def test_device_half_step_matches_numpy_double(built, golden):
     torch.cuda.synchronize()
     order_d = torch.empty(n, dtype=torch.int32, device="cuda")
     for it in range(nsteps):
-        order = R.ensemble_order(n, 99, it)
+        order = E.ensemble_order(n, 99, it)
         A.check(A.load().mp_ensemble_order(n, 99, it, 1, order_d.data_ptr(), None))
         assert (order_d.cpu().numpy() == order).all()
         for split in (0, 1):
             active = order[split * half:(split + 1) * half]
             comp = order[(1 - split) * half:(2 - split) * half]
-            R.half_step(coords, lnp, active, comp, 2.0, 99, 2 * it + split, lk.lnprob, acc)
+            E.half_step(coords, lnp, active, np.zeros(half, np.int64), comp[None, :], StretchMove(2.0), 99, 2 * it + split,
+                        lk.lnprob, accepted=acc)
         assert (chain[it].cpu().numpy() == coords).all()
         assert (lps[it].cpu().numpy() == lnp).all()
     assert (ens.accepted.cpu().numpy() == acc).all()

@@ -1,5 +1,5 @@
-"""Parallel-tempered ensembles and thermodynamic-integration evidence: the NumPy restatement against the stretch
-move and the host-compiled kernel helpers, the sampler on a Gaussian with a known evidence, argument checks of the C
+"""Parallel-tempered ensembles and thermodynamic-integration evidence: the NumPy restatement against the
+host-compiled kernel helpers, the sampler on a Gaussian with a known evidence, argument checks of the C
 ABI (CPU); the fused tempered half-step and swap against the restatement, determinism, and the evidence of a
 synthetic dataset against importance sampling (GPU)."""
 import ctypes as C
@@ -8,9 +8,9 @@ from math import erf
 import numpy as np
 import pytest
 
-import stretch_ref as R
-import tempered_ref as TR
-from magprop_b200.sampler import (DeviceEnsemble, TemperedEnsemble, geometric_betas, thermodynamic_log_evidence)
+import ensemble_ref as E
+from magprop_b200.sampler import (DeviceEnsemble, StretchMove, TemperedEnsemble, geometric_betas,
+                                  thermodynamic_log_evidence)
 
 SIG = np.array([1.0, 2.0, 0.5])
 BOX = 10.0
@@ -23,26 +23,6 @@ def gauss_box_lnprob(q):
     q = np.asarray(q)
     lnl = -0.5 * np.sum((q / SIG) ** 2, axis=1) - np.sum(np.log(SIG * np.sqrt(2 * np.pi)))
     return np.where(np.all(np.abs(q) <= BOX, axis=1), lnl, -np.inf)
-
-
-# ---- the restatement ------------------------------------------------------------------------------------
-def test_restatement_at_one_temperature_is_the_stretch_move():
-    rng = np.random.RandomState(0)
-    n, ndim = 40, 3
-    c1 = rng.randn(n, ndim)
-    l1 = gauss_box_lnprob(c1)
-    c2, l2 = c1.copy(), l1.copy()
-    a1, a2 = np.zeros(n, np.int32), np.zeros(n, np.int32)
-    for step in range(20):
-        order = R.ensemble_order(n, 7, step)
-        for split in (0, 1):
-            act = order[split * (n // 2):(split + 1) * (n // 2)]
-            comp = order[(1 - split) * (n // 2):(2 - split) * (n // 2)]
-            R.half_step(c1, l1, act, comp, 2.0, 7, 2 * step + split, gauss_box_lnprob, a1)
-            TR.half_step(c2, l2, [1.0], n, split, 2.0, 7, step, gauss_box_lnprob, a2)
-        TR.swap(c2, l2, [1.0], n, 7, step)
-    assert np.array_equal(c1, c2) and np.array_equal(l1, l2) and np.array_equal(a1, a2)
-    assert 0 < a1.sum() < 40 * n
 
 
 @pytest.fixture(scope="module")
@@ -72,7 +52,7 @@ def test_host_compiled_mapping_and_swap_decision_match_the_restatement(tempered_
             t, row, part = (np.empty(m, np.int32) for _ in range(3))
             tempered_rng.tr_tempered_rows(n, T, 99, step, split, randomize, pj.ctypes.data, t.ctypes.data, row.ctypes.data,
                                          part.ctypes.data)
-            wt, wrow, wcomp = TR.tempered_rows(n, T, 99, step, split, bool(randomize))
+            wt, wrow, wcomp = E.tempered_rows(n, T, 99, step, split, bool(randomize))
             assert np.array_equal(t, wt) and np.array_equal(row, wrow)
             assert np.array_equal(part, wcomp[wt, pj])
             assert np.array_equal(np.sort(row // n), wt)                      # movers stay in their temperature
@@ -82,13 +62,13 @@ def test_host_compiled_mapping_and_swap_decision_match_the_restatement(tempered_
         bh, bc = sorted(rng.rand(2))
         lh, lc = rng.choice(vals), rng.choice(vals)
         got = tempered_rng.tr_pt_swap_accept(5, 77 + (k << 33), row, bc, bh, lh, lc)
-        want = TR.swap_accept(5, 77 + (k << 33), np.array([row]), bc, bh, np.array([lh]), np.array([lc]))[0]
+        want = E.swap_accept(5, 77 + (k << 33), np.array([row]), bc, bh, np.array([lh]), np.array([lc]))[0]
         assert got == int(want), (row, bc, bh, lh, lc)
 
 
 # ---- the sampler on a Gaussian with a known evidence ----------------------------------------------------
 def _tempered(betas, n, seed, p0, nsteps):
-    ens = TemperedEnsemble(TR.NumpyTemperedBackend(gauss_box_lnprob), n, 3, betas, seed=seed, device="cpu")
+    ens = TemperedEnsemble(E.NumpyBackend(gauss_box_lnprob), n, 3, betas, seed=seed, device="cpu")
     ens.initialise(p0)
     chain, lps = ens.run(nsteps)
     return ens, chain.numpy(), lps.numpy()
@@ -113,7 +93,7 @@ def test_tempered_gaussian_recovers_evidence_and_posterior():
 def test_one_temperature_is_the_device_ensemble():
     p0 = np.random.RandomState(4).randn(16, 3)
     ens, chain, lps = _tempered([1.0], 16, 9, p0, 40)
-    ref = DeviceEnsemble(R.NumpyBackend(gauss_box_lnprob), 16, 3, seed=9, device="cpu")
+    ref = DeviceEnsemble(E.NumpyBackend(gauss_box_lnprob), 16, 3, seed=9, device="cpu")
     ref.set_state(p0, gauss_box_lnprob(p0))
     rc, rl = ref.run(40, store=True)
     assert np.array_equal(chain, rc.numpy()) and np.array_equal(lps[:, 0], rl.numpy())
@@ -122,7 +102,7 @@ def test_one_temperature_is_the_device_ensemble():
 
 
 def test_initialise_broadcasts_and_checks_shapes():
-    ens = TemperedEnsemble(TR.NumpyTemperedBackend(gauss_box_lnprob), 8, 3, [1.0, 0.5, 0.1], device="cpu")
+    ens = TemperedEnsemble(E.NumpyBackend(gauss_box_lnprob), 8, 3, [1.0, 0.5, 0.1], device="cpu")
     p0 = np.random.RandomState(0).randn(8, 3)
     ens.initialise(p0)
     assert np.array_equal(ens.coords.numpy().reshape(3, 8, 3), np.broadcast_to(p0, (3, 8, 3)))
@@ -130,7 +110,7 @@ def test_initialise_broadcasts_and_checks_shapes():
     with pytest.raises(ValueError):
         ens.initialise(np.zeros((2, 8, 3)))
     with pytest.raises(ValueError):
-        TemperedEnsemble(TR.NumpyTemperedBackend(gauss_box_lnprob), 8, 3, [1.0, 0.5], device="cpu", dist=object())
+        TemperedEnsemble(E.NumpyBackend(gauss_box_lnprob), 8, 3, [1.0, 0.5], device="cpu", dist=object())
     with pytest.raises(NotImplementedError):
         ens.run_until_converged(10)
 
@@ -244,10 +224,12 @@ def test_tempered_kernels_match_the_restatement(built, golden):
         for split in (0, 1):
             ens.backend.tempered_half_step(ens, step, split)
             stiff.append(lk.last_stiff_count())
-            TR.half_step(coords, lnp, betas, n, split, 2.0, 21, step, lk.lnprob, acc)
+            t, rows, comp = E.tempered_rows(n, T, 21, step, split)
+            E.half_step(coords, lnp, rows, t, comp, StretchMove(2.0), 21, 2 * step + split, lk.lnprob, betas=betas,
+                        accepted=acc)
             assert np.array_equal(ens.coords.cpu().numpy(), coords) and np.array_equal(ens.lnp.cpu().numpy(), lnp)
         ens.backend.tempered_swap(ens, step)
-        TR.swap(coords, lnp, betas, n, 21, step, swaps)
+        E.swap(coords, lnp, betas, n, 21, step, swaps)
         ens.step += 1
         torch.cuda.synchronize()
         assert np.array_equal(ens.coords.cpu().numpy(), coords) and np.array_equal(ens.lnp.cpu().numpy(), lnp)
@@ -293,6 +275,32 @@ def test_tempered_runs_are_deterministic_across_streams(built, golden):
         torch.cuda.synchronize()
     for a, b in zip(*out):
         assert torch.equal(a, b)
+    lk.close()
+
+
+@pytest.mark.gpu
+def test_run_concurrently_equals_run(built, golden):
+    """run_concurrently advances a tempered ensemble beside a plain one as run advances each: every temperature moves,
+    the swaps run, and the stored lnp holds every temperature."""
+    import torch
+    from magprop_b200.sampler import run_concurrently
+    lk = _humped(golden)
+    T, n = 4, 128
+    betas = geometric_betas(T, 1e-3)
+    p0 = _spread_start(T, n, 2)
+    out = []
+    for together in (False, True):
+        te = TemperedEnsemble.from_likelihood(lk, n, 6, betas, seed=12)
+        te.initialise(p0)
+        de = DeviceEnsemble.from_likelihood(lk, 64, 6, seed=13)
+        de.initialise(p0[0, :64])
+        res = run_concurrently([te, de], 5, store=True) if together else [te.run(5), de.run(5, store=True)]
+        torch.cuda.synchronize()
+        assert te.step == de.step == 5
+        out.append([*res[0], *res[1], te.accepted.clone(), te.swap_accepted.clone(), de.accepted.clone()])
+    for a, b in zip(*out):
+        assert a.shape == b.shape and torch.equal(a, b)
+    assert out[0][1].shape == (5, T, n) and out[0][5].sum() > 0
     lk.close()
 
 
