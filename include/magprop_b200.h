@@ -298,6 +298,8 @@ int mp_ensemble_moves_half_step(mp_handle* h, const mp_ensemble* e, const mp_mov
                                 uint64_t step, int32_t split, void* stream);
 int mp_tempered_moves_half_step(mp_handle* h, const mp_ensemble* e, int32_t ntemps, const double* betas,
                                 const mp_move* moves, int32_t n_moves, uint64_t step, int32_t split, void* stream);
+/* Sequential Monte Carlo (a half-step at one inverse temperature, the weights and their ESS, systematic resampling)
+ * is declared in magprop_smc.h, which includes this header.                                                          */
 
 /* Peer-mappable device memory for the replicas (CUDA IPC; one process per GPU on one node).
  * mp_peer_alloc: cudaMalloc + export a 64-byte handle other processes pass to mp_peer_open, which maps the

@@ -166,6 +166,10 @@ def declare(lib):
     lib.mp_kernels_launched.restype = C.c_int64
     lib.mp_fp64_peak_tflops.argtypes = [C.c_int32, _dp]
     lib.mp_last_stiff_count.argtypes = [vp, _ip]
+    lib.mp_smc_weights.argtypes = [vp, C.c_int64, C.c_double, vp, vp, C.c_int32, vp]
+    lib.mp_smc_resample.argtypes = [vp, C.c_int64, C.c_int32, C.c_uint64, C.c_uint64, vp, vp, vp, vp, vp, C.c_int32, vp]
+    lib.mp_annealed_moves_half_step.argtypes = [vp, C.POINTER(Ensemble), C.c_double, vp, C.c_int32, C.c_uint64, C.c_int32,
+                                                vp]
     return lib
 
 
@@ -177,6 +181,9 @@ EXPORTS = ["mp_abi_version", "mp_device_count", "mp_last_error", "mp_create", "m
            "mp_tempered_half_step", "mp_tempered_swap", "mp_ensemble_moves_half_step", "mp_tempered_moves_half_step",
            "mp_chain_moments", "mp_chain_order_statistics", "mp_chain_autocorr", "mp_gompertz_curves", "mp_kernels_launched",
            "mp_peer_alloc", "mp_peer_open", "mp_peer_close", "mp_peer_free", "mp_peer_barrier"]
+# The entry points include/magprop_smc.h declares (sequential Monte Carlo), exported by the same library.
+SMC_EXPORTS = ["mp_smc_weights", "mp_smc_resample", "mp_annealed_moves_half_step"]
+MP_SMC_TILE = 64
 
 
 def load():

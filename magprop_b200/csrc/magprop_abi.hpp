@@ -1,6 +1,6 @@
 // magprop_abi.hpp -- what the host code of every translation unit of the library shares (host only, internal):
 // the thread's last error message behind mp_last_error, the CUDA-call check, device selection, and DevBuf, the
-// device buffer that frees itself.  It includes only the public header: the per-walker core and its disc tables
+// device buffer that frees itself.  It includes only the public headers: the per-walker core and its disc tables
 // are compiled into magprop_kernels.cu alone.
 #pragma once
 #include <cuda_runtime.h>
@@ -10,6 +10,7 @@
 #include <vector>
 
 #include "../../include/magprop_b200.h"
+#include "../../include/magprop_smc.h"
 
 namespace mp {
 

@@ -1589,6 +1589,24 @@ extern "C" int mp_tempered_moves_half_step(mp_handle* h, const mp_ensemble* e, i
   return tempered_half_step(h, e, ntemps, betas, pick_move(moves, n_moves, e->seed, step), step, split, stream);
 }
 
+// ---- sequential Monte Carlo: one ensemble at one inverse temperature --------------------------------------------
+// The tempered half-step with the ladder {beta}; unlike a tempered ensemble's, that one beta need not be 1.
+extern "C" int mp_annealed_moves_half_step(mp_handle* h, const mp_ensemble* e, double beta, const mp_move* moves,
+                                           int32_t n_moves, uint64_t step, int32_t split, void* stream) {
+  const char* who = "mp_annealed_moves_half_step";
+  int rc = check_ensemble(e, who);
+  if (rc) return rc;
+  const std::string w(who);
+  if (e->world != 1 || e->n_peers != 0 || e->pack_out)
+    return fail(MP_ERR_BAD_ARG, w + ": an annealed ensemble runs on one rank (world 1, no peers, no pack_out)");
+  if (e->ndim < 1 || e->ndim > MP_MAX_NDIM) return fail(MP_ERR_BAD_ARG, w + ": bad ndim");
+  if (!(beta > 0.0 && beta <= 1.0)) return fail(MP_ERR_BAD_ARG, w + ": beta must lie in (0, 1]");   // (NaN fails too)
+  if (split != 0 && split != 1) return fail(MP_ERR_BAD_ARG, w + ": split must be 0 or 1");
+  if ((rc = check_moves(moves, n_moves, e->nwalkers / 2, who))) return rc;
+  if (!h) return fail(MP_ERR_BAD_ARG, w + ": null handle");
+  return tempered_half_step(h, e, 1, &beta, pick_move(moves, n_moves, e->seed, step), step, split, stream);
+}
+
 extern "C" int mp_tempered_swap(const mp_ensemble* e, int32_t ntemps, const double* betas, uint64_t step,
                                 int32_t* d_swap_accepted, void* stream) {
   int rc = check_tempered(e, ntemps, betas, "mp_tempered_swap");

@@ -189,4 +189,12 @@ MP_RNG_HD int choose_move(uint64_t seed, uint64_t step, const double* weights, i
   return last;
 }
 
+// ---- sequential Monte Carlo (mp_smc_resample) ---------------------------------------------------------------
+// The one uniform of SMC stage `stage`'s systematic resampling: u01 of words 0,1 of Philox counter (stage, 0, 7).
+// Word 7 is used by no other draw (stretch 0/1, permutation key 2, swap 3, DE/snooker 4/5, move choice 6).
+MP_RNG_HD double smc_stage_uniform(uint64_t seed, uint64_t stage) {
+  const Philox r = philox4x32_10((uint32_t)stage, (uint32_t)(stage >> 32), 0u, 7u, (uint32_t)seed, (uint32_t)(seed >> 32));
+  return u01(r.c[0], r.c[1]);
+}
+
 }  // namespace mp

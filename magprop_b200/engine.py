@@ -188,6 +188,25 @@ def chain_moments(d_chain: int, n: int, ndim: int, device=0, stream=0):
     return mean, cov
 
 
+def smc_weights(d_lnp: int, n: int, dbeta: float, d_w: int = 0, device=0, stream=0):
+    """(m, S1, S2) of the incremental weights w_i = exp(dbeta (lnp_i - m)) of a device array lnp [n] (raw pointer),
+    m its largest finite entry; ``d_w`` (raw pointer, or 0) receives the weights.  Synchronises ``stream``."""
+    lib = A.load()
+    out = np.empty(3)
+    A.check(lib.mp_smc_weights(d_lnp, n, float(dbeta), d_w or None, A.ptr(out), device, stream or None))
+    return float(out[0]), float(out[1]), float(out[2])
+
+
+def smc_resample(d_w: int, n: int, ndim: int, seed: int, stage: int, d_coords_in: int, d_lnp_in: int, d_coords_out: int,
+                 d_lnp_out: int, d_ancestors: int = 0, device=0, stream=0):
+    """Systematic resampling of n particles (raw device pointers) by the weights d_w into the out buffers, with the
+    stage's uniform from (seed, stage); ``d_ancestors`` (int64 [n], or 0) receives the ancestor indices.  Enqueued on
+    ``stream``, not synchronised."""
+    lib = A.load()
+    A.check(lib.mp_smc_resample(d_w, n, ndim, int(seed), int(stage), d_coords_in, d_lnp_in, d_coords_out, d_lnp_out,
+                                d_ancestors or None, device, stream or None))
+
+
 def chain_order_statistics(d_chain: int, n: int, ndim: int, col: int, ranks, device=0, stream=0) -> np.ndarray:
     """Exact order statistics (0-based ranks) of one column of a device-resident chain [n, ndim]."""
     lib = A.load()

@@ -25,6 +25,9 @@ so this module carries the minimum needed to run and measure the path:
                         per half-step (``mp_tempered_half_step``), then one swap
                         pass per step (``mp_tempered_swap``).
 ``thermodynamic_log_evidence``  ln Z by thermodynamic integration over the ladder.
+``SMCSampler``          sequential Monte Carlo with adaptive tempering: N particles annealed from the prior to the
+                        posterior in stages (weights, ESS bisection, systematic resampling, MCMC moves at the stage's
+                        beta), with ln Z from the stages' mean weights (include/magprop_smc.h).
 ``StretchMove``, ``DEMove``, ``DESnookerMove``  emcee 3's ``moves=``: both ensembles take a move, a list of
                         moves or a list of ``(move, weight)`` and run one of them per step
                         (``mp_ensemble_moves_half_step`` / ``mp_tempered_moves_half_step``).
@@ -41,6 +44,7 @@ rank evaluates on the fly (include/magprop_b200.h, ``mp_ensemble``).
 from __future__ import annotations
 
 import ctypes as C
+import math
 
 import numpy as np
 
@@ -300,6 +304,20 @@ class CudaBackend:
     def tempered_swap(self, ens, step):
         self.A.check(self.lib.mp_tempered_swap(C.byref(ens.desc), ens.ntemps, self.A.ptr(ens.betas), step,
                                                ens.swap_accepted.data_ptr(), self.stream() or None))
+
+    def annealed_half_step(self, ens, step, split):
+        self.A.check(self.lib.mp_annealed_moves_half_step(self.lik._h, C.byref(ens.desc), ens.beta, C.addressof(ens._moves_c),
+                                                          len(ens._moves_c), step, split, self.stream() or None))
+
+    def smc_weights(self, ens, dbeta, write):
+        from .engine import smc_weights
+        return smc_weights(ens.lnp.data_ptr(), ens.nwalkers, dbeta, ens.weights.data_ptr() if write else 0,
+                           self.lik.device, self.stream())
+
+    def smc_resample(self, ens, stage):
+        from .engine import smc_resample
+        smc_resample(ens.weights.data_ptr(), ens.nwalkers, ens.ndim, ens.seed, stage, ens.coords.data_ptr(), ens.lnp.data_ptr(),
+                     ens.resampled_coords.data_ptr(), ens.resampled_lnp.data_ptr(), 0, self.lik.device, self.stream())
 
 
 class DeviceEnsemble:
@@ -706,6 +724,152 @@ class TemperedEnsemble(DeviceEnsemble):
     def swap_acceptance_fraction(self):
         """Accepted swaps per step and column of each adjacent pair (t-1, t), [ntemps - 1]."""
         return self.swap_accepted.double() / (max(1, self.step) * self.nwalkers)
+
+
+class SMCResult:
+    """What ``SMCSampler.run`` returns: the final population ``coords`` [N, ndim] and ``lnp`` [N] (tensors on the
+    sampler's device), ``log_evidence``, and per stage ``betas`` (the beta the stage reached), ``ess`` (S1^2 / S2 of its
+    weights), ``steps`` (its MCMC steps) and ``acceptance`` (their mean acceptance); then the ``final_steps`` run at
+    beta = 1 after the last stage, their ``final_acceptance``, and ``n_evaluations`` (lnprob calls in all)."""
+
+    def __init__(self, coords, lnp, log_evidence, betas, ess, steps, acceptance, final_steps, final_acceptance,
+                 n_evaluations):
+        self.coords, self.lnp, self.log_evidence = coords, lnp, float(log_evidence)
+        self.betas, self.ess = np.asarray(betas, dtype=np.float64), np.asarray(ess, dtype=np.float64)
+        self.steps, self.acceptance = np.asarray(steps, dtype=np.int64), np.asarray(acceptance, dtype=np.float64)
+        self.final_steps, self.final_acceptance = int(final_steps), float(final_acceptance)
+        self.n_evaluations = int(n_evaluations)
+
+    @property
+    def n_stages(self):
+        return int(self.betas.size)
+
+
+class SMCSampler(DeviceEnsemble):
+    """Sequential Monte Carlo with adaptive tempering on one device: ``nparticles`` particles drawn from the prior are
+    annealed through p_beta ~ L^beta prior from beta = 0 to 1.  Each stage
+      1. bisects (50 halvings) for the largest dbeta in (0, 1 - beta] whose incremental weights w_i = L_i^dbeta keep
+         S1^2 / S2 >= target_ess * N, one weights call per probe (1 - beta itself is tried first and, if it passes,
+         beta becomes exactly 1);
+      2. adds dbeta m + ln(S1 / N) to ln Z (m the largest lnp; S1 of the call that keeps the weights);
+      3. resamples the population systematically by those weights;
+      4. runs K MCMC steps of the ensemble moves at the new beta, both halves moved against each other as in
+         ``DeviceEnsemble``, with the ensemble's global step counter (no Philox counter is used twice).
+         K = clip(ceil(ln(1 - p_move) / ln(1 - acc)), min_steps, max_steps), acc the mean acceptance of the previous
+         stage's steps (the first stage runs min_steps).  Right after resampling, duplicated particles can propose
+         exactly their own position (DE with two copies of one particle as partners, snooker with a copy of the mover as
+         z); such a proposal is accepted and counts as accepted, which raises acc a little.
+    After the stage that reaches beta = 1, max(K, min_steps) more steps run at beta = 1.  The returned population is
+    equally weighted.  ``moves`` as for ``DeviceEnsemble``; None is ``[(DEMove(), 0.8), (DESnookerMove(), 0.2)]``,
+    moves that use the whole population's spread as their scale.  ``lnp`` is untempered; ln Z is that of the
+    likelihood against the prior the particles were drawn from, with lnprior = 0 inside its support.
+    One device only: ``dist`` raises ``ValueError``.  ``backend`` as for ``DeviceEnsemble``, with
+    ``annealed_half_step``, ``smc_weights`` and ``smc_resample``."""
+
+    BISECTIONS = 50
+
+    def __init__(self, backend, nparticles, ndim, seed=0, moves=None, target_ess=0.5, p_move=0.99, min_steps=2,
+                 max_steps=50, device="cuda", dist=None):
+        import torch
+        if dist is not None:
+            raise ValueError("an SMC sampler runs on one device: dist is not supported")
+        self.target_ess, self.p_move = float(target_ess), float(p_move)
+        if not 0.0 < self.target_ess < 1.0:
+            raise ValueError("target_ess must lie in (0, 1)")
+        if not 0.0 < self.p_move < 1.0:
+            raise ValueError("p_move must lie in (0, 1)")
+        if int(min_steps) != min_steps or int(max_steps) != max_steps or not 1 <= min_steps <= max_steps:
+            raise ValueError("min_steps and max_steps must be integers with 1 <= min_steps <= max_steps")
+        self.min_steps, self.max_steps = int(min_steps), int(max_steps)
+        super().__init__(backend, nparticles, ndim, seed=seed, device=device,
+                         moves=[(DEMove(), 0.8), (DESnookerMove(), 0.2)] if moves is None else moves)
+        self.beta = 0.0
+        self.weights = torch.empty(nparticles, dtype=torch.float64, device=self.device)
+        self.resampled_coords = torch.empty_like(self.coords)
+        self.resampled_lnp = torch.empty_like(self.lnp)
+
+    @classmethod
+    def from_likelihood(cls, lik, nparticles, ndim, **kw):
+        import torch
+        smc = cls(CudaBackend(lik), nparticles, ndim, device=torch.device("cuda", lik.device), **kw)
+        smc._lik = lik
+        return smc
+
+    def run_until_converged(self, *args, **kwargs):
+        raise NotImplementedError("an SMC run stops when beta reaches 1; run() returns its final population")
+
+    def _steps_for(self, acc):
+        """K = clip(ceil(ln(1 - p_move) / ln(1 - acc)), min_steps, max_steps): the steps after which a particle has
+        moved at least once with probability p_move, were every step accepted with probability acc."""
+        if acc <= 0.0:
+            return self.max_steps
+        if acc >= 1.0:
+            return self.min_steps
+        return int(min(max(math.ceil(math.log(1.0 - self.p_move) / math.log(1.0 - acc)), self.min_steps), self.max_steps))
+
+    def _next_dbeta(self):
+        """(dbeta, reaches_one): the largest dbeta in (0, 1 - beta] with S1^2 / S2 >= target_ess * N, by bisection."""
+        need = self.target_ess * self.nwalkers
+
+        def passes(db):
+            m, s1, s2 = self.backend.smc_weights(self, db, False)
+            if m == -math.inf:
+                raise RuntimeError("SMCSampler: no particle has a finite lnp")
+            return s1 * s1 / s2 >= need
+
+        hi = 1.0 - self.beta
+        if passes(hi):
+            return hi, True
+        lo = 0.0
+        for _ in range(self.BISECTIONS):
+            mid = 0.5 * (lo + hi)
+            if passes(mid):
+                lo = mid
+            else:
+                hi = mid
+        if lo == 0.0:
+            raise RuntimeError(f"SMCSampler: no dbeta above {hi:.3g} keeps the ESS at beta = {self.beta:.6g}")
+        return lo, False
+
+    def _mutate(self, nsteps):
+        """nsteps MCMC steps at the current beta; their mean acceptance (one read of the counters)."""
+        self.accepted.zero_()
+        for _ in range(nsteps):
+            self.backend.annealed_half_step(self, self.step, 0)
+            self.backend.annealed_half_step(self, self.step, 1)
+            self.step += 1
+        return int(self.accepted.sum()) / (self.nwalkers * nsteps)
+
+    def run(self, p0, max_stages=1000):
+        """Anneal the prior draws p0 [N, ndim] to the posterior; returns an ``SMCResult``.  Raises ``RuntimeError`` if
+        no particle has a finite lnp, or if beta has not reached 1 after ``max_stages`` stages."""
+        n = self.nwalkers
+        self.beta = 0.0
+        self.initialise(p0)
+        log_z, n_eval, k = 0.0, n, self.min_steps
+        betas, ess, steps, acceptance = [], [], [], []
+        while self.beta < 1.0:
+            stage = len(betas)
+            if stage >= max_stages:
+                raise RuntimeError(f"SMCSampler: beta reached only {self.beta:.6g} after {max_stages} stages")
+            dbeta, to_one = self._next_dbeta()
+            m, s1, s2 = self.backend.smc_weights(self, dbeta, True)
+            log_z += dbeta * m + math.log(s1 / n)
+            self.backend.smc_resample(self, stage)
+            self.coords.copy_(self.resampled_coords)
+            self.lnp.copy_(self.resampled_lnp)
+            self.beta = 1.0 if to_one else min(1.0, self.beta + dbeta)
+            acc = self._mutate(k)
+            betas.append(self.beta)
+            ess.append(s1 * s1 / s2)
+            steps.append(k)
+            acceptance.append(acc)
+            n_eval += n * k
+            k = self._steps_for(acc)
+        final = max(k, self.min_steps)
+        final_acc = self._mutate(final)
+        n_eval += n * final
+        return SMCResult(self.coords, self.lnp, log_z, betas, ess, steps, acceptance, final, final_acc, n_eval)
 
 
 def run_concurrently(ensembles, nsteps, store=False):

@@ -124,6 +124,38 @@ def run_tempered(grb, x, y, yerr, n_walk, ntemps, n_step, beta_min, seed=0, disc
     return res
 
 
+def run_smc(grb, x, y, yerr, n_particles, seed=0, moves=None, device=0, max_stages=1000, **smc_kw):
+    """Sequential Monte Carlo (``SMCSampler``): ``n_particles`` drawn uniformly in the script prior box
+    (``mcmc_eqns.lower`` / ``upper``) with ``np.random.RandomState(seed)``, annealed to the posterior.  Returns the
+    ``RunResult`` of the final, equally weighted population as a one-step chain [1, n_particles, 6] (``write_outputs``
+    and ``posterior_summary_device`` take it as they take ``run``'s; its acceptance fraction is that of the steps at
+    beta = 1 after the last stage), with ``log_evidence``, the stage history ``betas``, ``ess``, ``steps``,
+    ``stage_acceptance``, ``n_evaluations`` and the device-resident population (``chain_device`` [1, N, 6],
+    ``lnp_device`` [1, N]) attached.  ``moves`` and ``smc_kw`` (target_ess, p_move, min_steps, max_steps) as for
+    ``SMCSampler``."""
+    from .. import _capi as A
+    from ..engine import Likelihood, time_grid
+    from ..sampler import SMCSampler
+    from .mcmc_eqns import lower, upper
+
+    rng = np.random.RandomState(seed)
+    p0 = lower + (upper - lower) * rng.rand(int(n_particles), lower.size)
+    lk = Likelihood(A.script_model_spec(), time_grid(None), x, y, yerr, lower, upper, device=device)
+    try:
+        smc = SMCSampler.from_likelihood(lk, int(n_particles), lower.size, seed=seed, moves=moves, **smc_kw)
+        out = smc.run(p0, max_stages=max_stages)
+        chain, lnp = out.coords.clone()[None], out.lnp.clone()[None]
+        acc = (smc.accepted.double() / out.final_steps).cpu().numpy()
+        res = RunResult(chain.cpu().numpy(), lnp.cpu().numpy(), acc, seed)
+        res.log_evidence = out.log_evidence
+        res.betas, res.ess, res.steps, res.stage_acceptance = out.betas, out.ess, out.steps, out.acceptance
+        res.final_steps, res.n_evaluations = out.final_steps, out.n_evaluations
+        res.chain_device, res.lnp_device = chain, lnp
+    finally:
+        lk.close()
+    return res
+
+
 # ---- integrated autocorrelation time (emcee.autocorr, restated; emcee is not installed) -----------
 def _next_pow_two(n):
     i = 1
