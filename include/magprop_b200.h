@@ -282,13 +282,30 @@ int mp_tempered_swap(const mp_ensemble* e, int32_t ntemps, const double* betas, 
  *     counters and pack_out as described for mp_ensemble.
  *   Which move runs: one per MCMC step, for both half-steps and every temperature.  u = u01 of Philox counter
  *     (step, 0, 6); the move is the first k with u*W < cum_k, W and cum_k the sequential sums of the weights.
+ *   MP_MOVE_KDE (gamma0; emcee's KDEMove): a Gaussian kernel-density estimate of the complement, sampled.  Centres:
+ *     the complement positions cpos0 + [0, M) in the ensemble order, M = min(Nc, MP_KDE_MAX_CENTRES) -- with a
+ *     randomised split a fresh uniform subset every half-step, fixed during it and independent of any mover (emcee
+ *     uses every complement walker; the cap bounds the density sums).  mu and Sigma: their mean and covariance
+ *     (ddof = 1), every sum in tiles of 64 centres, each tile left to right, then the tile sums left to right;
+ *     mu = S / M, Sigma = S2 / (M-1).  Sigma = L L^T by Cholesky in one thread in row order; a pivot <= 0 or not
+ *     finite makes every mover of that temperature propose q = x with ln f = -inf (rejected).  Bandwidth h = gamma0,
+ *     or Scott's M^(-1/(ndim+4)) (host pow) when gamma0 = 0.  Draws: u_c = u01 of words 0,1 of (hs, me, 8), ua of
+ *     its words 2,3; z from Box-Muller pairs of blocks (hs, me, 9 .. 8 + ceil(ndim/2)) with the library's own
+ *     ln / sincos (gauss_pair, magprop_rng.cuh), reproducible on the host.  Centre j = idx(u_c, M),
+ *     q = c_j + h L z (row r: c_r + h * sum_{k<=r} L_rk z_k, ascending k).  y(p) = L^-1 (p - mu) / h by forward
+ *     substitution in ascending rows, r2_j(p) = sum_c (y_c(p) - y_c(c_j))^2 (ascending c),
+ *     lk(p) = -0.5 min_j r2_j + log(sum_j exp(-0.5 (r2_j - min_j r2_j))) (ascending j), ln f = lk(x) - lk(q).
+ *     One rank only: world 1, no peers, no pack_out.
  * Checked on the host before any device work (MP_ERR_BAD_ARG): moves non-null, 1 <= n_moves <= MP_MAX_MOVES, known
  * kinds, weights finite and >= 0 with a positive sum, stretch a > 1, DE 0 <= sigma < 1 and gamma0 >= 0, snooker
- * gammas > 0, and a half (per temperature) of at least 2 walkers for DE and 3 for snooker when they have weight.   */
+ * gammas > 0, KDE gamma0 finite and >= 0, a half (per temperature) of at least 2 walkers for DE, 3 for snooker and
+ * ndim + 1 for KDE when they have weight, and a weighted KDE move on one rank.  Kind 3 is not assigned.            */
 #define MP_MOVE_STRETCH 0
 #define MP_MOVE_DE 1
 #define MP_MOVE_DE_SNOOKER 2
+#define MP_MOVE_KDE 4
 #define MP_MAX_MOVES 8
+#define MP_KDE_MAX_CENTRES 4096
 typedef struct mp_move {
   int32_t kind;
   int32_t pad;

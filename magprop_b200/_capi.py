@@ -16,7 +16,9 @@ MP_ABI_VERSION = 2
 MP_MAX_PEERS = 15
 MP_MAX_TEMPS = 256
 MP_MOVE_STRETCH, MP_MOVE_DE, MP_MOVE_DE_SNOOKER = range(3)
+MP_MOVE_KDE = 4                 # (kind 3 is not assigned)
 MP_MAX_MOVES = 8
+MP_KDE_MAX_CENTRES = 4096
 
 MP_OK, MP_ERR_BAD_ARG, MP_ERR_DATA_RANGE, MP_ERR_CUDA, MP_ERR_BAD_GRID, MP_ERR_NO_DATA = range(6)
 

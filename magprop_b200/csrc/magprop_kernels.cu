@@ -29,6 +29,7 @@
 #include "magprop_host.hpp"
 #include "magprop_rng.cuh"
 #include "magprop_abi.hpp"
+#include "magprop_kde.hpp"
 
 namespace mp {
 
@@ -377,6 +378,10 @@ __device__ __noinline__ void propose_de(const Move& m, int i, int ndim, double* 
 // The proposal of mover i: q in th and m.prop[i], ln f in m.lnf[i].  The stretch move draws u_z and u_partner from
 // Philox counter (half-step, row, 0):  z = ((a-1) u_z + 1)^2 / a,  q = c - (c - s) z,  ln f = (ndim-1) ln z.
 __device__ __forceinline__ void propose(const Move& m, int i, int ndim, double* th) {
+  if (m.kind == MP_MOVE_KDE) {    // formed by kde_propose (magprop_kde.cu) ahead of this launch
+    for (int c = 0; c < ndim; ++c) th[c] = m.prop[(size_t)i * ndim + c];
+    return;
+  }
   if (m.kind != MP_MOVE_STRETCH) {
     propose_de(m, i, ndim, th);
     return;
@@ -918,6 +923,7 @@ struct mp_handle {
     cudaStream_t stream = nullptr;   // the handle's own lanes only (a caller's stream is never kept here, nor destroyed)
     DevBuf<unsigned long long> recs;   // kRecWords rows, each as long as the lane's capacity in walkers
     DevBuf<double> ybuf, prop, lnf;  // lnf: ln of each proposal's Hastings factor (the DE moves), indexed as prop
+    DevBuf<double> kde_stats, kde_white;   // the KDE move's per-temperature factors and whitened centres (KdeMove)
     DevBuf<int> status, n_rhs, work, counters, key, hist, slot_wid;
     DevBuf<StiffRec> squeue;
     DevBuf<double> betas;        // the ladder of the tempered half-steps on this lane, and its host copy
@@ -1074,9 +1080,10 @@ static int ensure_work(mp_handle::Lane& L, int S, int Nn, int ndim_prop, Work& k
 //   MOVE = false: parameters from d_theta [W][ndim]; results to `sink` (lnprob), `out` (model at data
 //                 [W][D], or curves [W][3][Nn]) and `state` (curves, optional)
 //   MOVE = true : the W movers of an ensemble-move half-step described by `mv`
+//   kde         : with MOVE and the KDE move, its launches (prepared here, then run ahead of each slab)
 template <int MODE, bool MOVE>
 static int launch_eval(mp_handle* h, const Problem& p, const double* d_theta, int W, Sink sink, double* out, double* state,
-                       const Move* mv, cudaStream_t stream, int lane = -1) {
+                       const Move* mv, cudaStream_t stream, int lane = -1, const KdeMove* kde = nullptr) {
   if (W == 0) return MP_OK;
   mp_handle::Lane* Lp = nullptr;
   lane_for(h, stream, lane, &Lp);
@@ -1094,6 +1101,16 @@ static int launch_eval(mp_handle* h, const Problem& p, const double* d_theta, in
   // earlier launch of more walkers on fewer nodes may have made larger)
   k.ws = coop ? (size_t)Nn : 1;
   k.ns = coop ? 1 : (size_t)S;
+  KdeMove km;
+  if (MOVE && kde) {
+    km = *kde;
+    MP_CUDA(Lp->kde_stats.ensure((size_t)km.T * kKdeStats));
+    MP_CUDA(Lp->kde_white.ensure((size_t)km.T * km.M * km.ndim));
+    km.stats = Lp->kde_stats.get();
+    km.white = Lp->kde_white.get();
+    if ((rc = kde_prepare(km, stream))) return rc;
+    h->kernels_launched += 1;
+  }
   for (int i0 = 0; i0 < W; i0 += S) {
     const int n = std::min(S, W - i0);
     k.W = n;
@@ -1124,6 +1141,10 @@ static int launch_eval(mp_handle* h, const Problem& p, const double* d_theta, in
       const volatile int* e = Lp->hint_host;
       const int e0 = e[0], e1 = e[1], e2 = e[2], e3 = e[3];
       if (e0 > 0 && e0 + e1 - 257 <= kTightMdBins && e2 + e3 - 33 <= kTightEpsBins) ordered = false;
+    }
+    if (MOVE && kde) {
+      if ((rc = kde_propose(km, ms.mover0, n, ms.prop, ms.lnf, stream))) return rc;
+      h->kernels_launched += 1;
     }
     const double* th0 = MOVE ? nullptr : d_theta + (size_t)i0 * ndim;
     k.key = Lp->key.get();
@@ -1417,8 +1438,9 @@ static mp_move stretch_move(double a) {
   return mv;
 }
 
-// The host-side checks of a list of moves for halves (per temperature) of `half` walkers (see mp_move).
-static int check_moves(const mp_move* moves, int32_t n_moves, int half, const char* who) {
+// The host-side checks of a list of moves for the (checked) ensemble e, halves per temperature of nwalkers/2 (see mp_move).
+static int check_moves(const mp_move* moves, int32_t n_moves, const mp_ensemble* e, const char* who) {
+  const int half = e->nwalkers / 2;
   const std::string w(who);
   if (!moves || n_moves < 1 || n_moves > MP_MAX_MOVES)
     return fail(MP_ERR_BAD_ARG, w + ": moves must be non-null and n_moves in [1, MP_MAX_MOVES]");
@@ -1437,6 +1459,12 @@ static int check_moves(const mp_move* moves, int32_t n_moves, int half, const ch
     } else if (mv.kind == MP_MOVE_DE_SNOOKER) {
       if (!(mv.gammas > 0.0 && std::isfinite(mv.gammas))) return fail(MP_ERR_BAD_ARG, w + ": snooker move needs gammas > 0");
       need = 3;
+    } else if (mv.kind == MP_MOVE_KDE) {
+      if (!(mv.gamma0 >= 0.0 && std::isfinite(mv.gamma0)))
+        return fail(MP_ERR_BAD_ARG, w + ": KDE move needs a bandwidth factor gamma0 >= 0 (0: Scott's rule)");
+      if (mv.weight > 0.0 && (e->world != 1 || e->n_peers != 0 || e->pack_out))
+        return fail(MP_ERR_BAD_ARG, w + ": the KDE move runs on one rank (world 1, no peers, no pack_out)");
+      need = e->ndim + 1;
     } else {
       return fail(MP_ERR_BAD_ARG, w + ": unknown move kind");
     }
@@ -1483,6 +1511,24 @@ static void fill_ensemble_move(const mp_ensemble* e, uint64_t step, int split, c
   }
 }
 
+// The KDE launches of half `split` at MCMC step `step` over ntemps temperatures of the ensemble e (see KdeMove).
+static KdeMove kde_move(const mp_ensemble* e, int ntemps, const mp_move& mv, const Move& m) {
+  KdeMove k;
+  std::memset(&k, 0, sizeof(k));
+  k.coords = e->coords;
+  k.perm = m.perm;
+  k.pos0 = m.pos0;
+  k.cpos0 = m.cpos0;
+  k.T = ntemps;
+  k.n = e->nwalkers;
+  k.ndim = e->ndim;
+  k.M = std::min(m.n_complement, MP_KDE_MAX_CENTRES);
+  k.h = mv.gamma0 > 0.0 ? mv.gamma0 : std::pow((double)k.M, -1.0 / (e->ndim + 4));
+  k.seed = m.seed;
+  k.hs = m.step;
+  return k;
+}
+
 // One half-step of a (checked) ensemble with move `mv`: mp_ensemble_half_step and mp_ensemble_moves_half_step.
 static int ensemble_half_step(mp_handle* h, const mp_ensemble* e, const mp_move& mv, uint64_t step, int32_t split,
                               void* stream, const char* who) {
@@ -1494,8 +1540,9 @@ static int ensemble_half_step(mp_handle* h, const mp_ensemble* e, const mp_move&
   Move m;
   fill_ensemble_move(e, step, split, mv, m);
   if ((rc = fill_pull(e, step, m, who))) return rc;
+  const KdeMove km = kde_move(e, 1, mv, m);
   return launch_eval<kModeLnprob, true>(h, p, nullptr, n_mine, Sink{nullptr, nullptr, nullptr}, nullptr, nullptr, &m,
-                                        (cudaStream_t)stream);
+                                        (cudaStream_t)stream, -1, mv.kind == MP_MOVE_KDE ? &km : nullptr);
 }
 
 extern "C" int mp_ensemble_half_step(mp_handle* h, const mp_ensemble* e, uint64_t step, int32_t split, void* stream) {
@@ -1512,7 +1559,7 @@ extern "C" int mp_ensemble_moves_half_step(mp_handle* h, const mp_ensemble* e, c
   int rc = check_ensemble(e, who);
   if (rc) return rc;
   if (split != 0 && split != 1) return fail(MP_ERR_BAD_ARG, std::string(who) + ": split must be 0 or 1");
-  if ((rc = check_moves(moves, n_moves, e->nwalkers / 2, who))) return rc;
+  if ((rc = check_moves(moves, n_moves, e, who))) return rc;
   if (!h) return fail(MP_ERR_BAD_ARG, std::string(who) + ": null handle");
   return ensemble_half_step(h, e, pick_move(moves, n_moves, e->seed, step), step, split, stream, who);
 }
@@ -1566,7 +1613,9 @@ static int tempered_half_step(mp_handle* h, const mp_ensemble* e, int32_t ntemps
   m.rank = 0;
   m.half = m.n_mine = half;
   m.betas = L->betas.get();
-  return launch_eval<kModeLnprob, true>(h, p, nullptr, n_movers, Sink{nullptr, nullptr, nullptr}, nullptr, nullptr, &m, s);
+  const KdeMove km = kde_move(e, ntemps, mv, m);
+  return launch_eval<kModeLnprob, true>(h, p, nullptr, n_movers, Sink{nullptr, nullptr, nullptr}, nullptr, nullptr, &m, s, -1,
+                                        mv.kind == MP_MOVE_KDE ? &km : nullptr);
 }
 
 extern "C" int mp_tempered_half_step(mp_handle* h, const mp_ensemble* e, int32_t ntemps, const double* betas, uint64_t step,
@@ -1584,7 +1633,7 @@ extern "C" int mp_tempered_moves_half_step(mp_handle* h, const mp_ensemble* e, i
   int rc = check_tempered(e, ntemps, betas, who);
   if (rc) return rc;
   if (split != 0 && split != 1) return fail(MP_ERR_BAD_ARG, std::string(who) + ": split must be 0 or 1");
-  if ((rc = check_moves(moves, n_moves, e->nwalkers / 2, who))) return rc;
+  if ((rc = check_moves(moves, n_moves, e, who))) return rc;
   if (!h) return fail(MP_ERR_BAD_ARG, std::string(who) + ": null handle");
   return tempered_half_step(h, e, ntemps, betas, pick_move(moves, n_moves, e->seed, step), step, split, stream);
 }
@@ -1602,7 +1651,7 @@ extern "C" int mp_annealed_moves_half_step(mp_handle* h, const mp_ensemble* e, d
   if (e->ndim < 1 || e->ndim > MP_MAX_NDIM) return fail(MP_ERR_BAD_ARG, w + ": bad ndim");
   if (!(beta > 0.0 && beta <= 1.0)) return fail(MP_ERR_BAD_ARG, w + ": beta must lie in (0, 1]");   // (NaN fails too)
   if (split != 0 && split != 1) return fail(MP_ERR_BAD_ARG, w + ": split must be 0 or 1");
-  if ((rc = check_moves(moves, n_moves, e->nwalkers / 2, who))) return rc;
+  if ((rc = check_moves(moves, n_moves, e, who))) return rc;
   if (!h) return fail(MP_ERR_BAD_ARG, w + ": null handle");
   return tempered_half_step(h, e, 1, &beta, pick_move(moves, n_moves, e->seed, step), step, split, stream);
 }

@@ -5,6 +5,7 @@
 #pragma once
 #include <math.h>
 #include <stdint.h>
+#include <string.h>
 
 #if defined(__CUDACC__)
 #define MP_RNG_HD __host__ __device__ inline
@@ -148,10 +149,11 @@ MP_RNG_HD MoveDraws move_draws(uint64_t seed, uint64_t hs, uint32_t me) {
   return d;
 }
 // The accept draw u of mover `me` (row) at half-step hs, ln u compared with ln f + lp(q) - lp(s): the stretch move's
-// (kind 0) from Philox counter (hs, me, 1), words 0-1; DE's and snooker's from block B of move_draws, = u[3].
+// (kind 0) from Philox counter (hs, me, 1), words 0-1; DE's and snooker's from block B of move_draws, = u[3]; the KDE
+// move's (kind 4, MP_MOVE_KDE) from words 2-3 of counter (hs, me, 8).
 MP_RNG_HD double accept_uniform(int kind, uint64_t seed, uint64_t hs, uint32_t me) {
-  const Philox r = philox4x32_10((uint32_t)hs, (uint32_t)(hs >> 32), me, kind == 0 ? 1u : 5u, (uint32_t)seed,
-                                 (uint32_t)(seed >> 32));
+  const Philox r = philox4x32_10((uint32_t)hs, (uint32_t)(hs >> 32), me, kind == 0 ? 1u : (kind == 4 ? 8u : 5u),
+                                 (uint32_t)seed, (uint32_t)(seed >> 32));
   return kind == 0 ? u01(r.c[0], r.c[1]) : u01(r.c[2], r.c[3]);
 }
 // DE: an ordered pair of distinct positions of the complement (nc >= 2).
@@ -187,6 +189,107 @@ MP_RNG_HD int choose_move(uint64_t seed, uint64_t step, const double* weights, i
     if (uw < cum) return k;
   }
   return last;
+}
+
+// ---- the kernel-density move: Gaussians that the host reproduces bit for bit -----------------------------------
+// libdevice's log / sincos and libm's differ in the last bit, so the KDE proposal uses its own, built from exact IEEE
+// operations only (the library is compiled with -fmad=false; a host build needs -ffp-contract=off).
+// ln x for a positive normal x: x = 2^e m with m in [sqrt(1/2), sqrt(2)] (bit manipulation), s = (m - 1)/(m + 1),
+// ln m = 2 atanh s by its series to s^23 (|s| <= 0.172), ln x = e ln2_hi + (e ln2_lo + ln m); ln2_hi has 32 bits, so
+// e ln2_hi is exact.
+MP_RNG_HD double kde_log(double x) {
+  uint64_t b;
+  memcpy(&b, &x, sizeof(b));
+  int e = (int)((b >> 52) & 0x7ffu) - 1023;
+  b = (b & 0x000FFFFFFFFFFFFFull) | 0x3FF0000000000000ull;
+  double m;
+  memcpy(&m, &b, sizeof(m));
+  if (m > 1.4142135623730951) {
+    m = m * 0.5;
+    e += 1;
+  }
+  const double s = (m - 1.0) / (m + 1.0);
+  const double s2 = s * s;
+  double p = 1.0 / 23.0;
+  p = p * s2 + 1.0 / 21.0;
+  p = p * s2 + 1.0 / 19.0;
+  p = p * s2 + 1.0 / 17.0;
+  p = p * s2 + 1.0 / 15.0;
+  p = p * s2 + 1.0 / 13.0;
+  p = p * s2 + 1.0 / 11.0;
+  p = p * s2 + 1.0 / 9.0;
+  p = p * s2 + 1.0 / 7.0;
+  p = p * s2 + 1.0 / 5.0;
+  p = p * s2 + 1.0 / 3.0;
+  p = p * s2 + 1.0;
+  const double ln2_hi = 6.93147180369123816490e-01, ln2_lo = 1.90821492927058770002e-10;
+  return (double)e * ln2_hi + ((double)e * ln2_lo + (2.0 * s) * p);
+}
+// sin and cos of x in [0, pi/4]: Taylor polynomials to x^19 and x^20 in Horner form.
+MP_RNG_HD void kde_sincos_poly(double x, double* s, double* c) {
+  const double x2 = x * x;
+  double p = -8.22063524662433e-18;
+  p = p * x2 + 2.8114572543455206e-15;
+  p = p * x2 + -7.647163731819816e-13;
+  p = p * x2 + 1.6059043836821613e-10;
+  p = p * x2 + -2.505210838544172e-08;
+  p = p * x2 + 2.7557319223985893e-06;
+  p = p * x2 + -0.0001984126984126984;
+  p = p * x2 + 0.008333333333333333;
+  p = p * x2 + -0.16666666666666666;
+  *s = x + x * (x2 * p);
+  double q = 4.110317623312165e-19;
+  q = q * x2 + -1.5619206968586225e-16;
+  q = q * x2 + 4.779477332387385e-14;
+  q = q * x2 + -1.1470745597729725e-11;
+  q = q * x2 + 2.08767569878681e-09;
+  q = q * x2 + -2.755731922398589e-07;
+  q = q * x2 + 2.48015873015873e-05;
+  q = q * x2 + -0.001388888888888889;
+  q = q * x2 + 0.041666666666666664;
+  q = q * x2 + -0.5;
+  *c = 1.0 + x2 * q;
+}
+// One Box-Muller pair: z = sqrt(-2 ln u1) (cos 2 pi u2, sin 2 pi u2), u1, u2 in (0, 1).  The quadrant is the integer
+// part of 4 u2 (exact), f its fraction (exact); the angle f pi/2 is reflected to (1 - f) pi/2 (exact) when f > 1/2,
+// so the polynomials see [0, pi/4] only.
+MP_RNG_HD void gauss_pair(double u1, double u2, double* z0, double* z1) {
+  const double r = sqrt(-2.0 * kde_log(u1));
+  const double t = 4.0 * u2;
+  const int quad = (int)t;
+  const double f = t - (double)quad;
+  const bool refl = f > 0.5;
+  double s, c;
+  kde_sincos_poly((refl ? 1.0 - f : f) * 1.5707963267948966, &s, &c);
+  if (refl) {
+    const double tmp = s;
+    s = c;
+    c = tmp;
+  }
+  // (c, s) = (cos, sin) of f pi/2; turn by quad quarter turns
+  double C = c, S = s;
+  if (quad == 1) { C = -s; S = c; }
+  else if (quad == 2) { C = -c; S = -s; }
+  else if (quad == 3) { C = s; S = -c; }
+  *z0 = r * C;
+  *z1 = r * S;
+}
+// The KDE mover's draws: u_c (which centre) from words 0,1 of Philox counter (hs, me, 8) -- words 2,3 are its accept
+// uniform -- and ndim standard normals, pair k from counter (hs, me, 9 + k), u1 = u01(words 0,1), u2 = u01(words 2,3).
+// Words 8 to 13 are used by no other draw.
+MP_RNG_HD double kde_centre_uniform(uint64_t seed, uint64_t hs, uint32_t me) {
+  const Philox r = philox4x32_10((uint32_t)hs, (uint32_t)(hs >> 32), me, 8u, (uint32_t)seed, (uint32_t)(seed >> 32));
+  return u01(r.c[0], r.c[1]);
+}
+MP_RNG_HD void kde_gaussians(uint64_t seed, uint64_t hs, uint32_t me, int ndim, double* z) {
+  for (int k = 0; 2 * k < ndim; ++k) {
+    const Philox r = philox4x32_10((uint32_t)hs, (uint32_t)(hs >> 32), me, 9u + (uint32_t)k, (uint32_t)seed,
+                                   (uint32_t)(seed >> 32));
+    double a, b;
+    gauss_pair(u01(r.c[0], r.c[1]), u01(r.c[2], r.c[3]), &a, &b);
+    z[2 * k] = a;
+    if (2 * k + 1 < ndim) z[2 * k + 1] = b;
+  }
 }
 
 // ---- sequential Monte Carlo (mp_smc_resample) ---------------------------------------------------------------

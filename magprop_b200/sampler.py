@@ -28,7 +28,7 @@ so this module carries the minimum needed to run and measure the path:
 ``SMCSampler``          sequential Monte Carlo with adaptive tempering: N particles annealed from the prior to the
                         posterior in stages (weights, ESS bisection, systematic resampling, MCMC moves at the stage's
                         beta), with ln Z from the stages' mean weights (include/magprop_smc.h).
-``StretchMove``, ``DEMove``, ``DESnookerMove``  emcee 3's ``moves=``: both ensembles take a move, a list of
+``StretchMove``, ``DEMove``, ``DESnookerMove``, ``KDEMove``  emcee 3's ``moves=``: the ensembles take a move, a list of
                         moves or a list of ``(move, weight)`` and run one of them per step
                         (``mp_ensemble_moves_half_step`` / ``mp_tempered_moves_half_step``).
 
@@ -179,15 +179,42 @@ class DESnookerMove:
         return f"DESnookerMove(gammas={self.gammas})"
 
 
-_PARTNERS = {0: 1, 1: 2, 2: 3}        # distinct complement walkers a move needs
+class KDEMove:
+    """emcee's ``KDEMove(bw_method=None)``: a fresh point drawn from a Gaussian kernel-density estimate of the complement
+    half, with the Hastings factor kde(x) / kde(q) -- nearly an independence proposal, so it can jump between modes.
+    ``bw_method``: None or ``"scott"`` (Scott's factor M^(-1/(ndim+4))) or a positive bandwidth factor.  The estimate is
+    built from at most ``MP_KDE_MAX_CENTRES`` complement walkers, a fresh random subset each half-step (emcee uses all
+    of them); one device only (include/magprop_b200.h, MP_MOVE_KDE)."""
+    kind = 4
+
+    def __init__(self, bw_method=None):
+        self.bw_method = bw_method
+
+    def _check(self):
+        b = self.bw_method
+        if b is None or (isinstance(b, str) and b == "scott"):
+            return
+        if isinstance(b, (bool, np.bool_)) or not isinstance(b, (int, float, np.integer, np.floating)) \
+                or not (np.isfinite(b) and b > 0.0):
+            raise ValueError("KDEMove needs bw_method None, 'scott' or a positive finite factor")
+
+    def _fill(self, m):
+        m.gamma0 = 0.0 if (self.bw_method is None or isinstance(self.bw_method, str)) else float(self.bw_method)
+
+    def __repr__(self):
+        return f"KDEMove(bw_method={self.bw_method!r})"
 
 
-def move_table(moves, half=None):
+_PARTNERS = {0: 1, 1: 2, 2: 3}        # distinct complement walkers a move needs (KDE: ndim + 1)
+
+
+def move_table(moves, half=None, ndim=None):
     """``moves`` as emcee accepts it -- a move, a list of moves (equal weights) or a list of ``(move, weight)`` --
     checked (``ValueError``) and returned as ``(list of (move, weight), ctypes array of mp_move)``.  ``half``: the
-    walkers in a half of the ensemble (per temperature), which must hold every partner a weighted move draws."""
+    walkers in a half of the ensemble (per temperature), which must hold every partner a weighted move draws, and
+    ndim + 1 centres for a weighted ``KDEMove`` (``ndim`` None: 1)."""
     from . import _capi as A
-    single = (StretchMove, DEMove, DESnookerMove)
+    single = (StretchMove, DEMove, DESnookerMove, KDEMove)
     if isinstance(moves, single):
         moves = [moves]
     try:
@@ -211,8 +238,9 @@ def move_table(moves, half=None):
         if not (np.isfinite(w) and w >= 0.0):
             raise ValueError("move weights must be finite and >= 0")
         mv._check()
-        if half is not None and w > 0.0 and half < _PARTNERS[mv.kind]:
-            raise ValueError(f"{mv!r} needs at least {_PARTNERS[mv.kind]} walkers in each half of the ensemble")
+        need = (1 if ndim is None else int(ndim)) + 1 if mv.kind == A.MP_MOVE_KDE else _PARTNERS[mv.kind]
+        if half is not None and w > 0.0 and half < need:
+            raise ValueError(f"{mv!r} needs at least {need} walkers in each half of the ensemble")
         table.append((mv, w))
     total = sum(w for _, w in table)
     if not (np.isfinite(total) and total > 0.0):
@@ -340,7 +368,7 @@ class DeviceEnsemble:
         from . import _capi as A
         if nwalkers % 2 or nwalkers < 2 * ndim:
             raise ValueError("nwalkers must be even and at least 2*ndim")
-        self.moves, self._moves_c = move_table(StretchMove(a) if moves is None else moves, nwalkers // 2)
+        self.moves, self._moves_c = move_table(StretchMove(a) if moves is None else moves, nwalkers // 2, ndim)
         self.torch, self.backend = torch, backend
         self.nwalkers, self.ndim, self.a, self.seed = nwalkers, ndim, float(a), int(seed)
         self.randomize_split = bool(randomize_split)
@@ -348,6 +376,8 @@ class DeviceEnsemble:
         self.dist = dist if (dist is not None and dist.is_initialized() and dist.get_world_size() > 1) else None
         self.rank = self.dist.get_rank() if self.dist else 0
         self.world = self.dist.get_world_size() if self.dist else 1
+        if self.dist and any(mv.kind == A.MP_MOVE_KDE and w > 0.0 for mv, w in self.moves):
+            raise ValueError("the KDE move runs on one device: dist is not supported with a weighted KDEMove")
         half = nwalkers // 2
         lo, hi = rank_slice(half, self.rank, self.world)
         self.n_mine = hi - lo

@@ -8,10 +8,13 @@ synthetic datasets (script model) and each particle count N in --sizes, over --s
   and the weights call of each stage) and resampling; the rest (lnprob of the prior draws, copies, the host) is what
   the three leave of the wall time.
 Then the thermodynamic-integration rows of profiles/r04_tempered_bench.txt, for comparison.  Every run is run_smc
-with its defaults (target_ess 0.5, DE 0.8 / snooker 0.2, p_move 0.99, 2..50 steps per stage), prior draws from the
-seed.
+with its defaults (target_ess 0.5, p_move 0.99, 2..50 steps per stage), prior draws from the seed, and the moves of
+--moves, one table per entry: "default" (DE 0.8 / snooker 0.2), "kde" (KDEMove() alone) and "kde_mix" (KDE 0.5 / DE 0.4
+/ snooker 0.1).  Each row also gives the mean acceptance of every stage.  For a move list with the KDE move,
+--profile-sizes adds one torch.profiler run of Sloped (seed 0) per particle count: the time of the KDE kernels
+(kde_prepare_kernel, kde_propose_kernel) per half-step that ran them and their share of the run's wall time.
 
-    python tools/smc_bench.py [--out FILE]
+    python tools/smc_bench.py [--moves default,kde,kde_mix] [--out FILE]
 """
 import argparse
 import json
@@ -64,7 +67,12 @@ def timed_backend(torch, base_cls):
     return Timed
 
 
-def one_run(torch, Timed, name, g, n, seed):
+def move_sets():
+    from magprop_b200.sampler import DEMove, DESnookerMove, KDEMove
+    return {"default": None, "kde": KDEMove(), "kde_mix": [(KDEMove(), 0.5), (DEMove(), 0.4), (DESnookerMove(), 0.1)]}
+
+
+def one_run(torch, Timed, name, g, n, seed, moves=None):
     from magprop_b200 import _capi as A
     from magprop_b200.engine import Likelihood, time_grid
     from magprop_b200.sampler import SMCSampler
@@ -75,7 +83,7 @@ def one_run(torch, Timed, name, g, n, seed):
     lk = Likelihood(A.script_model_spec(), time_grid(None), x, y, yerr, lower, upper)
     try:
         backend = Timed(lk)
-        smc = SMCSampler(backend, n, lower.size, seed=seed, device=torch.device("cuda", lk.device))
+        smc = SMCSampler(backend, n, lower.size, seed=seed, device=torch.device("cuda", lk.device), moves=moves)
         torch.cuda.synchronize()
         t0 = time.perf_counter()
         res = smc.run(p0)
@@ -87,12 +95,36 @@ def one_run(torch, Timed, name, g, n, seed):
     return res, wall, parts
 
 
+def kde_profile(torch, Timed, g, n, moves):
+    """One run of Sloped (seed 0) under torch.profiler: the KDE kernels' total time, launches and share of the wall."""
+    from torch.profiler import ProfilerActivity, profile
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        res, wall, _ = one_run(torch, Timed, "Sloped", g, n, 0, moves)
+    kde = {}
+    for ev in prof.key_averages():
+        if ev.key.startswith("_ZN2mp18kde_") or "kde_p" in ev.key:
+            kind = "prepare" if "prepare" in ev.key else "propose"
+            t = getattr(ev, "device_time_total", None)
+            if t is None:
+                t = ev.cuda_time_total
+            kde[kind] = (kde.get(kind, (0.0, 0))[0] + t / 1e3, kde.get(kind, (0.0, 0))[1] + ev.count)
+    half_steps = kde.get("prepare", (0.0, 0))[1]
+    total_ms = sum(v[0] for v in kde.values())
+    return {"kde_profile": "Sloped", "n_particles": n, "kde_half_steps": half_steps,
+            "kde_ms_per_half_step": round(total_ms / max(1, half_steps), 4),
+            "prepare_ms_per_half_step": round(kde.get("prepare", (0.0, 0))[0] / max(1, half_steps), 4),
+            "propose_ms_per_half_step": round(kde.get("propose", (0.0, 0))[0] / max(1, half_steps), 4),
+            "kde_share_of_wall": round(total_ms / 1e3 / wall, 4), "wall_s_profiled": round(wall, 3)}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--datasets", default="Humped,Classic,Sloped,Stuttering")
     ap.add_argument("--sizes", default="16384,65536,262144")
     ap.add_argument("--seeds", type=int, default=8)
     ap.add_argument("--seeds-large", type=int, default=2)
+    ap.add_argument("--moves", default="default")
+    ap.add_argument("--profile-sizes", default="16384,65536,262144")
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
 
@@ -115,29 +147,37 @@ def main():
                 f.write(s + "\n")
 
     emit({"card": card(), "torch_device": torch.cuda.get_device_name(0)})
-    one_run(torch, Timed, "Sloped", g, 1024, 0)                   # warm-up: module load, allocator pools
-    for n in (int(v) for v in args.sizes.split(",")):
-        for name in args.datasets.split(","):
-            seeds = args.seeds if n < (1 << 18) else args.seeds_large
-            rows = []
-            for seed in range(seeds):
-                res, wall, parts = one_run(torch, Timed, name, g, n, seed)
-                rows.append((res.log_evidence, res.n_stages, int(res.steps.sum()) + res.final_steps, res.n_evaluations,
-                             wall, parts))
-                del res
-            lz = np.array([r[0] for r in rows])
-            wall = np.mean([r[4] for r in rows])
-            evals = np.mean([r[3] for r in rows])
-            share = {k: round(float(np.mean([r[5][k] for r in rows])) / 1e3 / wall, 4) for k in rows[0][5]}
-            emit({"dataset": name, "n_particles": n, "seeds": seeds,
-                  "stages": round(float(np.mean([r[1] for r in rows])), 1),
-                  "mcmc_steps": round(float(np.mean([r[2] for r in rows])), 1),
-                  "lnprob_evals": int(evals), "wall_s": round(float(wall), 3), "evals_per_s": round(float(evals / wall), 1),
-                  "log_evidence_mean": round(float(lz.mean()), 4),
-                  "log_evidence_seed_sd": round(float(lz.std(ddof=1)), 4) if seeds > 1 else None,
-                  "log_evidence": [round(float(v), 4) for v in lz],
-                  "time_share": share,
-                  "time_s": {k: round(float(np.mean([r[5][k] for r in rows])) / 1e3, 4) for k in rows[0][5]}})
+    sets = move_sets()
+    for mname in args.moves.split(","):
+        moves = sets[mname]
+        one_run(torch, Timed, "Sloped", g, 1024, 0, moves)             # warm-up: module load, allocator pools
+        for n in (int(v) for v in args.sizes.split(",")):
+            for name in args.datasets.split(","):
+                seeds = args.seeds if n < (1 << 18) else args.seeds_large
+                rows = []
+                for seed in range(seeds):
+                    res, wall, parts = one_run(torch, Timed, name, g, n, seed, moves)
+                    rows.append((res.log_evidence, res.n_stages, int(res.steps.sum()) + res.final_steps, res.n_evaluations,
+                                 wall, parts, res.acceptance))
+                    del res
+                lz = np.array([r[0] for r in rows])
+                wall = np.mean([r[4] for r in rows])
+                evals = np.mean([r[3] for r in rows])
+                share = {k: round(float(np.mean([r[5][k] for r in rows])) / 1e3 / wall, 4) for k in rows[0][5]}
+                n_st = min(len(r[6]) for r in rows)
+                emit({"moves": mname, "dataset": name, "n_particles": n, "seeds": seeds,
+                      "stages": round(float(np.mean([r[1] for r in rows])), 1),
+                      "mcmc_steps": round(float(np.mean([r[2] for r in rows])), 1),
+                      "lnprob_evals": int(evals), "wall_s": round(float(wall), 3), "evals_per_s": round(float(evals / wall), 1),
+                      "log_evidence_mean": round(float(lz.mean()), 4),
+                      "log_evidence_seed_sd": round(float(lz.std(ddof=1)), 4) if seeds > 1 else None,
+                      "log_evidence": [round(float(v), 4) for v in lz],
+                      "acceptance_per_stage": [round(float(np.mean([r[6][k] for r in rows])), 4) for k in range(n_st)],
+                      "time_share": share,
+                      "time_s": {k: round(float(np.mean([r[5][k] for r in rows])) / 1e3, 4) for k in rows[0][5]}})
+        if mname != "default" and args.profile_sizes:
+            for n in (int(v) for v in args.profile_sizes.split(",")):
+                emit(dict(kde_profile(torch, Timed, g, n, moves), moves=mname))
     r04 = os.path.join(ROOT, "profiles", "r04_tempered_bench.txt")
     for line in open(r04):
         d = json.loads(line)
