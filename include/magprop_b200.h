@@ -349,6 +349,7 @@ int mp_chain_moments(const double* d_chain, int64_t n, int32_t ndim, double* mea
                      int32_t device, void* stream);
 int mp_chain_order_statistics(const double* d_chain, int64_t n, int32_t ndim, int32_t col,
                               const int64_t* ranks, int32_t n_ranks, double* values, int32_t device, void* stream);
+/* The order statistics of many columns at once, for credible bands of light curves, are declared in magprop_band.h. */
 /* Walker-averaged normalised autocorrelation function of a device-resident chain [n_steps][nwalkers][ndim]
  * (emcee's integrated_time before the window): rows first, first+thin, ...; lags [lag_begin, lag_end) of the
  * n = ceil((n_steps-first)/thin) retained rows; acf is a HOST array [ndim][lag_end-lag_begin].  Synchronises.

@@ -161,6 +161,7 @@ def declare(lib):
     lib.mp_peer_barrier.argtypes = [C.c_int32, vp, C.POINTER(vp), C.c_int32, C.c_int32, C.c_uint64, vp, vp]
     lib.mp_chain_moments.argtypes = [vp, C.c_int64, C.c_int32, vp, vp, C.c_int32, vp]
     lib.mp_chain_order_statistics.argtypes = [vp, C.c_int64, C.c_int32, C.c_int32, vp, C.c_int32, vp, C.c_int32, vp]
+    lib.mp_columns_order_statistics.argtypes = [vp, C.c_int64, C.c_int64, C.c_int64, vp, C.c_int32, vp, C.c_int32, vp]
     lib.mp_chain_autocorr.argtypes = [vp, C.c_int64, C.c_int32, C.c_int32, C.c_int64, C.c_int64, C.c_int64, C.c_int64,
                                       vp, C.c_int32, vp]
     lib.mp_gompertz_curves.argtypes = [vp, C.c_int32, vp, C.c_int64, C.c_int32, vp, C.c_int32]
@@ -186,6 +187,9 @@ EXPORTS = ["mp_abi_version", "mp_device_count", "mp_last_error", "mp_create", "m
 # The entry points include/magprop_smc.h declares (sequential Monte Carlo), exported by the same library.
 SMC_EXPORTS = ["mp_smc_weights", "mp_smc_resample", "mp_annealed_moves_half_step"]
 MP_SMC_TILE = 64
+# The entry point include/magprop_band.h declares (order statistics of many columns, for credible bands).
+BAND_EXPORTS = ["mp_columns_order_statistics"]
+MP_COLUMN_SELECT_MAX = 16384
 
 
 def load():

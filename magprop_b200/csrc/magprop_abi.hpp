@@ -10,6 +10,7 @@
 #include <vector>
 
 #include "../../include/magprop_b200.h"
+#include "../../include/magprop_band.h"
 #include "../../include/magprop_smc.h"
 
 namespace mp {
@@ -42,6 +43,13 @@ inline int select_device(int device, const char* who) {
   const cudaError_t e = cudaSetDevice(device);
   if (e != cudaSuccess) return fail(MP_ERR_CUDA, std::string(who) + ": cudaSetDevice: " + cudaGetErrorString(e));
   return MP_OK;
+}
+
+// [p, p + bytes) and [q, q + qbytes) share a byte (a null range shares none).
+inline bool overlaps(const void* p, __int128 bytes, const void* q, __int128 qbytes) {
+  if (!p || !q) return false;
+  const __int128 a = (__int128)(uintptr_t)p, b = (__int128)(uintptr_t)q;
+  return a < b + qbytes && b < a + bytes;
 }
 
 // A device array that owns its memory: moved, never copied, and freed by its destructor.  Its size is the capacity in elements.

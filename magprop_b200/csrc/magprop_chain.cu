@@ -1,7 +1,8 @@
 // magprop_chain.cu -- posterior summaries of a device-resident chain: column means and covariances
 // (mp_chain_moments), exact order statistics (mp_chain_order_statistics) and the walker-averaged autocorrelation
 // function (mp_chain_autocorr).  They read a chain the caller keeps on the device and return a few numbers to the
-// host; none of them uses a likelihood handle.
+// host; none of them uses a likelihood handle.  mp_columns_order_statistics selects ranks of many columns at once (a
+// credible band over a set of light curves) and leaves its result on the device.
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -105,6 +106,10 @@ __device__ __forceinline__ unsigned long long order_key(double v) {
   if ((b & 0x7fffffffffffffffull) > 0x7ff0000000000000ull) b &= 0x7fffffffffffffffull;
   return (b >> 63) ? ~b : (b | 0x8000000000000000ull);
 }
+// The bits of the double a key stands for (the inverse of order_key; a NaN comes back with its sign bit cleared).
+__host__ __device__ __forceinline__ unsigned long long key_bits(unsigned long long key) {
+  return (key >> 63) ? (key & 0x7fffffffffffffffull) : ~key;
+}
 constexpr int kSelectBins = 1 << 16;   // one per value of the 16-bit digit a radix-select pass sorts on
 // One pass of the radix select on column `col`: histogram of the 16-bit digit at `shift` over the elements whose
 // higher digits equal those of `prefix`.  64-bit bins, so a column of 2^32 or more equal digits cannot wrap one.  The
@@ -125,6 +130,42 @@ __global__ void select_hist_kernel(const double* __restrict__ x, long long n, in
     }
     const unsigned peers = __match_any_sync(kFull, bin);
     if (bin != 0xffffffffu && lane == __ffs(peers) - 1) atomicAdd(hist + bin, (unsigned long long)__popc(peers));
+  }
+}
+
+// ---- exact order statistics of many columns at once (the credible band of a set of light curves) ------------------
+// One block per column: the column's n keys go to dynamic shared memory, padded to npad = the next power of two with
+// all-ones keys.  That is the largest key, so the padding sorts after every element, and a NaN whose key it equals
+// decodes to the same NaN.  A bitonic network sorts the keys in place; the block then writes the requested ranks.
+// Ranks travel in the launch's parameters, kColRanks per launch: more ranks take more launches, each sorting again.
+constexpr int kColRanks = 256, kColThreads = 1024;
+struct ColRanks {
+  long long r[kColRanks];
+};
+
+__global__ void __launch_bounds__(kColThreads) column_select_kernel(const double* __restrict__ x, int n, int npad,
+                                                                    long long n_cols, long long ld,
+                                                                    const __grid_constant__ ColRanks ranks, int n_ranks,
+                                                                    double* __restrict__ out /*[n_ranks][n_cols]*/) {
+  extern __shared__ unsigned long long col_keys[];
+  for (long long c = blockIdx.x; c < n_cols; c += gridDim.x) {
+    __syncthreads();                                   // the previous column's ranks have been read
+    for (int i = threadIdx.x; i < npad; i += blockDim.x) col_keys[i] = i < n ? order_key(x[i * ld + c]) : ~0ull;
+    __syncthreads();
+    for (int k = 2; k <= npad; k <<= 1)
+      for (int j = k >> 1; j > 0; j >>= 1) {
+        for (int t = threadIdx.x; t < (npad >> 1); t += blockDim.x) {
+          const int i = ((t & ~(j - 1)) << 1) | (t & (j - 1)), p = i + j;   // pair (i, i + j), bit j of i clear
+          const unsigned long long a = col_keys[i], b = col_keys[p];
+          if ((a > b) == ((i & k) == 0)) {               // ascending where bit k of i is clear
+            col_keys[i] = b;
+            col_keys[p] = a;
+          }
+        }
+        __syncthreads();
+      }
+    for (int r = threadIdx.x; r < n_ranks; r += blockDim.x)
+      out[r * n_cols + c] = __longlong_as_double((long long)key_bits(col_keys[ranks.r[r]]));
   }
 }
 
@@ -339,14 +380,47 @@ extern "C" int mp_chain_order_statistics(const double* d_chain, int64_t n, int32
       for (; digit < kSelectBins - 1u && k >= hist[digit]; ++digit) k -= hist[digit];
       prefix |= (unsigned long long)digit << shift;
     }
-    // key -> double
-    const unsigned long long b = (prefix >> 63) ? (prefix & 0x7fffffffffffffffull) : ~prefix;
+    const unsigned long long b = key_bits(prefix);
     std::memcpy(values + r, &b, sizeof(double));
   }
   const cudaError_t ef = cudaFreeAsync(d_hist, st);
   if (e == cudaSuccess) e = ef;
   if (e == cudaSuccess) e = cudaStreamSynchronize(st);
   if (e != cudaSuccess) return fail(MP_ERR_CUDA, std::string("mp_chain_order_statistics: ") + cudaGetErrorString(e));
+  return MP_OK;
+}
+
+extern "C" int mp_columns_order_statistics(const double* d_x, int64_t n, int64_t n_cols, int64_t ld, const int64_t* ranks,
+                                           int32_t n_ranks, double* d_out, int32_t device, void* stream) {
+  if (!d_x || !d_out || !ranks) return fail(MP_ERR_BAD_ARG, "mp_columns_order_statistics: null x, ranks or out");
+  if (n < 1 || n > MP_COLUMN_SELECT_MAX)
+    return fail(MP_ERR_BAD_ARG, "mp_columns_order_statistics: n must lie in 1..MP_COLUMN_SELECT_MAX");
+  if (n_cols < 1 || ld < n_cols) return fail(MP_ERR_BAD_ARG, "mp_columns_order_statistics: need 1 <= n_cols <= ld");
+  if (n_ranks < 1) return fail(MP_ERR_BAD_ARG, "mp_columns_order_statistics: n_ranks must be >= 1");
+  for (int r = 0; r < n_ranks; ++r)
+    if (ranks[r] < 0 || ranks[r] >= n) return fail(MP_ERR_BAD_ARG, "mp_columns_order_statistics: rank outside [0, n)");
+  const __int128 x_bytes = ((__int128)(n - 1) * ld + n_cols) * 8, out_bytes = (__int128)n_ranks * n_cols * 8;
+  if (overlaps(d_out, out_bytes, d_x, x_bytes)) return fail(MP_ERR_BAD_ARG, "mp_columns_order_statistics: out overlaps x");
+  int rc = select_device(device, "mp_columns_order_statistics");
+  if (rc) return rc;
+  MP_CUDA(cudaFuncSetAttribute(column_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                               (int)(MP_COLUMN_SELECT_MAX * sizeof(unsigned long long))));
+  cudaStream_t st = (cudaStream_t)stream;
+  int npad = 1;
+  while (npad < n) npad <<= 1;
+  // shared memory sized from n, so that short columns fit several blocks on an SM
+  const size_t smem = (size_t)npad * sizeof(unsigned long long);
+  const int threads = std::min(kColThreads, std::max(32, npad >> 1));
+  const unsigned blocks = (unsigned)std::min<int64_t>(n_cols, 1 << 24);
+  cudaError_t e = cudaSuccess;
+  for (int r0 = 0; r0 < n_ranks && e == cudaSuccess; r0 += kColRanks) {
+    ColRanks cr;
+    const int m = std::min(kColRanks, n_ranks - r0);
+    for (int i = 0; i < m; ++i) cr.r[i] = ranks[r0 + i];
+    column_select_kernel<<<blocks, threads, smem, st>>>(d_x, (int)n, npad, n_cols, ld, cr, m, d_out + (int64_t)r0 * n_cols);
+    e = cudaGetLastError();
+  }
+  if (e != cudaSuccess) return fail(MP_ERR_CUDA, std::string("mp_columns_order_statistics: ") + cudaGetErrorString(e));
   return MP_OK;
 }
 

@@ -174,13 +174,6 @@ __global__ void smc_ancestor_kernel(const double* __restrict__ w, long long n, i
   }
 }
 
-// [p, p + bytes) and [q, q + qbytes) share a byte (a null range shares none).
-static bool overlaps(const void* p, __int128 bytes, const void* q, __int128 qbytes) {
-  if (!p || !q) return false;
-  const __int128 a = (__int128)(uintptr_t)p, b = (__int128)(uintptr_t)q;
-  return a < b + qbytes && b < a + bytes;
-}
-
 static int grid_for(long long items) { return (int)std::min<long long>((items + 255) / 256, 1LL << 20); }
 
 }  // namespace mp

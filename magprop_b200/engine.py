@@ -9,6 +9,7 @@ launch or raises ``MagpropCudaError``.
 from __future__ import annotations
 
 import ctypes as C
+import dataclasses
 
 import numpy as np
 
@@ -31,6 +32,31 @@ def _f64(a, ndim=None):
     if ndim is not None and a.ndim != ndim:
         raise ValueError(f"expected a {ndim}-D array, got shape {a.shape}")
     return a
+
+
+def band_percentiles(percentiles) -> np.ndarray:
+    """The percentiles of a credible band as a float64 array; ValueError unless a non-empty list of finite values in
+    [0, 100]."""
+    q = np.asarray(percentiles, dtype=np.float64).reshape(-1)
+    if q.size == 0 or not (np.isfinite(q) & (q >= 0.0) & (q <= 100.0)).all():
+        raise ValueError(f"percentiles must be finite and lie in [0, 100], got {percentiles!r}")
+    return q
+
+
+@dataclasses.dataclass
+class CurveBand:
+    """Percentiles of the model light curve over posterior draws, at every node: ``ltot``, ``lprop``, ``ldip`` (and,
+    with state, ``mdisc`` and ``omega``) are ``[len(percentiles), len(t)]``, luminosities in units of 1e50 erg/s.
+    ``n_used`` draws went in; ``n_flagged`` were dropped because their integration failed (model_lum's 'flag')."""
+    t: np.ndarray
+    percentiles: np.ndarray
+    ltot: np.ndarray
+    lprop: np.ndarray
+    ldip: np.ndarray
+    n_used: int
+    n_flagged: int
+    mdisc: np.ndarray = None
+    omega: np.ndarray = None
 
 
 class Likelihood:
@@ -145,6 +171,58 @@ class Likelihood:
             idx.append(self.grid.size - 1)
         return self.grid[idx]
 
+    def curve_band(self, pars, percentiles, node_stride=1, with_state=False) -> CurveBand:
+        """Credible band of the light curve over the posterior draws ``pars``, a float64 CUDA tensor [S, ndim] of
+        physical parameters on this handle's device: ``np.percentile(curves, percentiles, axis=0)`` of their full curves
+        (and, ``with_state``, of M_disc and omega), equal to it bit for bit.  The curves are solved and their columns'
+        order statistics selected on the device, on torch's current stream; draws whose integration fails are dropped
+        (the one host read is how many are kept), and only the selected [ranks, columns] come to the host, where
+        NumPy's interpolation is applied (``plot_synth.percentile_ranks``, ``interpolate_percentiles``).  Draws with
+        parameters outside the physical domain stay in; where their state is not finite their luminosity is 0, as the
+        reference's clamps make it."""
+        import torch
+
+        from .synthetic.plot_synth import interpolate_percentiles, percentile_ranks
+        q = band_percentiles(percentiles)
+        if not (isinstance(pars, torch.Tensor) and pars.dtype == torch.float64 and pars.dim() == 2):
+            raise ValueError("curve_band: pars must be a 2-D float64 torch tensor [S, ndim]")
+        S, ndim = pars.shape
+        if not 1 <= S <= A.MP_COLUMN_SELECT_MAX:
+            raise ValueError(f"curve_band: the number of draws must lie in [1, {A.MP_COLUMN_SELECT_MAX}], got {S}")
+        if not (pars.is_cuda and pars.device.index == self.device):
+            raise ValueError(f"curve_band: pars must be on cuda:{self.device}, got {pars.device}")
+        pars = pars.contiguous()
+        st = torch.cuda.current_stream(pars.device).cuda_stream
+        Gs = self.curve_nodes(node_stride)
+        curves = torch.empty((S, 3, Gs), dtype=torch.float64, device=pars.device)
+        state = torch.empty((S, 2, Gs), dtype=torch.float64, device=pars.device) if with_state else None
+        status = torch.empty(S, dtype=torch.int32, device=pars.device)
+        self.curves_device(pars.data_ptr(), S, ndim, node_stride, curves.data_ptr(),
+                           state.data_ptr() if with_state else 0, status.data_ptr(), st)
+        keep = torch.nonzero((status & A.WALKER_INTEGRATOR_FAIL) == 0).squeeze(1)
+        n_used = keep.numel()
+        if n_used == 0:
+            raise RuntimeError(f"curve_band: the integration failed for every one of the {S} draws")
+        k0, k1, gamma, ranks = percentile_ranks(n_used, q)
+        i0, i1, top = np.searchsorted(ranks, k0), np.searchsorted(ranks, k1), ranks.size - 1
+
+        def band(x):
+            if n_used < S:
+                x = x.index_select(0, keep)
+            cols = x[0].numel()
+            sel = torch.empty((ranks.size, cols), dtype=torch.float64, device=x.device)
+            columns_order_statistics(x.data_ptr(), n_used, cols, cols, ranks, sel.data_ptr(), device=self.device,
+                                     stream=st)
+            h = sel.cpu().numpy()
+            return interpolate_percentiles(h[i0], h[i1], gamma, h[top]).reshape((q.size,) + tuple(x.shape[1:]))
+
+        lum = band(curves)
+        out = CurveBand(self.node_times(node_stride), q, lum[:, 0], lum[:, 1], lum[:, 2], n_used, S - n_used)
+        if with_state:
+            st2 = band(state)
+            out.mdisc, out.omega = st2[:, 0], st2[:, 1]
+        return out
+
     def last_stiff_count(self) -> int:
         """Walkers of the last launch that were handed to the implicit integrator (synchronises)."""
         n = C.c_int32(0)
@@ -214,6 +292,15 @@ def chain_order_statistics(d_chain: int, n: int, ndim: int, col: int, ranks, dev
     out = np.empty(ranks.size)
     A.check(lib.mp_chain_order_statistics(d_chain, n, ndim, col, A.ptr(ranks), ranks.size, A.ptr(out), device, stream or None))
     return out
+
+
+def columns_order_statistics(d_x: int, n: int, n_cols: int, ld: int, ranks, d_out: int, device=0, stream=0):
+    """Exact order statistics (0-based ranks) of every column of a device array of n rows, element (i, c) at
+    ``d_x[i*ld + c]`` (raw pointer), into the device array ``d_out`` [len(ranks), n_cols].  Enqueued on ``stream``, not
+    synchronised."""
+    lib = A.load()
+    ranks = np.ascontiguousarray(ranks, dtype=np.int64)
+    A.check(lib.mp_columns_order_statistics(d_x, n, n_cols, ld, A.ptr(ranks), ranks.size, d_out, device, stream or None))
 
 
 def chain_autocorr(d_chain: int, n_steps: int, nwalkers: int, ndim: int, first=0, thin=1, lag_begin=0, lag_end=None,
